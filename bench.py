@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: edge-updates/sec per message-passing layer (forward + backward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4], SURVEY.md s8 cfg 5): synthetic 1000 x 1000 triangulated grid,
 N = 1 000 000 nodes, E = 5 992 002 directed mesh edges, latent 128, 15 unshared GraphNet layers, `sum`
@@ -193,6 +193,39 @@ def make_processor(weights, layers, precision, device, aggregator="sum"):
     return proc
 
 
+DUMP_ROWS = 16384                        # rows kept per latent / latent-gradient array by --dump-outputs
+DUMP_SEED = 7
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_rows(n):
+    """The fixed sample of `n` rows that --dump-outputs keeps: all of them up to DUMP_ROWS, else DUMP_ROWS seeded rows in order."""
+    if n <= DUMP_ROWS:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(DUMP_SEED))[:DUMP_ROWS].sort().values
+
+
+def dump_outputs(out_dir, loss, out, v, ed, named_params):
+    """--dump-outputs: what one step hands its caller, as float32 ``<out_dir>/<name>.npy`` -- the loss, the output node and edge
+    latents and the gradients of the input latents (each on the fixed row sample of `dump_rows`), and every parameter gradient in
+    full (``grad.<parameter name>.npy``).  The inputs are seeded, so two builds run with the same arguments can be compared array by
+    array."""
+    import numpy as np
+    arrays = {"loss": loss.detach().reshape(())}
+    for name, t in (("node_latents", out.node_features[0]), ("edge_latents", out.edge_sets[0].features),
+                    ("node_latents_grad", v.grad), ("edge_latents_grad", ed.grad)):
+        arrays[name] = t.detach()[dump_rows(t.shape[0]).to(t.device)]
+    for name, p in named_params:
+        if p.grad is not None:
+            arrays["grad." + name] = p.grad.detach()
+    total = sum(t.numel() * 4 for t in arrays.values())
+    if total > DUMP_BYTES_MAX:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES_MAX}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def fp32_parity_mode(dev):
     """The 1e-5 parity mode (`precision = "fp32"`: fp32 storage, FFMA kernels) beside the bf16 headline, against an fp32 denominator
     measured here the way MEASURED_PEAKS.json measures bf16 (SURVEY.md s8d): torch.matmul fp32 8192^3 with TF32 off, best of 10 and a
@@ -302,6 +335,8 @@ def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs: single-GPU runs only")
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
@@ -331,7 +366,7 @@ def run_ours(args):
     e_dev = e0_host.to(dev).to(torch.bfloat16)
     loss_host = torch.empty(1, dtype=torch.float32).pin_memory()
 
-    def step(v_in, e_in):
+    def step(v_in, e_in, keep=None):
         for p in params:
             p.grad = None
         v = v_in.requires_grad_(True)
@@ -341,6 +376,8 @@ def run_ours(args):
         loss.backward()
         if world > 1:
             partition.allreduce_gradients(proc)
+        if keep is not None:                    # the step whose results --dump-outputs writes
+            keep.update(loss=loss, out=out, v=v, ed=ed)
         return loss
 
     def max_over_ranks(ms):
@@ -355,8 +392,8 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def step_resident():
-        return step(v_dev.detach(), e_dev.detach())
+    def step_resident(keep=None):
+        return step(v_dev.detach(), e_dev.detach(), keep)
 
     copy_stream = torch.cuda.Stream(device=dev)
 
@@ -390,12 +427,13 @@ def run_ours(args):
     # ---- timed region: inputs resident in HBM --------------------------------------------------------
     _cabi.profile(True)
     launches0 = ops.launch_count
+    last = {} if args.dump_outputs else None
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local_rank) as clocks:
         fence()
         start.record()
-        for _ in range(args.steps):
-            step_resident()
+        for i in range(args.steps):
+            step_resident(last if i == args.steps - 1 else None)
         stop.record()
         fence()
     ms_per_step = max_over_ranks(start.elapsed_time(stop) / args.steps)
@@ -403,13 +441,16 @@ def run_ours(args):
     kernels = _cabi.profile_report()
     _cabi.profile(False)
     value = e * layers * world / (ms_per_step * 1e-3)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last["loss"], last["out"], last["v"], last["ed"], proc.named_parameters())
+        del last
 
     # ---- end to end: pinned host inputs -> H2D -> fwd+bwd -> D2H loss ---------------------------------
     run_e2e(3)                                  # warm-up: two input sets are alive at a time, let the allocator cache both
     fence()
-    # the first step's copy has nothing to hide behind (65 ms of PCIe time at cfg5); a pipeline is quoted over enough steps that this
-    # start-up share is small: at least 12, every one of them with its own H2D copy and loss read-back inside the region
-    e2e_steps = max(12, args.steps)
+    # --steps steps, every one of them with its own H2D copy and loss read-back inside the region; the first step's copy has nothing
+    # to hide behind (65 ms of PCIe time at cfg5), so its share of the quote shrinks as --steps grows
+    e2e_steps = args.steps
     t0 = torch.cuda.Event(enable_timing=True); t1 = torch.cuda.Event(enable_timing=True)
     t0.record()                                 # on the compute stream, which waits for every copy it consumes
     run_e2e(e2e_steps)
@@ -645,7 +686,7 @@ def graphed_step(step_fn, params, steps, edge_updates_per_step):
             graph.replay()
         torch.cuda.synchronize()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        reps = max(steps, 20)
+        reps = steps
         a.record()
         for _ in range(reps):
             graph.replay()
@@ -1090,7 +1131,14 @@ def main():
     ap.add_argument("--workload", default="cfg5", choices=sorted(WORKLOADS) + ["cfg3"],
                     help="cfg5 = the headline 1M/6M mesh (the bench line); cfg2 / cfg4 = small-mesh batched training shapes; "
                          "cfg3 = HeteroGraphNet on a plateCluster-shaped batch (single GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, sampled output latents and input-latent "
+                         "gradients, parameter gradients) as float32 DIR/<name>.npy, at most 64 MB; single GPU, cfg2 / cfg4 / cfg5")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "cfg3"):
+        ap.error("--dump-outputs covers the single-GPU path of --impl ours on cfg2 / cfg4 / cfg5")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "cfg3":

@@ -103,6 +103,34 @@ def test_cfg3_plate_clustering_and_batched_graph(monkeypatch):
         assert int(max(es.senders.max(), es.receivers.max())) < n + sizes["hyper_nodes"]
 
 
+def test_dump_outputs_writes_float32_arrays_on_a_fixed_row_sample(tmp_path):
+    """--dump-outputs: loss, sampled latents and latent gradients, full parameter gradients, all float32, within 64 MB; the row
+    sample is a fixed, sorted, duplicate-free function of the row count."""
+    import numpy as np
+    from hgn_b200.util import EdgeSet, MultiGraph
+    n, e = 300, bench.DUMP_ROWS + 500
+    g = torch.Generator().manual_seed(3)
+    v = torch.randn(n, 128, generator=g).to(torch.bfloat16)
+    ed = torch.randn(e, 128, generator=g)
+    v.grad, ed.grad = torch.randn(n, 128, generator=g).to(torch.bfloat16), torch.randn(e, 128, generator=g)
+    out = MultiGraph([v * 2], [EdgeSet("mesh_edges", ed * 3, None, None)])
+    w = torch.nn.Parameter(torch.randn(128, 384, generator=g))
+    w.grad = torch.randn(128, 384, generator=g)
+    unused = torch.nn.Parameter(torch.zeros(4))
+    bench.dump_outputs(str(tmp_path / "d"), torch.tensor(1.5), out, v, ed, [("blk.w", w), ("blk.unused", unused)])
+    files = {f.name[:-4]: np.load(f) for f in (tmp_path / "d").iterdir()}
+    assert set(files) == {"loss", "node_latents", "edge_latents", "node_latents_grad", "edge_latents_grad", "grad.blk.w"}
+    assert all(a.dtype == np.float32 for a in files.values()) and sum(a.nbytes for a in files.values()) <= bench.DUMP_BYTES_MAX
+    rows = bench.dump_rows(e)
+    assert torch.equal(rows, bench.dump_rows(e)) and rows.numel() == bench.DUMP_ROWS
+    assert bool((rows[1:] > rows[:-1]).all()) and int(rows[-1]) < e
+    assert torch.equal(bench.dump_rows(n), torch.arange(n))
+    assert float(files["loss"]) == 1.5 and files["node_latents"].shape == (n, 128) and files["edge_latents"].shape == (bench.DUMP_ROWS, 128)
+    assert np.array_equal(files["node_latents"], (v * 2).float().numpy())
+    assert np.array_equal(files["edge_latents_grad"], ed.grad[rows].numpy())
+    assert np.array_equal(files["grad.blk.w"], w.grad.numpy())
+
+
 def test_clock_sampler_summary_from_nvml_and_nvidia_smi_rows():
     """The `clocks` object of the bench line: median SM clock, max clock and the set of active clock-event reasons, from NVML samples
     (numbers + 'Active' / 'Not Active') and from `nvidia-smi --format=csv` rows (strings); 'unavailable' without samples or a GPU."""

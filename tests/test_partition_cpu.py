@@ -223,7 +223,9 @@ def _norm_worker(rank, world, port, tmpdir):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
+        from hgn_b200 import util
         from hgn_b200.migration.normalizer import Normalizer
+        util.device = torch.device("cpu")                                # host statistics, also where a GPU is visible
         nzs = [Normalizer(5, "a"), Normalizer(5, "b")]
         outs = []
         for step in range(3):
@@ -238,10 +240,12 @@ def _norm_worker(rank, world, port, tmpdir):
         dist.destroy_process_group()
 
 
-def test_two_rank_normalizer_statistics_match_one_process_seeing_all_batches(tmp_path):
+def test_two_rank_normalizer_statistics_match_one_process_seeing_all_batches(tmp_path, monkeypatch):
     """Replicas accumulate their own batches; `allreduce_normalizers` leaves every rank with the totals of a single process that
     accumulated all ranks' batches (rank order within a step), so normalised features agree across replicas and with that process."""
+    from hgn_b200 import util
     from hgn_b200.migration.normalizer import Normalizer
+    monkeypatch.setattr(util, "device", torch.device("cpu"))            # the workers keep their statistics on the host too
     world = 2
     port = 33500 + (os.getpid() % 2000)
     mp.spawn(_norm_worker, args=(world, port, str(tmp_path)), nprocs=world, join=True)
