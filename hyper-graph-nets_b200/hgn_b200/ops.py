@@ -299,20 +299,105 @@ def fused_mlp(params: Sequence[torch.Tensor], packed_cache: dict, sources: Seque
 # ------------------------------------------------------------------------------------------------
 # projected edge update (bf16): node-side pre-projection + fused edge kernels (csrc/edge_tc.cu)
 # ------------------------------------------------------------------------------------------------
+# One binding per entry point: marshal the pointers, check the return code, count the kernels the C side launches.
+_BF = _cabi.HGN_BF16
+
+
+def _edge_project_forward(v, packed, ps, pr) -> None:
+    n = v.shape[0]
+    _cabi.check(_cabi.load().hgn_edge_project_forward(_BF, n, v.data_ptr(), packed.data_ptr(), ps.data_ptr(), pr.data_ptr(),
+                                                      _cabi.stream_ptr()), "hgn_edge_project_forward")
+    _count(int(n > 0))          # edge_project_forward_tc: one proj_tc_kernel
+
+
+def _edge_project_backward(v, packed, gs, gr, grad_v_add, grad_v, grad_w0, ws=None) -> None:
+    lib, n = _cabi.load(), v.shape[0]
+    if ws is None:
+        ws = torch.empty(lib.hgn_edge_project_backward_workspace_bytes(_BF, n), dtype=torch.uint8, device=v.device)
+    _cabi.check(lib.hgn_edge_project_backward(_BF, n, v.data_ptr(), packed.data_ptr(), gs.data_ptr(), gr.data_ptr(), _cabi.ptr(grad_v_add),
+                                              grad_v.data_ptr(), grad_w0.data_ptr(), ws.data_ptr(), ws.numel(), _cabi.stream_ptr()),
+                "hgn_edge_project_backward")
+    _count(4)                   # edge_project_backward_tc: dgrad, pair wgrad, two reduce_w0_block_kernel
+
+
+def _edge_update_forward(e, ps, pr, s_plan, r_plan, packed, out) -> None:
+    E = e.shape[0]
+    _cabi.check(_cabi.load().hgn_edge_update_forward(_BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(),
+                                                     r_plan.ids32.data_ptr(), packed.data_ptr(), out.data_ptr(), _cabi.stream_ptr()),
+                "hgn_edge_update_forward")
+    _count(int(E > 0))          # edge_fwd_tc_launch: one edge_fwd_tc_kernel
+
+
+def _edge_update_backward(e, ps, pr, s_plan, r_plan, packed, grad_out, grad_agg, grad_e, g0, gparams, ws=None) -> None:
+    lib, E = _cabi.load(), e.shape[0]
+    if ws is None:
+        ws = torch.empty(lib.hgn_edge_update_backward_workspace_bytes(_BF, E), dtype=torch.uint8, device=e.device)
+    _cabi.check(lib.hgn_edge_update_backward(
+        _BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(), r_plan.ids32.data_ptr(), packed.data_ptr(),
+        _cabi.ptr(grad_out), _cabi.ptr(grad_agg), grad_e.data_ptr(), g0.data_ptr(), *[g.data_ptr() for g in gparams], ws.data_ptr(),
+        ws.numel(), _cabi.stream_ptr()), "hgn_edge_update_backward")
+    _count(2)                   # projected_backward_launch: edge_bwd_tc_kernel, edge_bwd_reduce_kernel
+
+
+def _node_update_forward(v, aggs, packed, q1, q2, out) -> None:
+    n, k = v.shape[0], len(aggs)
+    agg_ptrs = (ctypes.c_void_p * k)(*[a.data_ptr() for a in aggs])
+    _cabi.check(_cabi.load().hgn_node_update_forward(_BF, n, v.data_ptr(), k, agg_ptrs, packed.data_ptr(), q1.data_ptr(), _cabi.ptr(q2),
+                                                     out.data_ptr(), _cabi.stream_ptr()), "hgn_node_update_forward")
+    _count((k + 1) // 2 + 1 if n > 0 else 0)    # node_update_forward_tc: one projection per table of two aggregates, node_fwd_tc
+
+
+def _node_update_backward(v, aggs, q1, q2, packed, grad_out, grad_v, grad_aggs, gparams, ws=None) -> None:
+    lib, n, k = _cabi.load(), v.shape[0], len(aggs)
+    if ws is None:
+        ws = torch.empty(lib.hgn_node_update_backward_workspace_bytes(_BF, n), dtype=torch.uint8, device=v.device)
+    agg_ptrs = (ctypes.c_void_p * k)(*[a.data_ptr() for a in aggs])
+    gagg_ptrs = (ctypes.c_void_p * k)(*[g.data_ptr() for g in grad_aggs])
+    _cabi.check(lib.hgn_node_update_backward(_BF, n, v.data_ptr(), k, agg_ptrs, q1.data_ptr(), _cabi.ptr(q2), packed.data_ptr(),
+                                             grad_out.data_ptr(), grad_v.data_ptr(), gagg_ptrs, *[g.data_ptr() for g in gparams],
+                                             ws.data_ptr(), ws.numel(), _cabi.stream_ptr()), "hgn_node_update_backward")
+    # node_update_backward_tc: node_bwd_tc and its reduction; per table a dgrad, a pair wgrad and one reduce_w0_block_kernel per aggregate
+    _count(2 + 2 * ((k + 1) // 2) + k)
+
+
+def _segment_sum(data, plan: SegmentPlan, out) -> None:
+    """``out[s] = sum of data's rows in segment s`` for the ``out.shape[0]`` segments of ``plan`` (bf16 rows of width 128)."""
+    S = out.shape[0]
+    _cabi.check(_cabi.load().hgn_segment_reduce(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(),
+                                                S, out.data_ptr(), None, None, None, None, None, 0, _cabi.stream_ptr()),
+                "hgn_segment_reduce")
+    _count(int(S > 0))          # segment_reduce_impl: one kernel
+
+
+def _segment_sum_pair(data, plan_a: SegmentPlan, out_a, plan_b: SegmentPlan, out_b) -> None:
+    """Two ``_segment_sum``s of the same rows under two groupings."""
+    S_a, S_b = out_a.shape[0], out_b.shape[0]
+    _cabi.check(_cabi.load().hgn_segment_sum_pair(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan_a.perm.data_ptr(),
+                                                  plan_a.rowptr.data_ptr(), S_a, out_a.data_ptr(), plan_b.perm.data_ptr(),
+                                                  plan_b.rowptr.data_ptr(), S_b, out_b.data_ptr(), _cabi.stream_ptr()),
+                "hgn_segment_sum_pair")
+    _count(1 if S_a > 0 and S_b > 0 else int(S_a > 0) + int(S_b > 0))   # hgn_segment_sum_pair: the paired kernel, else one sum per side
+
+
+def _rows_add(rows, index32, dst) -> None:
+    """``dst[index32[i]] += rows[i]`` (bf16; ``index32`` has no duplicates)."""
+    n = rows.shape[0]
+    _cabi.check(_cabi.load().hgn_rows_scatter(_BF, rows.data_ptr(), index32.data_ptr(), n, dst.shape[1], dst.data_ptr(), 1,
+                                              _cabi.stream_ptr()), "hgn_rows_scatter")
+    _count(int(n > 0))          # hgn_rows_scatter: one rows_scatter_kernel
+
+
 class _NodeProjection(torch.autograd.Function):
     """``Ps = v W0[:, 0:128]^T``, ``Pr = v W0[:, 128:256]^T`` -- the sender / receiver blocks of the edge MLP's first
     linear (graphnet.py:28-31 concatenation order), applied once per node instead of once per edge."""
 
     @staticmethod
     def forward(ctx, v, W0, packed):
-        lib = _cabi.load()
         n = v.shape[0]
         ps = torch.empty((n, D_LATENT), dtype=v.dtype, device=v.device)
         pr = torch.empty((n, D_LATENT), dtype=v.dtype, device=v.device)
         with torch.cuda.device(v.device):
-            _cabi.check(lib.hgn_edge_project_forward(_cabi.HGN_BF16, n, v.data_ptr(), packed.data_ptr(), ps.data_ptr(), pr.data_ptr(),
-                                                     _cabi.stream_ptr()), "hgn_edge_project_forward")
-        _count()
+            _edge_project_forward(v, packed, ps, pr)
         ctx.save_for_backward(v)
         ctx.packed = packed
         ctx.w0_shape = tuple(W0.shape)
@@ -320,20 +405,13 @@ class _NodeProjection(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gs, gr):
-        lib = _cabi.load()
         (v,) = ctx.saved_tensors
-        n = v.shape[0]
         gs = gs.contiguous() if gs is not None else torch.zeros_like(v)
         gr = gr.contiguous() if gr is not None else torch.zeros_like(v)
         grad_v = torch.empty_like(v)
         grad_w0 = torch.zeros(ctx.w0_shape, dtype=torch.float32, device=v.device)
         with torch.cuda.device(v.device):
-            ws_bytes = lib.hgn_edge_project_backward_workspace_bytes(_cabi.HGN_BF16, n)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=v.device)
-            _cabi.check(lib.hgn_edge_project_backward(_cabi.HGN_BF16, n, v.data_ptr(), ctx.packed.data_ptr(), gs.data_ptr(), gr.data_ptr(), None,
-                                                      grad_v.data_ptr(), grad_w0.data_ptr(), ws.data_ptr(), ws_bytes, _cabi.stream_ptr()),
-                        "hgn_edge_project_backward")
-        _count(4)
+            _edge_project_backward(v, ctx.packed, gs, gr, None, grad_v, grad_w0)
         return grad_v, grad_w0, None
 
 
@@ -344,21 +422,13 @@ class _EdgeUpdate(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, ps, pr, e, W0, b0, W1, b1, W2, b2, gamma, beta, packed, s_plan, r_plan, want_agg):
-        lib = _cabi.load()
-        E = e.shape[0]
         out = torch.empty_like(e)
         with torch.cuda.device(e.device):
-            _cabi.check(lib.hgn_edge_update_forward(_cabi.HGN_BF16, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(),
-                                                    r_plan.ids32.data_ptr(), packed.data_ptr(), out.data_ptr(), _cabi.stream_ptr()),
-                        "hgn_edge_update_forward")
-            _count()
+            _edge_update_forward(e, ps, pr, s_plan, r_plan, packed, out)
             agg = None
             if want_agg:
                 agg = torch.empty((r_plan.num_segments, D_LATENT), dtype=e.dtype, device=e.device)
-                _cabi.check(lib.hgn_segment_reduce(_cabi.HGN_BF16, out.data_ptr(), E, D_LATENT, r_plan.perm.data_ptr(), r_plan.rowptr.data_ptr(),
-                                                   r_plan.num_segments, agg.data_ptr(), None, None, None, None, None, 0, _cabi.stream_ptr()),
-                            "hgn_segment_reduce")
-                _count()
+                _segment_sum(out, r_plan, agg)
         ctx.save_for_backward(e, ps, pr)              # the hidden activations are recomputed by the backward kernel
         ctx.n_nodes = ps.shape[0]
         ctx.packed, ctx.s_plan, ctx.r_plan = packed, s_plan, r_plan
@@ -369,10 +439,8 @@ class _EdgeUpdate(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out, grad_agg):
-        lib = _cabi.load()
         e, ps, pr = ctx.saved_tensors
-        s_plan, r_plan = ctx.s_plan, ctx.r_plan
-        E, dev = e.shape[0], e.device
+        dev = e.device
         n = ctx.n_nodes
         if grad_out is not None:
             grad_out = grad_out.contiguous().to(e.dtype)
@@ -385,18 +453,9 @@ class _EdgeUpdate(torch.autograd.Function):
         gs = torch.empty((n, D_LATENT), dtype=e.dtype, device=dev)
         gr = torch.empty((n, D_LATENT), dtype=e.dtype, device=dev)
         with torch.cuda.device(dev):
-            ws_bytes = lib.hgn_edge_update_backward_workspace_bytes(_cabi.HGN_BF16, E)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            _cabi.check(lib.hgn_edge_update_backward(
-                _cabi.HGN_BF16, E, e.data_ptr(), _cabi.ptr(ps), _cabi.ptr(pr), s_plan.ids32.data_ptr(), r_plan.ids32.data_ptr(),
-                ctx.packed.data_ptr(), _cabi.ptr(grad_out), _cabi.ptr(grad_agg), grad_e.data_ptr(), g0.data_ptr(),
-                *[g.data_ptr() for g in gparams], ws.data_ptr(), ws_bytes, _cabi.stream_ptr()), "hgn_edge_update_backward")
-            _count(2)
+            _edge_update_backward(e, ps, pr, ctx.s_plan, ctx.r_plan, ctx.packed, grad_out, grad_agg, grad_e, g0, gparams)
             # d loss / d Ps, d Pr: sender- and receiver-keyed segment sums of G0 (deterministic CSR passes)
-            _cabi.check(lib.hgn_segment_sum_pair(_cabi.HGN_BF16, g0.data_ptr(), E, D_LATENT, s_plan.perm.data_ptr(), s_plan.rowptr.data_ptr(), n,
-                                                 gs.data_ptr(), r_plan.perm.data_ptr(), r_plan.rowptr.data_ptr(), n, gr.data_ptr(),
-                                                 _cabi.stream_ptr()), "hgn_segment_sum_pair")
-            _count()
+            _segment_sum_pair(g0, ctx.s_plan, gs, ctx.r_plan, gr)
         return (gs, gr, grad_e, *gparams, None, None, None, None)
 
 
@@ -424,17 +483,12 @@ class _NodeUpdate(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, v, W0, b0, W1, b1, W2, b2, gamma, beta, packed, *aggs):
-        lib = _cabi.load()
-        n, k = v.shape[0], len(aggs)
+        k = len(aggs)
         q1 = torch.empty_like(v)
         q2 = torch.empty_like(v) if k > 2 else None
         out = torch.empty_like(v)
-        agg_ptrs = (ctypes.c_void_p * k)(*[a.data_ptr() for a in aggs])
         with torch.cuda.device(v.device):
-            _cabi.check(lib.hgn_node_update_forward(_cabi.HGN_BF16, n, v.data_ptr(), k, agg_ptrs, packed.data_ptr(), q1.data_ptr(),
-                                                    _cabi.ptr(q2), out.data_ptr(), _cabi.stream_ptr()),
-                        "hgn_node_update_forward")
-        _count(1 + (k + 1) // 2)
+            _node_update_forward(v, aggs, packed, q1, q2, out)
         ctx.save_for_backward(v, *aggs, q1, *([q2] if q2 is not None else []))
         ctx.k = k
         ctx.packed = packed
@@ -443,27 +497,18 @@ class _NodeUpdate(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _cabi.load()
         saved = list(ctx.saved_tensors)
         k = ctx.k
         v, aggs, rest = saved[0], saved[1:1 + k], saved[1 + k:]
         q1 = rest[0]
         q2 = rest[1] if len(rest) > 1 else None
-        n, dev = v.shape[0], v.device
+        dev = v.device
         grad_out = grad_out.contiguous().to(v.dtype)
         grad_v = torch.empty_like(v)
         grad_aggs = [torch.empty_like(a) for a in aggs]
         gparams = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes]
-        agg_ptrs = (ctypes.c_void_p * k)(*[a.data_ptr() for a in aggs])
-        gagg_ptrs = (ctypes.c_void_p * k)(*[g.data_ptr() for g in grad_aggs])
         with torch.cuda.device(dev):
-            ws_bytes = lib.hgn_node_update_backward_workspace_bytes(_cabi.HGN_BF16, n)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            _cabi.check(lib.hgn_node_update_backward(
-                _cabi.HGN_BF16, n, v.data_ptr(), k, agg_ptrs, _cabi.ptr(q1), _cabi.ptr(q2),
-                ctx.packed.data_ptr(), grad_out.data_ptr(), grad_v.data_ptr(), gagg_ptrs, *[g.data_ptr() for g in gparams],
-                ws.data_ptr(), ws_bytes, _cabi.stream_ptr()), "hgn_node_update_backward")
-        _count(2 + 3 * ((k + 1) // 2))
+            _node_update_backward(v, aggs, q1, q2, ctx.packed, grad_out, grad_v, grad_aggs, gparams)
         return (grad_v, *gparams, None, *grad_aggs)
 
 
@@ -487,6 +532,15 @@ def node_update(params: Sequence[torch.Tensor], packed_cache: dict, v: torch.Ten
     return _NodeUpdate.apply(v, *params, packed, *aggs)
 
 
+def _layer_workspace(n: int, E: int, device) -> torch.Tensor:
+    """One workspace for the backward entry points of a layer of ``n`` nodes and ``E`` edges (they run one after another on one
+    stream)."""
+    lib = _cabi.load()
+    nbytes = max(lib.hgn_node_update_backward_workspace_bytes(_BF, n), lib.hgn_edge_update_backward_workspace_bytes(_BF, E),
+                 lib.hgn_edge_project_backward_workspace_bytes(_BF, n))
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
+
+
 class _GraphNetSumLayer(torch.autograd.Function):
     """One whole ``GraphNet`` block with the 'sum' aggregator and ONE edge set (graphnet.py:72-84) as a single autograd node:
 
@@ -496,68 +550,59 @@ class _GraphNetSumLayer(torch.autograd.Function):
 
     Same kernels and same arithmetic as ``edge_update`` + ``node_update``; what goes away is the autograd glue between them: the
     ``at::add`` of the two partial gradients of ``v`` ([N,128] read twice and written once per layer), zero fills, and four autograd
-    nodes' worth of Python per layer."""
+    nodes' worth of Python per layer.
+
+    ``halo`` (not a tensor: passed through untouched, like the plans) makes this the block of one rank of a partitioned graph
+    (``partition.PeerLayerHalo``).  ``v`` then holds the owned nodes, and the senders index ``[owned | ghosts]``.  The halo provides
+    the sender table ``Ps`` (``[n_own + n_ghost, 128]``; this rank writes the owned rows), a forward exchange that fills the ghost
+    rows after the projection, and a backward exchange that sends the ghost rows of the sender sums home and adds the rows the peers
+    return into the owned ones.  Everything else is this schedule, so an owned row sees the kernels and the rounding points of the
+    one-GPU layer."""
 
     @staticmethod
-    def forward(ctx, v, e, s_plan, r_plan, packed_e, packed_n, *params):
-        lib, BF = _cabi.load(), _cabi.HGN_BF16
-        n, E = v.shape[0], e.shape[0]
-        ps, pr, q1 = torch.empty_like(v), torch.empty_like(v), torch.empty_like(v)
+    def forward(ctx, v, e, s_plan, r_plan, packed_e, packed_n, halo, *params):
+        ps = halo.sender_table() if halo is not None else torch.empty_like(v)
+        pr, q1 = torch.empty_like(v), torch.empty_like(v)
         e_new, v_new, agg = torch.empty_like(e), torch.empty_like(v), torch.empty_like(v)
         with torch.cuda.device(v.device):
-            st = _cabi.stream_ptr()
-            _cabi.check(lib.hgn_edge_project_forward(BF, n, v.data_ptr(), packed_e.data_ptr(), ps.data_ptr(), pr.data_ptr(), st), "hgn_edge_project_forward")
-            _cabi.check(lib.hgn_edge_update_forward(BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(), r_plan.ids32.data_ptr(),
-                                                    packed_e.data_ptr(), e_new.data_ptr(), st), "hgn_edge_update_forward")
-            _cabi.check(lib.hgn_segment_reduce(BF, e_new.data_ptr(), E, D_LATENT, r_plan.perm.data_ptr(), r_plan.rowptr.data_ptr(), n, agg.data_ptr(),
-                                               None, None, None, None, None, 0, st), "hgn_segment_reduce")
-            agg_ptrs = (ctypes.c_void_p * 1)(agg.data_ptr())
-            _cabi.check(lib.hgn_node_update_forward(BF, n, v.data_ptr(), 1, agg_ptrs, packed_n.data_ptr(), q1.data_ptr(), None, v_new.data_ptr(), st),
-                        "hgn_node_update_forward")
-        _count(5)
+            _edge_project_forward(v, packed_e, ps, pr)
+            if halo is not None:
+                halo.exchange_forward()
+            _edge_update_forward(e, ps, pr, s_plan, r_plan, packed_e, e_new)
+            _segment_sum(e_new, r_plan, agg)
+            _node_update_forward(v, [agg], packed_n, q1, None, v_new)
         ctx.save_for_backward(v, e, ps, pr, agg, q1)
-        ctx.plans, ctx.packed = (s_plan, r_plan), (packed_e, packed_n)
+        ctx.plans, ctx.packed, ctx.halo = (s_plan, r_plan), (packed_e, packed_n), halo
         ctx.param_shapes = [tuple(p.shape) for p in params]
         return v_new, e_new
 
     @staticmethod
     def backward(ctx, grad_v_new, grad_e_new):
-        lib, BF = _cabi.load(), _cabi.HGN_BF16
         v, e, ps, pr, agg, q1 = ctx.saved_tensors
         s_plan, r_plan = ctx.plans
         packed_e, packed_n = ctx.packed
-        n, E, dev = v.shape[0], e.shape[0], v.device
+        dev = v.device
         grad_v_new = grad_v_new.contiguous().to(v.dtype) if grad_v_new is not None else torch.zeros_like(v)
         grad_e_new = grad_e_new.contiguous().to(e.dtype) if grad_e_new is not None else None
         new = lambda like: torch.empty_like(like)
-        grad_v_node, grad_agg, grad_v, gs, gr = new(v), new(v), new(v), new(v), new(v)
+        grad_v_node, grad_agg, grad_v, gs, gr = new(v), new(v), new(v), new(ps), new(v)
         grad_e, g0 = new(e), new(e)
         ge = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[:8]]
         gn = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[8:]]
         with torch.cuda.device(dev):
-            st = _cabi.stream_ptr()
-            agg_ptrs = (ctypes.c_void_p * 1)(agg.data_ptr())
-            gagg_ptrs = (ctypes.c_void_p * 1)(grad_agg.data_ptr())
-            ws_bytes = max(lib.hgn_node_update_backward_workspace_bytes(BF, n), lib.hgn_edge_update_backward_workspace_bytes(BF, E),
-                           lib.hgn_edge_project_backward_workspace_bytes(BF, n))
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            _cabi.check(lib.hgn_node_update_backward(BF, n, v.data_ptr(), 1, agg_ptrs, q1.data_ptr(), None, packed_n.data_ptr(), grad_v_new.data_ptr(),
-                                                     grad_v_node.data_ptr(), gagg_ptrs, *[g.data_ptr() for g in gn], ws.data_ptr(), ws_bytes, st),
-                        "hgn_node_update_backward")
-            _cabi.check(lib.hgn_edge_update_backward(BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(), r_plan.ids32.data_ptr(),
-                                                     packed_e.data_ptr(), _cabi.ptr(grad_e_new), grad_agg.data_ptr(), grad_e.data_ptr(), g0.data_ptr(),
-                                                     *[g.data_ptr() for g in ge], ws.data_ptr(), ws_bytes, st), "hgn_edge_update_backward")
-            _cabi.check(lib.hgn_segment_sum_pair(BF, g0.data_ptr(), E, D_LATENT, s_plan.perm.data_ptr(), s_plan.rowptr.data_ptr(), n, gs.data_ptr(),
-                                                 r_plan.perm.data_ptr(), r_plan.rowptr.data_ptr(), n, gr.data_ptr(), st), "hgn_segment_sum_pair")
+            ws = _layer_workspace(v.shape[0], e.shape[0], dev)
+            _node_update_backward(v, [agg], q1, None, packed_n, grad_v_new, grad_v_node, [grad_agg], gn, ws)
+            _edge_update_backward(e, ps, pr, s_plan, r_plan, packed_e, grad_e_new, grad_agg, grad_e, g0, ge, ws)
+            _segment_sum_pair(g0, s_plan, gs, r_plan, gr)
+            if ctx.halo is not None:
+                ctx.halo.exchange_backward(gs)
             # the edge backward wrote only the We block of d W0 (columns 256:384); the node-level kernel fills columns 0:256
-            _cabi.check(lib.hgn_edge_project_backward(BF, n, v.data_ptr(), packed_e.data_ptr(), gs.data_ptr(), gr.data_ptr(), grad_v_node.data_ptr(),
-                                                      grad_v.data_ptr(), ge[0].data_ptr(), ws.data_ptr(), ws_bytes, st), "hgn_edge_project_backward")
-        _count(5 + 2 + 1 + 4)
-        return (grad_v, grad_e, None, None, None, None, *ge, *gn)
+            _edge_project_backward(v, packed_e, gs, gr, grad_v_node, grad_v, ge[0], ws)
+        return (grad_v, grad_e, None, None, None, None, None, *ge, *gn)
 
 
 def graphnet_sum_layer(edge_params: Sequence[torch.Tensor], edge_cache: dict, node_params: Sequence[torch.Tensor], node_cache: dict,
-                       v: torch.Tensor, e: torch.Tensor, s_plan: SegmentPlan, r_plan: SegmentPlan):
+                       v: torch.Tensor, e: torch.Tensor, s_plan: SegmentPlan, r_plan: SegmentPlan, halo=None):
     """``(v', e')`` of one GraphNet block ('sum', one edge set, bf16 latents of width 128): see ``_GraphNetSumLayer``."""
     _cabi.require_cuda(v, e)
     if v.dtype != torch.bfloat16 or e.dtype != torch.bfloat16 or v.shape[-1] != D_LATENT or e.shape[-1] != D_LATENT:
@@ -568,7 +613,7 @@ def graphnet_sum_layer(edge_params: Sequence[torch.Tensor], edge_cache: dict, no
     with torch.cuda.device(v.device):
         packed_e = _pack_weights(edge_cache, torch.bfloat16, 3, edge_params)
         packed_n = _pack_weights(node_cache, torch.bfloat16, 2, node_params)
-    return _GraphNetSumLayer.apply(v, e, s_plan, r_plan, packed_e, packed_n, *edge_params, *node_params)
+    return _GraphNetSumLayer.apply(v, e, s_plan, r_plan, packed_e, packed_n, halo, *edge_params, *node_params)
 
 
 def colsum(x: torch.Tensor) -> torch.Tensor:

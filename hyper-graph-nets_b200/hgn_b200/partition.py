@@ -21,12 +21,12 @@ Nothing here does arithmetic on latents besides the pack / scatter-add row kerne
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import List, NamedTuple, Optional, Sequence
 
 import torch
 import torch.distributed as dist
 
-from . import _cabi
+from . import _cabi, ops
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -320,7 +320,8 @@ class PeerHalo:
 
     def push_backward(self, step: int, layer: int, gs: torch.Tensor) -> None:
         """Ghost rows of ``gs`` (sender-keyed sums of G0, ``[n_own + n_ghost, width]``) -> their owners' inboxes; then wait for the
-        rows the peers return to this rank."""
+        rows the peers return to this rank and add them into the owned rows of ``gs``, peer by peer in rank order (a fixed summation
+        order)."""
         lib = _cabi.load()
         epoch = self._epoch(step, layer, True)
         peers, flags = _cabi.HaloPeers(), _cabi.HaloFlags()
@@ -341,6 +342,13 @@ class PeerHalo:
                 n_wait += 1
         peers.row_begin[n_push] = lo
         self._run(lib, gs, self.ghost_index32, peers, n_push, flags, n_wait, epoch, compact=False)
+        inbox = self.inbox(layer)
+        lo = 0
+        for q in range(self.world):
+            n = self.lg.send_splits[q]
+            if n and q != self.rank:
+                ops._rows_add(inbox[lo:lo + n], self.send_index32[lo:lo + n], gs)
+            lo += n
 
     def _run(self, lib, table, index32, peers, n_push, flags, n_wait, epoch, compact):
         import ctypes
@@ -351,96 +359,23 @@ class PeerHalo:
             _cabi.check(lib.hgn_halo_push(_cabi.HGN_BF16, table.data_ptr(), index32.data_ptr(), self.width, ctypes.byref(peers), n_push, epoch,
                                           self.base + self.off_counter, st), "hgn_halo_push")
             _cabi.check(lib.hgn_halo_wait(ctypes.byref(flags), n_wait, epoch, st), "hgn_halo_wait")
+        ops._count(int(n_push > 0) + int(n_wait > 0))     # csrc/peer.cu: each entry point launches one kernel, none without peers
 
 
-class _PeerGraphNetLayer(torch.autograd.Function):
-    """One whole partitioned ``GraphNet`` block ('sum', one edge set, bf16) with the halo in peer memory, as a single autograd node --
-    the partitioned twin of ``ops._GraphNetSumLayer``.  Forward: project the owned rows into this layer's table, push the boundary
-    rows of ``Ps`` to the peers and wait for theirs, fused edge kernel over all local edges, receiver aggregate, projected node update: the same kernels in the same order on the owned
-    rows, so an owned row sees the arithmetic (and the rounding points) of the single-GPU layer; the only difference is where the
-    ghost rows of ``Ps`` come from and that the ghost rows of the sender sums are added at their owners.  Backward: node backward ->
-    edge backward -> sender / receiver sums of G0 -> ghost sums go home -> node-level dgrad with the node update's share of
-    d loss / d v added in its epilogue -> node-level wgrads.  No ``at::`` kernel between its launches."""
+class PeerLayerHalo(NamedTuple):
+    """The halo of one (step, layer) of a ``PeerHalo``, in the form ``ops.graphnet_sum_layer`` takes it."""
+    peer: PeerHalo
+    step: int
+    layer: int
 
-    @staticmethod
-    def forward(ctx, owned, e, packed_e, packed_n, halo: PeerHalo, step: int, layer: int, *params):
-        import ctypes
-        lib, BF = _cabi.load(), _cabi.HGN_BF16
-        No, E = halo.n_own, e.shape[0]
-        owned, e = owned.contiguous(), e.contiguous()
-        ps = halo.table(step & 1, layer)
-        pr, q1, agg, v_new = (torch.empty((No, owned.shape[1]), dtype=owned.dtype, device=owned.device) for _ in range(4))
-        out = torch.empty_like(e)
-        s32, r32 = halo.s_plan.ids32, halo.r_plan.ids32
-        with torch.cuda.device(owned.device):
-            st = _cabi.stream_ptr()
-            _cabi.check(lib.hgn_edge_project_forward(BF, No, owned.data_ptr(), packed_e.data_ptr(), ps.data_ptr(), pr.data_ptr(), st),
-                        "hgn_edge_project_forward")
-            halo.push_forward(step, layer)
-            _cabi.check(lib.hgn_edge_update_forward(BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s32.data_ptr(), r32.data_ptr(),
-                                                    packed_e.data_ptr(), out.data_ptr(), st), "hgn_edge_update_forward")
-            _cabi.check(lib.hgn_segment_reduce(BF, out.data_ptr(), E, owned.shape[1], halo.r_plan.perm.data_ptr(), halo.r_plan.rowptr.data_ptr(), No,
-                                               agg.data_ptr(), None, None, None, None, None, 0, st), "hgn_segment_reduce")
-            agg_ptrs = (ctypes.c_void_p * 1)(agg.data_ptr())
-            _cabi.check(lib.hgn_node_update_forward(BF, No, owned.data_ptr(), 1, agg_ptrs, packed_n.data_ptr(), q1.data_ptr(), None, v_new.data_ptr(), st),
-                        "hgn_node_update_forward")
-        from . import ops as _ops
-        _ops._count(7)
-        ctx.save_for_backward(owned, e, pr, agg, q1)
-        ctx.halo, ctx.packed, ctx.step, ctx.layer = halo, (packed_e, packed_n), step, layer
-        ctx.param_shapes = [tuple(p.shape) for p in params]
-        return v_new, out
+    def sender_table(self) -> torch.Tensor:
+        return self.peer.table(self.step & 1, self.layer)
 
-    @staticmethod
-    def backward(ctx, grad_v_new, grad_e_new):
-        import ctypes
-        lib, BF, halo = _cabi.load(), _cabi.HGN_BF16, ctx.halo
-        owned, e, pr, agg, q1 = ctx.saved_tensors
-        packed_e, packed_n = ctx.packed
-        step, layer = ctx.step, ctx.layer
-        ps = halo.table(step & 1, layer)                     # still this step's rows: see PeerHalo
-        No, G, E = halo.n_own, halo.n_ghost, e.shape[0]
-        D, dev = owned.shape[1], owned.device
-        s_plan, r_plan = halo.s_plan, halo.r_plan
-        grad_v_new = grad_v_new.contiguous().to(owned.dtype) if grad_v_new is not None else torch.zeros_like(owned)
-        grad_e_new = grad_e_new.contiguous().to(e.dtype) if grad_e_new is not None else None
-        grad_e, g0 = torch.empty_like(e), torch.empty_like(e)
-        ge = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[:8]]
-        gn = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[8:]]
-        gs = torch.empty((No + G, D), dtype=e.dtype, device=dev)
-        gr, grad_owned, grad_v_node, grad_agg = (torch.empty((No, D), dtype=e.dtype, device=dev) for _ in range(4))
-        with torch.cuda.device(dev):
-            st = _cabi.stream_ptr()
-            ws_bytes = max(lib.hgn_node_update_backward_workspace_bytes(BF, No), lib.hgn_edge_update_backward_workspace_bytes(BF, E),
-                           lib.hgn_edge_project_backward_workspace_bytes(BF, No))
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            agg_ptrs = (ctypes.c_void_p * 1)(agg.data_ptr())
-            gagg_ptrs = (ctypes.c_void_p * 1)(grad_agg.data_ptr())
-            _cabi.check(lib.hgn_node_update_backward(BF, No, owned.data_ptr(), 1, agg_ptrs, q1.data_ptr(), None, packed_n.data_ptr(), grad_v_new.data_ptr(),
-                                                     grad_v_node.data_ptr(), gagg_ptrs, *[g.data_ptr() for g in gn], ws.data_ptr(), ws_bytes, st),
-                        "hgn_node_update_backward")
-            _cabi.check(lib.hgn_edge_update_backward(
-                BF, E, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), s_plan.ids32.data_ptr(), r_plan.ids32.data_ptr(), packed_e.data_ptr(),
-                _cabi.ptr(grad_e_new), grad_agg.data_ptr(), grad_e.data_ptr(), g0.data_ptr(), *[g.data_ptr() for g in ge], ws.data_ptr(),
-                ws_bytes, st), "hgn_edge_update_backward")
-            _cabi.check(lib.hgn_segment_sum_pair(BF, g0.data_ptr(), E, D, s_plan.perm.data_ptr(), s_plan.rowptr.data_ptr(), No + G, gs.data_ptr(),
-                                                 r_plan.perm.data_ptr(), r_plan.rowptr.data_ptr(), No, gr.data_ptr(), st), "hgn_segment_sum_pair")
-            halo.push_backward(step, layer, gs)              # ghost rows of gs go home; the rows of this rank's boundary nodes arrive
-            inbox = halo.inbox(layer)
-            lo = 0
-            for q in range(halo.world):                      # peers in rank order: a fixed summation order
-                n = halo.lg.send_splits[q]
-                if n and q != halo.rank:
-                    _cabi.check(lib.hgn_rows_scatter(BF, inbox[lo:lo + n].data_ptr(), halo.send_index32[lo:lo + n].data_ptr(), n, D, gs.data_ptr(), 1, st),
-                                "hgn_rows_scatter")
-                lo += n
-            # the edge backward wrote only the We block of d W0 (columns 256:384); the node-level kernel fills columns 0:256
-            _cabi.check(lib.hgn_edge_project_backward(BF, No, owned.data_ptr(), packed_e.data_ptr(), gs.data_ptr(), gr.data_ptr(), grad_v_node.data_ptr(),
-                                                      grad_owned.data_ptr(), ge[0].data_ptr(), ws.data_ptr(), ws_bytes, st),
-                        "hgn_edge_project_backward")
-        from . import ops as _ops
-        _ops._count(5 + 11)
-        return (grad_owned, grad_e, None, None, None, None, None, *ge, *gn)
+    def exchange_forward(self) -> None:
+        self.peer.push_forward(self.step, self.layer)
+
+    def exchange_backward(self, gs: torch.Tensor) -> None:
+        self.peer.push_backward(self.step, self.layer, gs)
 
 
 class PartitionedProcessor(torch.nn.Module):
@@ -448,8 +383,9 @@ class PartitionedProcessor(torch.nn.Module):
 
     Generic path (any block type, any aggregator, fp32 or bf16): ghosts are refreshed before every block with a grouped NCCL
     send/recv; the block itself is unchanged (it sees ``[owned | ghosts]`` as ``[mesh | hyper]`` rows).
-    Fast path (``PeerHalo`` given; bf16, plain ``GraphNet`` blocks, 'sum', one edge set -- the cfg5 benchmark): ``_PeerGraphNetLayer``
-    per block -- halo rows travel as peer-memory stores issued by a kernel of the sending rank -- then the projected node update."""
+    Fast path (``PeerHalo`` given, and every block takes the whole-layer route of ``GraphNet`` -- the cfg5 benchmark):
+    ``ops.graphnet_sum_layer`` per block with the halo of that layer; halo rows travel as peer-memory stores issued by a kernel of
+    the sending rank."""
 
     def __init__(self, processor: torch.nn.Module, plan: HaloPlan, peer: Optional[PeerHalo] = None):
         super().__init__()
@@ -464,11 +400,10 @@ class PartitionedProcessor(torch.nn.Module):
             peer.r_plan = segment_plan(peer.receivers, lg.n_own)
 
     def _fast_path(self, owned, edge_sets) -> bool:
-        from .migration.graphnet import GraphNet
+        from .migration.graphnet import takes_whole_layer
         blocks = self.processor.graphnet_blocks
-        return (self.peer is not None and owned.is_cuda and len(edge_sets) == 1 and len(blocks) == self.peer.layers
-                and all(type(b) is GraphNet and b.message_passing_aggregator == "sum"
-                        and list(b.edge_models.keys()) == [edge_sets[0].name] for b in blocks))
+        return (self.peer is not None and len(blocks) == self.peer.layers
+                and all(takes_whole_layer(b, owned, edge_sets) for b in blocks))
 
     def forward(self, owned: torch.Tensor, edge_sets):
         from . import config
@@ -479,20 +414,12 @@ class PartitionedProcessor(torch.nn.Module):
             owned = owned.to(torch.bfloat16)
             edge_sets = [es._replace(features=es.features.to(torch.bfloat16)) for es in edge_sets]
         if precision == "bf16" and self._fast_path(owned, edge_sets):
-            from . import ops as _ops
-            from .migration.graphnet import _mlp_parameters, _packed_cache
             es = edge_sets[0]
             e = es.features
             step = self.peer.steps_done
             self.peer.steps_done += 1
             for layer, block in enumerate(self.processor.graphnet_blocks):
-                edge_model = block.edge_models[es.name]
-                ep = _mlp_parameters(edge_model, 3 * owned.shape[1], owned)
-                np_ = _mlp_parameters(block.node_model_cross, 2 * owned.shape[1], owned)
-                with torch.cuda.device(owned.device):
-                    packed_e = _ops._pack_weights(_packed_cache(edge_model), torch.bfloat16, 3, ep)
-                    packed_n = _ops._pack_weights(_packed_cache(block.node_model_cross), torch.bfloat16, 2, np_)
-                owned, e = _PeerGraphNetLayer.apply(owned, e, packed_e, packed_n, self.peer, step, layer, *ep, *np_)
+                owned, e = block._sum_layer(owned, e, es.name, self.peer.s_plan, self.peer.r_plan, PeerLayerHalo(self.peer, step, layer))
             return owned.to(in_dtype), [es._replace(features=e)]
         graph = MultiGraph([owned, None], list(edge_sets))
         for block in self.processor.graphnet_blocks:

@@ -58,7 +58,7 @@ def rel(x, y):
     return float((x.double() - y.double()).norm() / y.double().norm().clamp_min(1e-30))
 
 
-assert fast._fast_path(v0.to(torch.bfloat16), [EdgeSet("mesh_edges", e0, s_loc, r_loc)])
+assert fast._fast_path(v0.to(torch.bfloat16), [EdgeSet("mesh_edges", e0.to(torch.bfloat16), s_loc, r_loc)])
 worst_paths = worst_single = 0.0
 for step in range(3):
     shift = 0.01 * step
