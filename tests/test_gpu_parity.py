@@ -280,10 +280,14 @@ def test_rows_gather_scatter_and_colsum():
 
 
 def _bf16_emulated_mlp(x, w):
-    """torch fp32 arithmetic on bf16-rounded operands, rounding H1/H2 where the kernel does."""
+    """torch fp32 arithmetic on bf16-rounded operands, rounding H1/H2 where the kernel does.  ``x``: the [rows, 128 n] input, or
+    the list of its n 128-wide chunks (no concatenated copy: the multi-slab case is 2 M rows)."""
     W0, b0, W1, b1, W2, b2, g, b = w
     r = lambda t: t.to(torch.bfloat16).float()
-    h = torch.relu(x @ r(W0).t() + b0)
+    if isinstance(x, (list, tuple)):
+        h = torch.relu(sum(c @ r(W0[:, 128 * i: 128 * (i + 1)]).t() for i, c in enumerate(x)) + b0)
+    else:
+        h = torch.relu(x @ r(W0).t() + b0)
     h = torch.relu(r(h) @ r(W1).t() + b1)
     return torch.nn.functional.layer_norm(r(h) @ r(W2).t() + b2, (128,), g, b, 1e-5)
 
@@ -314,14 +318,132 @@ def test_bf16_kernels_vs_bf16_emulation(rows, n_nodes):
         assert rel_l2(a.grad, b.grad) < 1e-2
 
 
+def _mlp_params(w):
+    """The eight parameters of ``_random_mlp_weights`` on the GPU, in the kernels' order, as leaves."""
+    params = [w[f"m.0.layers.linear_{k}.{p}"].cuda().requires_grad_(True) for k in range(3) for p in ("weight", "bias")]
+    return params + [w["m.1.weight"].cuda().requires_grad_(True), w["m.1.bias"].cuda().requires_grad_(True)]
+
+
+def _row_windows(rows, extra=None):
+    """Row windows of a tensor of more than one 128-row tile, where a persistent tile kernel goes wrong first: the first tile, the last
+    (partial) tile, and the 128 rows around the first wrap of the grid (one CTA per SM: CTA 0 takes its second tile at row SMs x 128).
+    A defect confined to a window moves a global relative L2 by only about sqrt(window / rows)."""
+    if rows <= 128:
+        return {}
+    wins = {"first tile": (0, 128), "last tile": ((rows - 1) // 128 * 128, rows)}
+    wrap = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count * 128
+    if wrap < rows:
+        wins["grid wrap"] = (wrap - 64, min(wrap + 64, rows))
+    wins.update(extra or {})
+    return wins
+
+
+def _row_errs(got, want, metric, extra_windows=None):
+    """(global error under ``metric``, worst relative L2 over the row windows; 0 for a single tile)."""
+    wins = _row_windows(got.shape[0], extra_windows).values()
+    return metric(got, want), max((rel_l2(got[lo:hi], want[lo:hi]) for lo, hi in wins), default=0.0, key=_nan_last)
+
+
+def _param_errs(got, want, names):
+    """(worst relative L2 over the parameter gradients, its name).  A parameter the reference's loss does not reach has gradient None
+    there: the kernels must then give exact zeros."""
+    return max(((rel_l2(a.grad, b.grad if b.grad is not None else torch.zeros_like(b)), n) for a, b, n in zip(got, want, names)),
+               key=lambda t: _nan_last(t[0]))
+
+
+def _nan_last(x):
+    """Sort key under which NaN (e.g. a never-written output) is the worst error."""
+    return (x != x, x)
+
+
+def _report(tag, checks):
+    """Print every figure of ``checks`` (name -> (global, worst window, bound)), then assert them all (NaN fails)."""
+    print(f"\n{tag}: " + ", ".join(f"{k} {g:.2e}" + (f" / windows {win:.2e}" if win else "") for k, (g, win, _) in checks.items()))
+    bad = [k for k, (g, win, bound) in checks.items() if not (g < bound and win < bound)]
+    assert not bad, f"{tag}: beyond the bound: {bad}"
+
+
+_MLP_NAMES = [f"linear_{k}.{p}" for k in range(3) for p in ("weight", "bias")] + ["ln.weight", "ln.bias"]
+
+
+def _node_update_tile_kernel_vs_emulation(n_chunks, target, n_mesh, n_hyper, agg_grad, extra_windows=None):
+    """ops.fused_mlp called the way GraphNet._fused_node_update calls it when the projected node kernels do not apply (more than four
+    aggregates): sources [v_stacked] + aggregates, each of n_mesh + n_hyper rows, every chunk dense at the target's row offset, the
+    residual read from v_stacked at that offset.  Above kMaxResidentChunks = 3 chunks the tile kernels stream W0 instead of keeping it
+    in shared memory.  Against _bf16_emulated_mlp on the same rows."""
+    torch.manual_seed(1000 * n_chunks + n_mesh + n_hyper + (target == "hyper"))
+    offset, rows = (0, n_mesh) if target == "mesh" else (n_mesh, n_hyper)
+    params = _mlp_params(_random_mlp_weights(n_chunks, 9))
+    srcs = [torch.randn(n_mesh + n_hyper, 128, device="cuda").to(torch.bfloat16).requires_grad_(c == 0 or agg_grad) for c in range(n_chunks)]
+    gup = torch.randn(rows, 128, device="cuda").to(torch.bfloat16)
+    # Kernel and emulation round H1 to bf16 from fp32 sums taken in different orders; where that moves a hidden pre-activation across
+    # zero, the row's ReLU mask differs and so does its whole gradient (measured: one row in 200, 20 % off, a unit 1.4e-4 sigma from
+    # zero).  Rows with a unit that close to the edge get no upstream gradient: every gradient is linear in it, so both sides give
+    # exactly zero there, and the forward is still compared on every row.
+    edge = _relu_edge_rows([t.detach()[offset: offset + rows] for t in srcs], params)
+    gup[edge] = 0
+    out = ops.fused_mlp(params, {}, srcs, [ops.ChunkSpec(c, None, offset) for c in range(n_chunks)], rows, resid_source=0, resid_offset=offset)
+    out.backward(gup)
+    out, grads = out.detach(), [t.grad for t in srcs]
+    sf = [t.detach()[offset: offset + rows].float().requires_grad_(True) for t in srcs]
+    del srcs
+    wr = [p.detach().clone().requires_grad_(True) for p in params]
+    ref = sf[0] + _bf16_emulated_mlp(sf, wr)
+    ref.backward(gup.float())
+    checks = {"out": (*_row_errs(out.float(), ref.detach(), rel_err, extra_windows), 1e-2)}
+    for c, (g, f) in enumerate(zip(grads, sf)):
+        if not agg_grad and c > 0:
+            assert g is None
+            continue
+        # the grad_chunk rows outside [offset, offset + rows) belong to the other node type: nothing may be written there
+        assert int(torch.count_nonzero(g[:offset])) == 0 and int(torch.count_nonzero(g[offset + rows:])) == 0, f"source {c}"
+        checks[f"grad src{c}"] = (*_row_errs(g[offset: offset + rows].float(), f.grad, rel_l2, extra_windows), 1e-2 if c == 0 else 1.5e-2)
+    err, name = _param_errs(params, wr, _MLP_NAMES)
+    checks[f"weights (worst {name})"] = (err, 0.0, 1.5e-2)
+    _report(f"tile kernel, {n_chunks} chunks, {target} rows {rows} at offset {offset} ({int(edge.sum())} rows on a ReLU edge)", checks)
+
+
+def _relu_edge_rows(chunks, w, rel=3e-4):
+    """Rows of the emulated MLP whose hidden pre-activations (either layer) include one within ``rel`` x that layer's std of zero."""
+    W0, b0, W1, b1 = (p.detach() for p in w[:4])
+    rd = lambda t: t.to(torch.bfloat16).float()
+    with torch.no_grad():
+        pre1 = sum(c.float() @ rd(W0[:, 128 * i: 128 * (i + 1)]).t() for i, c in enumerate(chunks)) + b0
+        edge = (pre1.abs() < rel * pre1.std()).any(1)
+        pre2 = rd(torch.relu(pre1)) @ rd(W1).t() + b1
+        return edge | (pre2.abs() < rel * pre2.std()).any(1)
+
+
+# (n_chunks, target, mesh rows, hyper rows, aggregates need grad): 4 = first streamed-W0 count, 5 / 13 leave a partial group of the
+# W0 weight gradient (three chunks per group), 6 = 'sum' over five edge sets, 9 = hyper 'pna' over two inter sets, 21 = hetero 'pna' over
+# five sets, 24 = HGN_MAX_CHUNKS.  The last two leave the aggregates' grad_chunk entries NULL.
+_NODE_UPDATE_LAYOUTS = [(k, t, n, c, True) for k in (4, 5, 6, 9, 13, 21, 24) for t in ("mesh", "hyper") for n, c in ((1600, 16), (40000, 200))]
+_NODE_UPDATE_LAYOUTS += [(9, "hyper", 1600, 16, False), (21, "mesh", 40000, 200, False)]
+
+
+@pytest.mark.parametrize("n_chunks,target,n_mesh,n_hyper,agg_grad", _NODE_UPDATE_LAYOUTS)
+def test_tile_kernel_node_update_layouts_vs_bf16_emulation(n_chunks, target, n_mesh, n_hyper, agg_grad):
+    """The layouts the bf16 models send the generic tile kernels (node updates with more than four aggregates) against torch arithmetic
+    with the same rounding points: output, the gradient of every source, every parameter gradient; the source gradients stay zero
+    outside the target's rows."""
+    _node_update_tile_kernel_vs_emulation(n_chunks, target, n_mesh, n_hyper, agg_grad)
+
+
 def _bf16_emulated_projected_edge(v, e, s, r, w):
     """torch fp32 arithmetic with the rounding points of the projected edge kernels (csrc/edge_tc.cu): bf16 operands,
     bf16 per-node projection tables, bf16 H1/H2."""
+    rd = lambda t: t.to(torch.bfloat16).float()
+    ps = rd(v @ rd(w[0][:, :128]).t())
+    pr = rd(v @ rd(w[0][:, 128:256]).t())
+    return _bf16_emulated_edge_from_table_rows(ps[s], pr[r], e, w)
+
+
+def _bf16_emulated_edge_from_table_rows(ps_s, pr_r, e, w):
+    """The edge kernels' arithmetic after the gathers: ``ps_s`` / ``pr_r`` are the table rows ``Ps[s]`` / ``Pr[r]``, so the gradient of
+    either is d loss / d (first-layer pre-activation), the kernel's grad_pre0."""
     W0, b0, W1, b1, W2, b2, g, b = w
     rd = lambda t: t.to(torch.bfloat16).float()
-    ps = rd(v @ rd(W0[:, :128]).t())
-    pr = rd(v @ rd(W0[:, 128:256]).t())
-    h = torch.relu(ps[s] + pr[r] + e @ rd(W0[:, 256:]).t() + b0)
+    h = torch.relu(ps_s + pr_r + e @ rd(W0[:, 256:]).t() + b0)
     h = torch.relu(rd(h) @ rd(W1).t() + b1)
     return e + torch.nn.functional.layer_norm(rd(h) @ rd(W2).t() + b2, (128,), g, b, 1e-5)
 
@@ -409,6 +531,134 @@ def test_projected_node_update_vs_bf16_emulation(n_nodes, n_agg):
         assert rel_l2(a.grad.float(), b.grad) < 1.5e-2
     for a, b in zip(params, wr):
         assert rel_l2(a.grad, b.grad) < 1.5e-2
+
+
+def _sum_layer_vs_emulation(s, r, n_nodes, loss, seed, repeat=True):
+    """ops.graphnet_sum_layer against the emulated edge update, receiver aggregate and node update composed at the layer's rounding
+    points (e' and the aggregate are bf16 tensors between the kernels).  ``loss``: 'both' outputs, only 'nodes' (v') or only 'edges'
+    (e') enter the loss; autograd hands the layer zeros for the output that does not.  ``repeat``: run the layer twice and require
+    bit-identical results."""
+    torch.manual_seed(seed)
+    rows = s.numel()
+    we, wn = _random_mlp_weights(3, 11), _random_mlp_weights(2, 13)
+    v0 = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16)
+    e0 = torch.randn(rows, 128, device="cuda").to(torch.bfloat16)
+    gv = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16)
+    ge = torch.randn(rows, 128, device="cuda").to(torch.bfloat16)
+    sp, rp = segment_plan(s, n_nodes), segment_plan(r, n_nodes)
+    pick = {"both": (0, 1), "nodes": (0,), "edges": (1,)}[loss]
+    runs = []
+    for _ in range(2 if repeat else 1):
+        pe, pn = _mlp_params(we), _mlp_params(wn)
+        v, e = v0.clone().requires_grad_(True), e0.clone().requires_grad_(True)
+        outs = ops.graphnet_sum_layer(pe, {}, pn, {}, v, e, sp, rp)
+        torch.autograd.backward([outs[i] for i in pick], [(gv, ge)[i] for i in pick])
+        runs.append([outs[0].detach(), outs[1].detach(), v.grad, e.grad] + [p.grad for p in pe + pn])
+    if repeat:
+        for a, b in zip(*runs):
+            assert torch.equal(a, b)
+    v_new, e_new, v_grad, e_grad = runs[-1][:4]
+    rd = lambda t: t.to(torch.bfloat16).float()
+    wer, wnr = [p.detach().clone().requires_grad_(True) for p in pe], [p.detach().clone().requires_grad_(True) for p in pn]
+    vf, ef = v0.float().requires_grad_(True), e0.float().requires_grad_(True)
+    e_ref = rd(_bf16_emulated_projected_edge(vf, ef, s, r, wer))
+    agg = rd(torch.zeros(n_nodes, 128, device="cuda").index_add(0, r, e_ref))
+    v_ref = _bf16_emulated_projected_node(vf, [agg], wnr)
+    torch.autograd.backward([(v_ref, e_ref)[i] for i in pick], [(gv.float(), ge.float())[i] for i in pick])
+    checks = {"v'": (*_row_errs(v_new.float(), v_ref.detach(), rel_err), 1e-2), "e'": (*_row_errs(e_new.float(), e_ref.detach(), rel_err), 1e-2),
+              "grad e": (*_row_errs(e_grad.float(), ef.grad, rel_l2), 1e-2), "grad v": (*_row_errs(v_grad.float(), vf.grad, rel_l2), 1.5e-2)}
+    err, name = _param_errs(pe + pn, wer + wnr, [f"edge {n}" for n in _MLP_NAMES] + [f"node {n}" for n in _MLP_NAMES])
+    checks[f"weights (worst {name})"] = (err, 0.0, 1.5e-2)
+    _report(f"sum layer, {rows} edges / {n_nodes} nodes, loss on {loss}", checks)
+
+
+@pytest.mark.parametrize("loss", ["both", "nodes", "edges"])
+@pytest.mark.parametrize("rows,n_nodes", [(1, 5), (63, 40), (129, 33), ("grid 40x40", 1600), (200000, 40000)])
+def test_graphnet_sum_layer_vs_bf16_emulation(rows, n_nodes, loss):
+    """The fused 'sum' block (bench.py's workload, also the partitioned layer) against the composed emulation: in its backward the node
+    update's share of d loss / d v is added in the epilogue of the node-level dgrad, and d W0 of the edge MLP is written in two column
+    blocks by two kernels (columns 256:384 by the edge backward, 0:256 by the node-level wgrad) into an uninitialised tensor."""
+    if rows == "grid 40x40":
+        s, r = (t.cuda() for t in synthetic.grid_edges_two_way(40, 40))
+        seed = 1600
+    else:
+        seed = rows
+        torch.manual_seed(rows)
+        s = torch.randint(0, n_nodes, (rows,), device="cuda")
+        r = torch.randint(0, n_nodes, (rows,), device="cuda")
+    _sum_layer_vs_emulation(s, r, n_nodes, loss, seed + ["both", "nodes", "edges"].index(loss))
+
+
+def _grid_wrap_rows():
+    return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count * 128
+
+
+@pytest.mark.parametrize("with_add", [False, True])
+@pytest.mark.parametrize("n", [1, 127, 129, "grid wrap + 1", 40000])
+def test_edge_project_backward_contract(n, with_add):
+    """hgn_edge_project_backward called directly: grad_v = gs Ws + gr Wr (+ grad_v_add, added in the kernel's epilogue) against fp64
+    arithmetic on the bf16 operands, grad_W0[:, 0:256] = [gs^T v | gr^T v], and grad_W0[:, 256:384] -- the edge backward's block, which
+    the fused layer writes first -- left bit for bit as it was."""
+    n = _grid_wrap_rows() + 1 if n == "grid wrap + 1" else n
+    lib, bf = _cabi.load(), _cabi.HGN_BF16
+    torch.manual_seed(n + int(with_add))
+    params = _mlp_params(_random_mlp_weights(3, 11))
+    packed = ops._pack_weights({}, torch.bfloat16, 3, params)
+    v, gs, gr, add = (torch.randn(n, 128, device="cuda").to(torch.bfloat16) for _ in range(4))
+    grad_v = torch.full_like(v, float("nan"))
+    grad_w0 = torch.full((128, 384), float("nan"), device="cuda")
+    sentinel = grad_w0[:, 256:].clone()
+    ws = torch.empty(lib.hgn_edge_project_backward_workspace_bytes(bf, n), dtype=torch.uint8, device="cuda")
+    _cabi.check(lib.hgn_edge_project_backward(bf, n, v.data_ptr(), packed.data_ptr(), gs.data_ptr(), gr.data_ptr(),
+                                              add.data_ptr() if with_add else None, grad_v.data_ptr(), grad_w0.data_ptr(), ws.data_ptr(),
+                                              ws.numel(), _cabi.stream_ptr()), "hgn_edge_project_backward")
+    W0 = params[0].detach().to(torch.bfloat16).double()
+    want_v = gs.double() @ W0[:, :128] + gr.double() @ W0[:, 128:256] + (add.double() if with_add else 0.0)
+    want_w = torch.cat([gs.double().t() @ v.double(), gr.double().t() @ v.double()], 1)
+    checks = {"grad v": (*_row_errs(grad_v.float(), want_v, rel_err), 1e-2),
+              "grad W0[:, 0:128]": (rel_err(grad_w0[:, :128], want_w[:, :128]), 0.0, 1e-2),
+              "grad W0[:, 128:256]": (rel_err(grad_w0[:, 128:256], want_w[:, 128:]), 0.0, 1e-2)}
+    _report(f"edge project backward, {n} nodes, grad_v_add {'set' if with_add else 'NULL'}", checks)
+    assert torch.equal(grad_w0[:, 256:].view(torch.int32), sentinel.view(torch.int32)), "grad_W0[:, 256:384] was written"
+
+
+@pytest.mark.parametrize("grad_of", ["out", "agg"])
+@pytest.mark.parametrize("rows,n_nodes", [(1, 5), (129, 33), (200000, 40000)])
+def test_edge_update_backward_contract(rows, n_nodes, grad_of):
+    """hgn_edge_update_backward called directly, once with only grad_out (grad_agg NULL) and once with only grad_agg (grad_out NULL: the
+    processor's last layer): grad_edge, grad_pre0 and the parameter gradients it completes against the emulation from the same tables;
+    grad_W0[:, 0:256], the node-level block, left bit for bit as it was."""
+    lib, bf = _cabi.load(), _cabi.HGN_BF16
+    torch.manual_seed(rows + (grad_of == "agg"))
+    params = _mlp_params(_random_mlp_weights(3, 11))
+    packed = ops._pack_weights({}, torch.bfloat16, 3, params)
+    s = torch.randint(0, n_nodes, (rows,), device="cuda")
+    r = torch.randint(0, n_nodes, (rows,), device="cuda")
+    sp, rp = segment_plan(s, n_nodes), segment_plan(r, n_nodes)
+    rd = lambda t: t.to(torch.bfloat16).float()
+    v = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16).float()
+    ps, pr = (rd(v @ rd(params[0].detach()[:, 128 * k: 128 * (k + 1)]).t()).to(torch.bfloat16) for k in range(2))
+    e = torch.randn(rows, 128, device="cuda").to(torch.bfloat16)
+    grad_out = torch.randn(rows, 128, device="cuda").to(torch.bfloat16) if grad_of == "out" else None
+    grad_agg = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16) if grad_of == "agg" else None
+    grad_e, g0 = torch.full_like(e, float("nan")), torch.full_like(e, float("nan"))
+    gparams = [torch.full(tuple(p.shape), float("nan"), device="cuda") for p in params]
+    sentinel = gparams[0][:, :256].clone()
+    ws = torch.empty(lib.hgn_edge_update_backward_workspace_bytes(bf, rows), dtype=torch.uint8, device="cuda")
+    _cabi.check(lib.hgn_edge_update_backward(bf, rows, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), sp.ids32.data_ptr(), rp.ids32.data_ptr(),
+                                             packed.data_ptr(), _cabi.ptr(grad_out), _cabi.ptr(grad_agg), grad_e.data_ptr(), g0.data_ptr(),
+                                             *[g.data_ptr() for g in gparams], ws.data_ptr(), ws.numel(), _cabi.stream_ptr()),
+                "hgn_edge_update_backward")
+    wr = [p.detach().clone().requires_grad_(True) for p in params]
+    ps_s, pr_r, ef = ps.float()[s].requires_grad_(True), pr.float()[r].requires_grad_(True), e.float().requires_grad_(True)
+    ref = _bf16_emulated_edge_from_table_rows(ps_s, pr_r, ef, wr)
+    ref.backward(grad_out.float() if grad_of == "out" else grad_agg.float()[r])
+    checks = {"grad e": (*_row_errs(grad_e.float(), ef.grad, rel_l2), 1e-2), "grad pre0": (*_row_errs(g0.float(), ps_s.grad, rel_l2), 1.5e-2),
+              "grad W0[:, 256:384]": (rel_l2(gparams[0][:, 256:], wr[0].grad[:, 256:]), 0.0, 1.5e-2)}
+    for g, p, name in zip(gparams[1:], wr[1:], _MLP_NAMES[1:]):
+        checks[name] = (rel_l2(g, p.grad), 0.0, 1.5e-2)
+    _report(f"edge update backward, {rows} edges, only grad_{grad_of} set", checks)
+    assert torch.equal(gparams[0][:, :256].view(torch.int32), sentinel.view(torch.int32)), "grad_W0[:, 0:256] was written"
 
 
 def test_receiver_sorted_edge_storage_is_transparent():

@@ -280,3 +280,26 @@ def test_cfg5_full_mesh_edge_kernels_vs_bf16_emulation():
     print("\ncfg5 full mesh, edge kernels vs bf16 emulation: " + ", ".join(f"{k} {x:.2e}" for k, x in errs.items()))
     assert errs["out"] < 1e-2 and errs["agg"] < 1e-2
     assert errs["grad_e"] < 1e-2 and errs["grad_v"] < 1.5e-2 and errs["grad_w"] < 1.5e-2
+
+
+def test_cfg5_full_mesh_sum_layer_vs_bf16_emulation():
+    """The fused 'sum' block (ops.graphnet_sum_layer, what bench.py times) on the FULL cfg5 mesh, both outputs in the loss, against the
+    composed emulation of tests/test_gpu_parity.py: globally and over the first tile, the last tile and the first wrap of the grid."""
+    from test_gpu_parity import _sum_layer_vs_emulation
+    s, r = (t.cuda() for t in synthetic.grid_edges_two_way(1000, 1000))
+    _sum_layer_vs_emulation(s, r, 1_000_000, "both", seed=8, repeat=False)
+    torch.cuda.empty_cache()
+
+
+def test_tile_kernel_multi_slab_backward_vs_bf16_emulation():
+    """Above 2^21 rows the tile kernels' backward runs in slabs: the tile kernel at a row offset slab0, the workspaces addressed with
+    slab-local rows, the weight-gradient partials and the bias / LayerNorm column sums accumulated from the second slab on.  A node update
+    of 6 chunks ('sum' over five edge sets) on 2^21 + 401 mesh rows -- two slabs, the last tile partial -- against the emulation, with
+    an extra window across the slab boundary.  A slab dropped or overwritten moves the parameter gradients by O(1)."""
+    from test_gpu_parity import _node_update_tile_kernel_vs_emulation
+    slab = 1 << 21
+    torch.cuda.empty_cache()
+    torch.cuda.reset_peak_memory_stats()
+    _node_update_tile_kernel_vs_emulation(6, "mesh", slab + 401, 16, True, extra_windows={"slab boundary": (slab - 128, slab + 128)})
+    print(f"multi-slab backward: peak device memory {torch.cuda.max_memory_allocated() / 2**30:.1f} GiB")
+    torch.cuda.empty_cache()
