@@ -345,8 +345,32 @@ edge_fwd_tc_kernel(int64_t rows, int64_t num_tiles, const uint8_t* __restrict__ 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+typedef CUresult (*CtxGetCurrentFn)(CUcontext*);
+
+// cuTensorMapEncodeTiled needs a current context on the calling thread.  The runtime binds the device's primary context to a thread
+// lazily, at the thread's first runtime call that needs one; a thread whose first call into the library encodes a map (e.g. the
+// autograd engine's device thread starting a backward with a node update) has none yet, and the encode fails with
+// CUDA_ERROR_INVALID_CONTEXT.  cudaSetDevice binds the primary context of the thread's current device.
+static int ensure_current_context() {
+  static CtxGetCurrentFn get = nullptr;
+  if (get == nullptr) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    HGN_CUDA_OK(cudaGetDriverEntryPoint("cuCtxGetCurrent", &p, cudaEnableDefault, &qres));
+    if (p == nullptr || qres != cudaDriverEntryPointSuccess) { set_error("cuCtxGetCurrent is not available from this driver"); return HGN_ERR_CUDA; }
+    get = reinterpret_cast<CtxGetCurrentFn>(p);
+  }
+  CUcontext ctx = nullptr;
+  if (get(&ctx) == CUDA_SUCCESS && ctx != nullptr) return HGN_OK;
+  int dev = 0;
+  HGN_CUDA_OK(cudaGetDevice(&dev));
+  HGN_CUDA_OK(cudaSetDevice(dev));
+  return HGN_OK;
+}
+
 // [rows][128] bf16 row-major tensor, boxes of 128 rows x 64 columns (one 128B-swizzled operand panel)
 int make_rows_tensor_map(CUtensorMap* tm, const void* base, int64_t rows) {
+  if (int rc = ensure_current_context()) return rc;
   static EncodeTiledFn fn = nullptr;
   if (fn == nullptr) {
     void* p = nullptr;

@@ -467,7 +467,8 @@ extern "C" int hgn_segment_reduce(int dtype, const void* data, int64_t E, int32_
 extern "C" int hgn_segment_sum_pair(int dtype, const void* data, int64_t E, int32_t D, const int32_t* perm_a, const int32_t* rowptr_a, int64_t S_a,
                                     void* out_a, const int32_t* perm_b, const int32_t* rowptr_b, int64_t S_b, void* out_b, void* stream) {
   HGN_CHECK_ARG(D >= 1 && E >= 0 && S_a >= 0 && S_b >= 0, "segment_sum_pair: bad sizes");
-  HGN_CHECK_ARG(rowptr_a && rowptr_b && out_a && out_b && (E == 0 || (data && perm_a && perm_b)), "segment_sum_pair: null input");
+  HGN_CHECK_ARG(rowptr_a && rowptr_b && (S_a == 0 || out_a) && (S_b == 0 || out_b) && (E == 0 || (data && perm_a && perm_b)),
+                "segment_sum_pair: null input");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (dtype == HGN_BF16 && D == 128 && S_a > 0 && S_b > 0) {
     const int64_t blocks = ceil_div((S_a > S_b ? S_a : S_b) * 16, 256);
@@ -645,9 +646,10 @@ extern "C" int hgn_colsum(int dtype, const void* x, int64_t rows, int32_t D, flo
 // multi-source segment sum (gather backward): one rounding, fixed order
 // ------------------------------------------------------------------------------------------------
 namespace hgn {
+// base and out are not __restrict__: the header lets out alias base (ops._FusedMLP chains calls with base = out).
 template <typename T>
 __global__ void __launch_bounds__(256)
-multi_segment_sum_kernel(hgn_segment_sources ms, int64_t S, int32_t D, const T* __restrict__ base, T* __restrict__ out) {
+multi_segment_sum_kernel(hgn_segment_sources ms, int64_t S, int32_t D, const T* base, T* out) {
   const int lane = threadIdx.x & 31;
   const int64_t seg = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 5;
   if (seg >= S) return;

@@ -206,7 +206,8 @@ int hgn_node_update_backward(int dtype, int64_t num_nodes, const void* v, int32_
 
 /* ---- column sums ------------------------------------------------------------------------------
  * out[D] (fp32) = sum over rows of x[rows, D]; two-stage fixed-order reduction (LayerNorm beta / bias
- * gradients).  D must be a multiple of 4 and <= 1024. */
+ * gradients).  D must be a multiple of 4, at most 256 and a divisor of 1024 (4, 8, 16, 32, 64, 128 or 256: one block's 256
+ * threads cover the D / 4 column groups); any other D returns HGN_ERR_INVALID_ARGUMENT. */
 size_t hgn_colsum_workspace_bytes(int64_t rows, int32_t D);
 int hgn_colsum(int dtype, const void* x, int64_t rows, int32_t D, float* out,
                void* workspace, size_t workspace_bytes, void* stream);

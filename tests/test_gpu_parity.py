@@ -589,6 +589,145 @@ def test_graphnet_sum_layer_vs_bf16_emulation(rows, n_nodes, loss):
     _sum_layer_vs_emulation(s, r, n_nodes, loss, seed + ["both", "nodes", "edges"].index(loss))
 
 
+class _KernelValue(torch.autograd.Function):
+    """Forward: the kernel's tensor (as fp32); backward: the gradient goes to the emulated tensor.  The emulated aggregates then
+    reduce the kernel's own e', so max / min pick the same winners on both sides, and the gradient still flows through the
+    emulation."""
+
+    @staticmethod
+    def forward(ctx, emulated, kernel):
+        return kernel.detach().float()
+
+    @staticmethod
+    def backward(ctx, grad):
+        return grad, None
+
+
+def _first_winner(e, r, n_nodes, largest):
+    """max / min of ``e``'s rows per receiver, the first edge (lowest id) winning ties, as a gather: its gradient goes to that edge
+    only (scatter_reduce's backward would split it among the tied edges).  An empty segment gives 0."""
+    E, D = e.shape
+    idx = r.view(-1, 1).expand(E, D)
+    with torch.no_grad():
+        ext = torch.zeros(n_nodes, D, device=e.device).scatter_reduce(0, idx, e, "amax" if largest else "amin", include_self=False)
+        pos = torch.arange(E, device=e.device).view(-1, 1).expand(E, D)
+        cand = torch.where(e == ext.gather(0, idx), pos, torch.full_like(pos, E))
+        arg = torch.full((n_nodes, D), E, dtype=torch.int64, device=e.device).scatter_reduce(0, idx, cand, "amin", include_self=True)
+    return torch.cat([e, e.new_zeros(1, D)]).gather(0, arg)
+
+
+def _bf16_emulated_aggregates(e, r, n_nodes, reducers):
+    """The aggregates of ``e`` over receivers as the segment kernels store them: fp32 sums rounded once to bf16; max / min exact."""
+    rd = lambda t: t.to(torch.bfloat16).float()
+    total = torch.zeros(n_nodes, e.shape[1], device=e.device).index_add(0, r, e)
+    count = torch.bincount(r, minlength=n_nodes).clamp(min=1).float().view(-1, 1)
+    by_op = {"sum": lambda: rd(total), "mean": lambda: rd(total / count),
+             "max": lambda: _first_winner(e, r, n_nodes, True), "min": lambda: _first_winner(e, r, n_nodes, False)}
+    return [by_op[op]() for op in reducers]
+
+
+def _module_params(m):
+    """The eight parameters of one reference MLP (Sequential(LazyMLP, LayerNorm)) in the kernels' order."""
+    p = dict(m.named_parameters())
+    return [p[f"0.layers.linear_{k}.{x}"] for k in range(3) for x in ("weight", "bias")] + [p["1.weight"], p["1.bias"]]
+
+
+def _block_vs_emulation(aggregator, edges, n_nodes, loss, seed):
+    """One GraphNet block ('mean' / 'max' / 'min' / 'pna' over one or two edge sets, or 'sum' over two) called with bf16 latents, so
+    that GraphNet.forward routes it through ops.edge_update per set, ops.segment_aggregate (or the 'sum' aggregate of the edge update)
+    and ops.node_update (<= 4 aggregates) or ops.fused_mlp (9 chunks: 'pna' over two sets), against the emulated edge update,
+    aggregation (each aggregate rounded to bf16 as the kernels store it) and node update.  Run twice: bit-identical."""
+    from hgn_b200.migration.graphnet import PNA_OPS
+    torch.manual_seed(seed)
+    names = ["mesh_edges", "world_edges"][:len(edges)]
+    w = synthetic.seeded_state_dict(synthetic.processor_shapes(1, names, aggregator), seed)
+    proc = MeshGraphNet(3, 128, 2, aggregator, 1, "none", names).processor
+    proc.load_state_dict({k[len("processor."):]: t for k, t in w.items()})
+    block = proc.cuda().graphnet_blocks[0]
+    mods = [block.edge_models[nm] for nm in names] + [block.node_model_cross]
+    params = [_module_params(m) for m in mods]
+    v0 = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16)
+    e0 = [torch.randn(s.numel(), 128, device="cuda").to(torch.bfloat16) for s, _ in edges]
+    gv = torch.randn(n_nodes, 128, device="cuda").to(torch.bfloat16)
+    ge = [torch.randn(s.numel(), 128, device="cuda").to(torch.bfloat16) for s, _ in edges]
+    reducers = PNA_OPS if aggregator == "pna" else (aggregator,)
+    rd = lambda t: t.to(torch.bfloat16).float()
+    runs, edge_rows = [], None
+    for run in range(2):
+        block.zero_grad(set_to_none=True)
+        v, es = v0.clone().requires_grad_(True), [e.clone().requires_grad_(True) for e in e0]
+        out = block(hutil.MultiGraph([v], [hutil.EdgeSet(nm, e, s, r) for nm, e, (s, r) in zip(names, es, edges)]))
+        v_new, e_new = out.node_features[0], [x.features for x in out.edge_sets]
+        if run == 0:
+            # the emulation's forward, on the kernel's e'
+            wr = [[p.detach().clone().requires_grad_(True) for p in ps] for ps in params]
+            vf, efs = v0.float().requires_grad_(True), [e.float().requires_grad_(True) for e in e0]
+            e_emul = [rd(_bf16_emulated_projected_edge(vf, ef, s, r, we)) for ef, (s, r), we in zip(efs, edges, wr)]
+            e_used = [_KernelValue.apply(em, k.detach()) for em, k in zip(e_emul, e_new)]
+            aggs = [a for e, (_, r) in zip(e_used, edges) for a in _bf16_emulated_aggregates(e, r, n_nodes, reducers)]
+            if len(aggs) <= 4:
+                v_ref = _bf16_emulated_projected_node(vf, aggs, wr[-1])
+                edge_rows = torch.zeros(n_nodes, dtype=torch.bool, device="cuda")
+            else:
+                # the generic tile kernel (9 chunks): rows with a hidden unit within rounding noise of a ReLU edge get no upstream
+                # gradient, as in _node_update_tile_kernel_vs_emulation
+                v_ref = vf + _bf16_emulated_mlp([vf] + aggs, wr[-1])
+                edge_rows = _relu_edge_rows([vf.detach()] + [a.detach() for a in aggs], wr[-1])
+            gv[edge_rows] = 0
+        outs, grads = [], []
+        if loss in ("both", "nodes"):
+            outs, grads = [v_new], [gv]
+        if loss in ("both", "edges"):
+            outs, grads = outs + e_new, grads + ge
+        torch.autograd.backward(outs, grads)
+        runs.append([v_new.detach(), *[e.detach() for e in e_new], v.grad, *[e.grad for e in es]]
+                    + [p.grad for ps in params for p in ps])
+    for a, b in zip(*runs):
+        assert (a is None and b is None) or torch.equal(a, b)
+    ref_outs, ref_grads = ([v_ref], [gv.float()]) if loss in ("both", "nodes") else ([], [])
+    if loss in ("both", "edges"):
+        ref_outs, ref_grads = ref_outs + e_used, ref_grads + [g.float() for g in ge]
+    torch.autograd.backward(ref_outs, ref_grads)
+    checks = {"v'": (*_row_errs(v_new.float(), v_ref.detach(), rel_err), 1e-2),
+              "grad v": (*_row_errs(v.grad.float(), vf.grad, rel_l2), 1.5e-2)}
+    for nm, en, em, e, ef in zip(names, e_new, e_emul, es, efs):
+        checks[f"{nm}'"] = (*_row_errs(en.float(), em.detach(), rel_err), 1e-2)
+        checks[f"grad {nm}"] = (*_row_errs(e.grad.float(), ef.grad, rel_l2), 1e-2)
+    got, want, pnames = [], [], []
+    for ps, ws_, tag in zip(params, wr, names + ["node"]):
+        for p, q, n in zip(ps, ws_, _MLP_NAMES):
+            if p.grad is None:                  # the node MLP when only e' enters the loss
+                assert q.grad is None, f"{tag} {n}"
+                continue
+            got, want, pnames = got + [p], want + [q], pnames + [f"{tag} {n}"]
+    err, name = _param_errs(got, want, pnames)
+    checks[f"weights (worst {name})"] = (err, 0.0, 1.5e-2)
+    E = "+".join(str(s.numel()) for s, _ in edges)
+    _report(f"{aggregator} block, {E} edges / {n_nodes} nodes, loss on {loss} ({int(edge_rows.sum())} rows on a ReLU edge)", checks)
+
+
+_BLOCK_AGGREGATORS = [(a, n) for a in ("mean", "max", "min", "pna") for n in (1, 2)] + [("sum", 2)]
+_BLOCK_CASES = [(a, n, rows, nodes, "both") for a, n in _BLOCK_AGGREGATORS
+                for rows, nodes in ((1, 5), (129, 33), ("grid 40x40", 1600), (200000, 40000))]
+_BLOCK_CASES += [(a, n, "grid 40x40", 1600, loss) for a, n in _BLOCK_AGGREGATORS for loss in ("nodes", "edges")]
+
+
+@pytest.mark.parametrize("aggregator,n_sets,rows,n_nodes,loss", _BLOCK_CASES)
+def test_graphnet_block_aggregators_vs_bf16_emulation(aggregator, n_sets, rows, n_nodes, loss):
+    """The non-fused bf16 blocks (the multi-set and 'pna' models) against the emulation; the second edge set is random, with about a
+    third as many edges as the first."""
+    seed = (1600 if rows == "grid 40x40" else rows) + 7 * n_sets + ["both", "nodes", "edges"].index(loss)
+    torch.manual_seed(seed)
+    if rows == "grid 40x40":
+        edges = [tuple(t.cuda() for t in synthetic.grid_edges_two_way(40, 40))]
+    else:
+        edges = [(torch.randint(0, n_nodes, (rows,), device="cuda"), torch.randint(0, n_nodes, (rows,), device="cuda"))]
+    if n_sets == 2:
+        m = max(1, edges[0][0].numel() // 3)
+        edges.append((torch.randint(0, n_nodes, (m,), device="cuda"), torch.randint(0, n_nodes, (m,), device="cuda")))
+    _block_vs_emulation(aggregator, edges, n_nodes, loss, seed)
+
+
 def _grid_wrap_rows():
     return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count * 128
 
@@ -709,6 +848,37 @@ def test_projected_edge_update_is_deterministic():
         runs.append([out.detach(), agg.detach(), v.grad, e.grad] + [p.grad for p in params])
     for a, b in zip(*runs):
         assert torch.equal(a, b)
+
+
+def test_edge_kernels_from_a_thread_without_a_current_context():
+    """A host thread's first call into the library may encode a TMA descriptor before any CUDA runtime call has bound a context to the
+    thread (the autograd engine's device thread, when a backward starts with a node update): the library binds the primary context
+    itself.  One edge update forward from a fresh thread, bit for bit that of the main thread."""
+    import threading
+    lib = _cabi.load()
+    torch.manual_seed(5)
+    params = _mlp_params(_random_mlp_weights(3, 11))
+    packed = ops._pack_weights({}, torch.bfloat16, 3, params)
+    n, rows = 300, 1000
+    s, r = torch.randint(0, n, (rows,), device="cuda"), torch.randint(0, n, (rows,), device="cuda")
+    sp, rp = segment_plan(s, n), segment_plan(r, n)
+    v = torch.randn(n, 128, device="cuda").to(torch.bfloat16)
+    e = torch.randn(rows, 128, device="cuda").to(torch.bfloat16)
+    ps, pr = torch.empty_like(v), torch.empty_like(v)
+    ops._edge_project_forward(v, packed, ps, pr)
+    want = torch.empty_like(e)
+    ops._edge_update_forward(e, ps, pr, sp, rp, packed, want)
+    got = torch.full_like(e, float("nan"))
+    args = (_cabi.HGN_BF16, rows, e.data_ptr(), ps.data_ptr(), pr.data_ptr(), sp.ids32.data_ptr(), rp.ids32.data_ptr(), packed.data_ptr(),
+            got.data_ptr(), _cabi.stream_ptr())
+    torch.cuda.synchronize()
+    result = []
+    worker = threading.Thread(target=lambda: result.append((lib.hgn_edge_update_forward(*args), lib.hgn_last_error())))
+    worker.start()
+    worker.join()
+    torch.cuda.synchronize()
+    assert result[0][0] == _cabi.HGN_OK, result[0][1]
+    assert torch.equal(got, want)
 
 
 def test_invalidate_packed_weights_after_a_write_through_data():
