@@ -384,6 +384,99 @@ segment_bwd_bf16_128_kernel(const int32_t* __restrict__ perm, const int32_t* __r
   }
 }
 
+// Incoming gradient of e' in a fused non-'sum' GraphNet layer, over the receiver CSR, half a warp per segment (like the kernel above):
+//   agg_grad[r]  = g_sum[r] + g_mean[r] * (1 / max(cnt_r, 1))           one row per segment, empty ones included; the edge backward
+//                                                                       gathers it through the receivers, so 'sum' / 'mean' need no per-edge pass
+//   edge_grad[e] = base[e] + [argmax[r] == e] g_max[r] + [argmin[r] == e] g_min[r]     every element of a non-empty segment
+// fp32 from +0 in that term order (absent terms skipped), the product without contraction, one bf16 rounding per output.  Up to eight
+// base rows in flight per lane: most segments (in-degree ~6 on triangle meshes) are one round.
+__global__ void __launch_bounds__(256)
+segment_layer_grad_bf16_128_kernel(const int32_t* __restrict__ perm, const int32_t* __restrict__ rowptr, int64_t S,
+                                   const __nv_bfloat16* __restrict__ g_sum, const __nv_bfloat16* __restrict__ g_mean,
+                                   const __nv_bfloat16* __restrict__ g_max, const __nv_bfloat16* __restrict__ g_min,
+                                   const int32_t* __restrict__ argmax, const int32_t* __restrict__ argmin,
+                                   const __nv_bfloat16* __restrict__ base, __nv_bfloat16* __restrict__ agg_grad,
+                                   __nv_bfloat16* __restrict__ edge_grad) {
+  const int l16 = threadIdx.x & 15;
+  const uint32_t hmask = 0xFFFFu << (threadIdx.x & 16);
+  const int64_t seg = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 4;
+  if (seg >= S) return;                                     // whole half-warps leave together (the shuffles below use hmask)
+  const int beg = rowptr[seg], end = rowptr[seg + 1];
+  const int64_t o = seg * 128 + l16 * 8;
+  auto unpack8 = [](const uint4& p, float (&f)[8]) {
+    const uint32_t w[4] = {p.x, p.y, p.z, p.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { f[2 * i] = __uint_as_float(w[i] << 16); f[2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u); }
+  };
+  auto pack8 = [](const float (&f)[8]) {
+    uint32_t w[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      __nv_bfloat162 t = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
+      w[i] = *reinterpret_cast<uint32_t*>(&t);
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
+  };
+  // Every load that depends only on the segment is issued first (the first eight element ids, the gradient rows, the winners), so a
+  // segment costs three dependent memory round trips: rowptr, then these, then the base rows.  agg_grad is stored last.
+  const bool edges = edge_grad != nullptr && end > beg;
+  const uint4 z4 = make_uint4(0u, 0u, 0u, 0u);
+  const int4 none = make_int4(-1, -1, -1, -1);
+  int mine = (edges && l16 < 8 && beg + l16 < end) ? __ldg(perm + beg + l16) : -1;
+  const uint4 ps = agg_grad && g_sum ? __ldg(reinterpret_cast<const uint4*>(g_sum + o)) : z4;
+  const uint4 pm = agg_grad && g_mean ? __ldg(reinterpret_cast<const uint4*>(g_mean + o)) : z4;
+  const uint4 px = edges && g_max ? __ldg(reinterpret_cast<const uint4*>(g_max + o)) : z4;
+  const uint4 pn = edges && g_min ? __ldg(reinterpret_cast<const uint4*>(g_min + o)) : z4;
+  const int4 ax0 = edges && g_max ? __ldg(reinterpret_cast<const int4*>(argmax + o)) : none;
+  const int4 ax1 = edges && g_max ? __ldg(reinterpret_cast<const int4*>(argmax + o + 4)) : none;
+  const int4 an0 = edges && g_min ? __ldg(reinterpret_cast<const int4*>(argmin + o)) : none;
+  const int4 an1 = edges && g_min ? __ldg(reinterpret_cast<const int4*>(argmin + o + 4)) : none;
+  if (edges) {
+    float gx[8], gn[8];
+    unpack8(px, gx);
+    unpack8(pn, gn);
+    const int ax[8] = {ax0.x, ax0.y, ax0.z, ax0.w, ax1.x, ax1.y, ax1.z, ax1.w};
+    const int an[8] = {an0.x, an0.y, an0.z, an0.w, an1.x, an1.y, an1.z, an1.w};
+    for (int j = beg; j < end; j += 8) {
+      if (j > beg) mine = (l16 < 8 && j + l16 < end) ? __ldg(perm + j + l16) : -1;
+      int e[8];
+      uint4 b[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        e[k] = __shfl_sync(hmask, mine, k, 16);
+        b[k] = z4;
+        if (base && e[k] >= 0) b[k] = __ldg(reinterpret_cast<const uint4*>(base + int64_t(e[k]) * 128) + l16);
+      }
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        if (e[k] < 0) break;
+        float g[8];
+        unpack8(b[k], g);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          g[i] = __fadd_rn(0.f, g[i]);
+          if (ax[i] == e[k]) g[i] = __fadd_rn(g[i], gx[i]);
+          if (an[i] == e[k]) g[i] = __fadd_rn(g[i], gn[i]);
+        }
+        *(reinterpret_cast<uint4*>(edge_grad + int64_t(e[k]) * 128) + l16) = pack8(g);
+      }
+    }
+  }
+  if (agg_grad) {
+    float a[8], f[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) a[i] = 0.f;
+    if (g_sum) { unpack8(ps, f);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) a[i] = __fadd_rn(a[i], f[i]); }
+    if (g_mean) { unpack8(pm, f);
+      const float inv = 1.0f / float(max(end - beg, 1));
+#pragma unroll
+      for (int i = 0; i < 8; ++i) a[i] = __fadd_rn(a[i], __fmul_rn(f[i], inv)); }
+    *reinterpret_cast<uint4*>(agg_grad + o) = pack8(a);
+  }
+}
+
 template <typename T>
 static int segment_reduce_bwd_impl(int64_t E, int32_t D, const int32_t* ids, const int32_t* perm, const int32_t* rowptr, int64_t S,
                                    const T* g_sum, const T* g_mean, const T* g_max, const T* g_min, const int32_t* argmax,
@@ -498,6 +591,32 @@ extern "C" int hgn_segment_reduce_bwd(int dtype, int64_t E, int32_t D, const int
                                                   (__nv_bfloat16*)grad_data, accumulate, st);
   set_error("segment_reduce_bwd: unknown dtype %d", dtype);
   return HGN_ERR_INVALID_ARGUMENT;
+}
+
+extern "C" int hgn_segment_layer_grad(int dtype, int64_t E, int32_t D, const int32_t* perm, const int32_t* rowptr, int64_t S,
+                                      const void* g_sum, const void* g_mean, const void* g_max, const void* g_min,
+                                      const int32_t* argmax, const int32_t* argmin, const void* base, void* agg_grad, void* edge_grad,
+                                      void* stream) {
+  if (dtype == HGN_F32) { set_error("segment_layer_grad: bf16 only"); return HGN_ERR_UNSUPPORTED; }
+  HGN_CHECK_ARG(dtype == HGN_BF16, "segment_layer_grad: unknown dtype %d", dtype);
+  HGN_CHECK_ARG(D == 128, "segment_layer_grad: D=%d, only 128 is supported", D);
+  HGN_CHECK_ARG(E >= 0 && S >= 0 && E < (int64_t(1) << 31) && S < (int64_t(1) << 31) - 1, "segment_layer_grad: bad sizes");
+  HGN_CHECK_ARG((!g_max || argmax) && (!g_min || argmin), "segment_layer_grad: max/min gradients need their arg indices");
+  HGN_CHECK_ARG((!g_sum && !g_mean) || agg_grad, "segment_layer_grad: sum/mean gradients need agg_grad");
+  HGN_CHECK_ARG((!g_max && !g_min && !base) || edge_grad, "segment_layer_grad: max/min gradients and base need edge_grad");
+  HGN_CHECK_ARG(S == 0 || rowptr, "segment_layer_grad: null rowptr");
+  HGN_CHECK_ARG(!edge_grad || E == 0 || perm, "segment_layer_grad: edge_grad needs perm");
+  HGN_CHECK_ARG(!edge_grad || edge_grad != base, "segment_layer_grad: edge_grad must not alias base");
+  HGN_CHECK_ARG(!agg_grad || (agg_grad != g_sum && agg_grad != g_mean && agg_grad != g_max && agg_grad != g_min),
+                "segment_layer_grad: agg_grad must not alias a gradient input");
+  if (S == 0 || (!agg_grad && !edge_grad)) return HGN_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  HGN_TIMED("segment_layer_grad", st);
+  segment_layer_grad_bf16_128_kernel<<<unsigned(ceil_div(S * 16, 256)), 256, 0, st>>>(
+      perm, rowptr, S, (const __nv_bfloat16*)g_sum, (const __nv_bfloat16*)g_mean, (const __nv_bfloat16*)g_max, (const __nv_bfloat16*)g_min,
+      argmax, argmin, (const __nv_bfloat16*)base, (__nv_bfloat16*)agg_grad, (__nv_bfloat16*)edge_grad);
+  HGN_LAUNCH_OK("segment_layer_grad");
+  return HGN_OK;
 }
 
 extern "C" int hgn_rows_gather(int dtype, const void* src, const int32_t* idx, int64_t n, int32_t D, void* dst, void* stream) {

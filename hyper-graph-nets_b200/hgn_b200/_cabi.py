@@ -55,6 +55,7 @@ SIGNATURES = {
                                       c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "hgn_segment_reduce_bwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    "hgn_segment_layer_grad": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_int64] + [c_void_p] * 9 + [c_void_p]),
     "hgn_multi_segment_sum": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
     "hgn_mlp_packed_bytes": (c_size_t, [c_int, c_int32]),
     "hgn_mlp_pack": (c_int, [c_int, c_int32] + [c_void_p] * 8 + [c_void_p, c_void_p]),

@@ -155,25 +155,26 @@ class GraphNet(nn.Module):
 
     # ---- schedules ---------------------------------------------------------------------------
     def _whole_layer(self, graph: MultiGraph):
-        """A block that ``takes_whole_layer`` on its one node list runs as a single autograd node (ops.graphnet_sum_layer)."""
+        """A block that ``takes_whole_layer`` on its one node list runs as a single autograd node (ops.graphnet_layer)."""
         if len(graph.node_features) != 1 or not takes_whole_layer(self, graph.node_features[0], graph.edge_sets):
             return None
         v, es = graph.node_features[0], graph.edge_sets[0]
         num_nodes = v.shape[0]
         senders = segment_plan(to_device_index(es.senders, v.device), num_nodes)
         receivers = segment_plan(to_device_index(es.receivers, v.device), num_nodes)
-        v_new, e_new = self._sum_layer(v, es.features.to(v.device), es.name, senders, receivers)
+        v_new, e_new = self._layer(v, es.features.to(v.device), es.name, senders, receivers)
         graph = graph._replace(edge_sets=[es._replace(features=e_new)])
         graph.node_features[0] = v_new
         return graph
 
-    def _sum_layer(self, v: Tensor, e: Tensor, edge_set_name: str, senders, receivers, halo=None):
-        """``(v', e')`` of ``ops.graphnet_sum_layer`` with this block's weights."""
+    def _layer(self, v: Tensor, e: Tensor, edge_set_name: str, senders, receivers, halo=None):
+        """``(v', e')`` of ``ops.graphnet_layer`` with this block's weights and aggregator."""
         edge_model = self.edge_models[edge_set_name]
+        k = 4 if self.message_passing_aggregator == 'pna' else 1
         ep = _mlp_parameters(edge_model, 3 * v.shape[1], v)
-        np_ = _mlp_parameters(self.node_model_cross, 2 * v.shape[1], v)
-        return ops.graphnet_sum_layer(ep, _packed_cache(edge_model), np_, _packed_cache(self.node_model_cross), v, e, senders, receivers,
-                                      halo)
+        np_ = _mlp_parameters(self.node_model_cross, (1 + k) * v.shape[1], v)
+        return ops.graphnet_layer(ep, _packed_cache(edge_model), np_, _packed_cache(self.node_model_cross), v, e, senders, receivers,
+                                  self.message_passing_aggregator, halo)
 
     def forward(self, graph: MultiGraph, mask=None) -> MultiGraph:
         """graphnet.py:72-84: every edge set from the OLD node latents, then one mesh-node update."""
@@ -200,10 +201,11 @@ class GraphNet(nn.Module):
 
 
 def takes_whole_layer(block: nn.Module, v: Tensor, edge_sets: Sequence[EdgeSet]) -> bool:
-    """Whether ``block`` runs on node latents ``v`` and ``edge_sets`` as one ``ops.graphnet_sum_layer``: the cfg5 shape -- plain
-    GraphNet, 'sum', one edge set with a model, bf16 latents of width 128 on the GPU, at least one edge and one node.  The one-GPU
-    block (``GraphNet._whole_layer``) and the partitioned processor (``partition.PartitionedProcessor``) both decide with it."""
-    if (type(block) is not GraphNet or block.message_passing_aggregator != 'sum' or len(edge_sets) != 1
+    """Whether ``block`` runs on node latents ``v`` and ``edge_sets`` as one ``ops.graphnet_layer``: plain GraphNet with the 'sum',
+    'mean', 'max', 'min' or 'pna' aggregator, one edge set with a model, bf16 latents of width 128 on the GPU, at least one edge and one
+    node.  The one-GPU block (``GraphNet._whole_layer``) and the partitioned processor (``partition.PartitionedProcessor``) both
+    decide with it."""
+    if (type(block) is not GraphNet or block.message_passing_aggregator not in PNA_OPS + ('pna',) or len(edge_sets) != 1
             or edge_sets[0].name not in block.edge_models.keys()):
         return False
     e = edge_sets[0].features

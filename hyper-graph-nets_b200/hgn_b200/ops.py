@@ -369,6 +369,27 @@ def _segment_sum(data, plan: SegmentPlan, out) -> None:
     _count(int(S > 0))          # segment_reduce_impl: one kernel
 
 
+def _segment_reduce(data, plan: SegmentPlan, outs, argmax, argmin) -> None:
+    """The reductions ``outs`` = (sum, mean, max, min; None = not requested) of ``data``'s bf16 rows of width 128 over the segments of
+    ``plan``, with the max / min winners when ``argmax`` / ``argmin`` are given."""
+    S = plan.num_segments
+    _cabi.check(_cabi.load().hgn_segment_reduce(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(),
+                                                S, *[_cabi.ptr(o) for o in outs], _cabi.ptr(argmax), _cabi.ptr(argmin), 0,
+                                                _cabi.stream_ptr()), "hgn_segment_reduce")
+    _count(int(S > 0))          # segment_reduce_impl: one kernel
+
+
+def _segment_layer_grad(plan: SegmentPlan, E: int, grads: dict, argmax, argmin, base, agg_grad, edge_grad) -> None:
+    """``agg_grad[r] = g_sum[r] + g_mean[r] / cnt_r`` and ``edge_grad[e] = base[e] + the max / min winners' gradients`` over the receiver
+    plan (``grads``: reducer name -> gradient of that aggregate)."""
+    S = plan.num_segments
+    _cabi.check(_cabi.load().hgn_segment_layer_grad(
+        _BF, E, D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S, *[_cabi.ptr(grads.get(op)) for op in OP_BITS],
+        _cabi.ptr(argmax), _cabi.ptr(argmin), _cabi.ptr(base), _cabi.ptr(agg_grad), _cabi.ptr(edge_grad), _cabi.stream_ptr()),
+        "hgn_segment_layer_grad")
+    _count(int(S > 0 and (agg_grad is not None or edge_grad is not None)))     # hgn_segment_layer_grad: one kernel
+
+
 def _segment_sum_pair(data, plan_a: SegmentPlan, out_a, plan_b: SegmentPlan, out_b) -> None:
     """Two ``_segment_sum``s of the same rows under two groupings."""
     S_a, S_b = out_a.shape[0], out_b.shape[0]
@@ -541,79 +562,114 @@ def _layer_workspace(n: int, E: int, device) -> torch.Tensor:
     return torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
-class _GraphNetSumLayer(torch.autograd.Function):
-    """One whole ``GraphNet`` block with the 'sum' aggregator and ONE edge set (graphnet.py:72-84) as a single autograd node:
+class _GraphNetLayer(torch.autograd.Function):
+    """One whole ``GraphNet`` block with ONE edge set (graphnet.py:72-84) as a single autograd node, for the reducers of its
+    aggregator (``('sum',)``, ``('mean',)``, ``('max',)``, ``('min',)`` or the four of 'pna', in the order of graphnet.py:53-64):
 
-        forward   node projection -> fused edge update -> receiver aggregate -> aggregate projection + fused node update
-        backward  fused node backward -> fused edge backward (aggregate gradient gathered inside) -> sender / receiver sums of G0 ->
-                  node-level dgrad with the node update's share of d loss / d v added in its epilogue -> node-level wgrads
+        forward   node projection -> fused edge update -> receiver aggregate(s) -> aggregate projection + fused node update
+        backward  fused node backward -> [not 'sum': incoming gradient of e' from the aggregate gradients] -> fused edge backward
+                  (the 'sum' / 'mean' share of the aggregate gradient gathered inside) -> sender / receiver sums of G0 -> node-level
+                  dgrad with the node update's share of d loss / d v added in its epilogue -> node-level wgrads
 
-    Same kernels and same arithmetic as ``edge_update`` + ``node_update``; what goes away is the autograd glue between them: the
-    ``at::add`` of the two partial gradients of ``v`` ([N,128] read twice and written once per layer), zero fills, and four autograd
-    nodes' worth of Python per layer.
+    Same kernels and same forward arithmetic as ``edge_update`` + ``segment_aggregate`` / the edge update's 'sum' + ``node_update``;
+    what goes away is the autograd glue between them: the bf16 ``at::add`` of the two partial gradients of ``v`` (the node update's
+    share is added in fp32 instead), zero fills, four autograd nodes' worth of Python per layer, and for a non-'sum' aggregator the
+    dense ``[E,128]`` aggregate gradient and its ``at::add`` to the next layer's d e' (``hgn_segment_layer_grad`` writes per-node rows
+    for 'sum' / 'mean' and adds the max / min winners to d e' in one pass).
 
     ``halo`` (not a tensor: passed through untouched, like the plans) makes this the block of one rank of a partitioned graph
     (``partition.PeerLayerHalo``).  ``v`` then holds the owned nodes, and the senders index ``[owned | ghosts]``.  The halo provides
     the sender table ``Ps`` (``[n_own + n_ghost, 128]``; this rank writes the owned rows), a forward exchange that fills the ghost
     rows after the projection, and a backward exchange that sends the ghost rows of the sender sums home and adds the rows the peers
-    return into the owned ones.  Everything else is this schedule, so an owned row sees the kernels and the rounding points of the
+    return into the owned ones.  Every edge of an owned receiver is local, so the aggregates and the max / min winners are complete
+    without further exchanges.  Everything else is this schedule, so an owned row sees the kernels and the rounding points of the
     one-GPU layer."""
 
     @staticmethod
-    def forward(ctx, v, e, s_plan, r_plan, packed_e, packed_n, halo, *params):
+    def forward(ctx, v, e, s_plan, r_plan, packed_e, packed_n, halo, reducers, *params):
+        k = len(reducers)
         ps = halo.sender_table() if halo is not None else torch.empty_like(v)
         pr, q1 = torch.empty_like(v), torch.empty_like(v)
-        e_new, v_new, agg = torch.empty_like(e), torch.empty_like(v), torch.empty_like(v)
+        q2 = torch.empty_like(v) if k > 2 else None
+        e_new, v_new = torch.empty_like(e), torch.empty_like(v)
+        aggs = [torch.empty_like(v) for _ in reducers]
+        winners = any(ctx.needs_input_grad)             # the backward needs the max / min winners
+        new_arg = lambda op: torch.empty(v.shape, dtype=torch.int32, device=v.device) if winners and op in reducers else None
+        argmax, argmin = new_arg("max"), new_arg("min")
         with torch.cuda.device(v.device):
             _edge_project_forward(v, packed_e, ps, pr)
             if halo is not None:
                 halo.exchange_forward()
             _edge_update_forward(e, ps, pr, s_plan, r_plan, packed_e, e_new)
-            _segment_sum(e_new, r_plan, agg)
-            _node_update_forward(v, [agg], packed_n, q1, None, v_new)
-        ctx.save_for_backward(v, e, ps, pr, agg, q1)
-        ctx.plans, ctx.packed, ctx.halo = (s_plan, r_plan), (packed_e, packed_n), halo
+            if reducers == ("sum",):
+                _segment_sum(e_new, r_plan, aggs[0])
+            else:
+                by_op = dict(zip(reducers, aggs))
+                _segment_reduce(e_new, r_plan, [by_op.get(op) for op in OP_BITS], argmax, argmin)
+            _node_update_forward(v, aggs, packed_n, q1, q2, v_new)
+        ctx.save_for_backward(v, e, ps, pr, q1, q2, argmax, argmin, *aggs)
+        ctx.plans, ctx.packed, ctx.halo, ctx.reducers = (s_plan, r_plan), (packed_e, packed_n), halo, reducers
         ctx.param_shapes = [tuple(p.shape) for p in params]
         return v_new, e_new
 
     @staticmethod
     def backward(ctx, grad_v_new, grad_e_new):
-        v, e, ps, pr, agg, q1 = ctx.saved_tensors
+        v, e, ps, pr, q1, q2, argmax, argmin, *aggs = ctx.saved_tensors
         s_plan, r_plan = ctx.plans
         packed_e, packed_n = ctx.packed
         dev = v.device
         grad_v_new = grad_v_new.contiguous().to(v.dtype) if grad_v_new is not None else torch.zeros_like(v)
         grad_e_new = grad_e_new.contiguous().to(e.dtype) if grad_e_new is not None else None
         new = lambda like: torch.empty_like(like)
-        grad_v_node, grad_agg, grad_v, gs, gr = new(v), new(v), new(v), new(ps), new(v)
+        grad_v_node, grad_v, gs, gr = new(v), new(v), new(ps), new(v)
+        grad_aggs = [new(v) for _ in aggs]
         grad_e, g0 = new(e), new(e)
         ge = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[:8]]
         gn = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes[8:]]
         with torch.cuda.device(dev):
             ws = _layer_workspace(v.shape[0], e.shape[0], dev)
-            _node_update_backward(v, [agg], q1, None, packed_n, grad_v_new, grad_v_node, [grad_agg], gn, ws)
-            _edge_update_backward(e, ps, pr, s_plan, r_plan, packed_e, grad_e_new, grad_agg, grad_e, g0, ge, ws)
+            _node_update_backward(v, aggs, q1, q2, packed_n, grad_v_new, grad_v_node, grad_aggs, gn, ws)
+            if ctx.reducers == ("sum",):
+                grad_out, grad_agg = grad_e_new, grad_aggs[0]
+            else:
+                g = dict(zip(ctx.reducers, grad_aggs))
+                grad_agg = new(v) if "sum" in g or "mean" in g else None
+                edge_grad = new(e) if "max" in g or "min" in g else None
+                _segment_layer_grad(r_plan, e.shape[0], g, argmax, argmin, grad_e_new if edge_grad is not None else None, grad_agg,
+                                    edge_grad)
+                grad_out = edge_grad if edge_grad is not None else grad_e_new
+            _edge_update_backward(e, ps, pr, s_plan, r_plan, packed_e, grad_out, grad_agg, grad_e, g0, ge, ws)
             _segment_sum_pair(g0, s_plan, gs, r_plan, gr)
             if ctx.halo is not None:
                 ctx.halo.exchange_backward(gs)
             # the edge backward wrote only the We block of d W0 (columns 256:384); the node-level kernel fills columns 0:256
             _edge_project_backward(v, packed_e, gs, gr, grad_v_node, grad_v, ge[0], ws)
-        return (grad_v, grad_e, None, None, None, None, None, *ge, *gn)
+        return (grad_v, grad_e, None, None, None, None, None, None, *ge, *gn)
+
+
+def graphnet_layer(edge_params: Sequence[torch.Tensor], edge_cache: dict, node_params: Sequence[torch.Tensor], node_cache: dict,
+                   v: torch.Tensor, e: torch.Tensor, s_plan: SegmentPlan, r_plan: SegmentPlan, aggregator: str, halo=None):
+    """``(v', e')`` of one GraphNet block (one edge set, bf16 latents of width 128) with ``aggregator`` 'sum', 'mean', 'max', 'min' or
+    'pna': see ``_GraphNetLayer``."""
+    _cabi.require_cuda(v, e)
+    if aggregator != "pna" and aggregator not in OP_BITS:
+        raise _cabi.HgnError(f"graphnet_layer: unknown aggregator {aggregator!r}")
+    reducers = tuple(OP_BITS) if aggregator == "pna" else (aggregator,)
+    if v.dtype != torch.bfloat16 or e.dtype != torch.bfloat16 or v.shape[-1] != D_LATENT or e.shape[-1] != D_LATENT:
+        raise _cabi.HgnError("graphnet_layer is the bf16 tcgen05 path for latent 128")
+    if edge_params[0].shape != (D_LATENT, 3 * D_LATENT) or node_params[0].shape != (D_LATENT, (1 + len(reducers)) * D_LATENT):
+        raise _cabi.HgnError(f"graphnet_layer ({aggregator}): first linears {tuple(edge_params[0].shape)} / {tuple(node_params[0].shape)}")
+    v, e = v.contiguous(), e.contiguous()
+    with torch.cuda.device(v.device):
+        packed_e = _pack_weights(edge_cache, torch.bfloat16, 3, edge_params)
+        packed_n = _pack_weights(node_cache, torch.bfloat16, 1 + len(reducers), node_params)
+    return _GraphNetLayer.apply(v, e, s_plan, r_plan, packed_e, packed_n, halo, reducers, *edge_params, *node_params)
 
 
 def graphnet_sum_layer(edge_params: Sequence[torch.Tensor], edge_cache: dict, node_params: Sequence[torch.Tensor], node_cache: dict,
                        v: torch.Tensor, e: torch.Tensor, s_plan: SegmentPlan, r_plan: SegmentPlan, halo=None):
-    """``(v', e')`` of one GraphNet block ('sum', one edge set, bf16 latents of width 128): see ``_GraphNetSumLayer``."""
-    _cabi.require_cuda(v, e)
-    if v.dtype != torch.bfloat16 or e.dtype != torch.bfloat16 or v.shape[-1] != D_LATENT or e.shape[-1] != D_LATENT:
-        raise _cabi.HgnError("graphnet_sum_layer is the bf16 tcgen05 path for latent 128")
-    if edge_params[0].shape != (D_LATENT, 3 * D_LATENT) or node_params[0].shape != (D_LATENT, 2 * D_LATENT):
-        raise _cabi.HgnError(f"graphnet_sum_layer: first linears {tuple(edge_params[0].shape)} / {tuple(node_params[0].shape)}")
-    v, e = v.contiguous(), e.contiguous()
-    with torch.cuda.device(v.device):
-        packed_e = _pack_weights(edge_cache, torch.bfloat16, 3, edge_params)
-        packed_n = _pack_weights(node_cache, torch.bfloat16, 2, node_params)
-    return _GraphNetSumLayer.apply(v, e, s_plan, r_plan, packed_e, packed_n, halo, *edge_params, *node_params)
+    """``graphnet_layer`` with the 'sum' aggregator."""
+    return graphnet_layer(edge_params, edge_cache, node_params, node_cache, v, e, s_plan, r_plan, "sum", halo)
 
 
 def colsum(x: torch.Tensor) -> torch.Tensor:

@@ -363,7 +363,7 @@ class PeerHalo:
 
 
 class PeerLayerHalo(NamedTuple):
-    """The halo of one (step, layer) of a ``PeerHalo``, in the form ``ops.graphnet_sum_layer`` takes it."""
+    """The halo of one (step, layer) of a ``PeerHalo``, in the form ``ops.graphnet_layer`` takes it."""
     peer: PeerHalo
     step: int
     layer: int
@@ -383,9 +383,10 @@ class PartitionedProcessor(torch.nn.Module):
 
     Generic path (any block type, any aggregator, fp32 or bf16): ghosts are refreshed before every block with a grouped NCCL
     send/recv; the block itself is unchanged (it sees ``[owned | ghosts]`` as ``[mesh | hyper]`` rows).
-    Fast path (``PeerHalo`` given, and every block takes the whole-layer route of ``GraphNet`` -- the cfg5 benchmark):
-    ``ops.graphnet_sum_layer`` per block with the halo of that layer; halo rows travel as peer-memory stores issued by a kernel of
-    the sending rank."""
+    Fast path (``PeerHalo`` given, and every block takes the whole-layer route of ``GraphNet``: one edge set, bf16, any of the
+    'sum' / 'mean' / 'max' / 'min' / 'pna' aggregators -- the cfg5 benchmark): ``ops.graphnet_layer`` per block with the halo of that
+    layer; halo rows travel as peer-memory stores issued by a kernel of the sending rank.  Every edge of an owned receiver is local,
+    so the aggregates (max / min winners included) need no exchange of their own."""
 
     def __init__(self, processor: torch.nn.Module, plan: HaloPlan, peer: Optional[PeerHalo] = None):
         super().__init__()
@@ -419,7 +420,7 @@ class PartitionedProcessor(torch.nn.Module):
             step = self.peer.steps_done
             self.peer.steps_done += 1
             for layer, block in enumerate(self.processor.graphnet_blocks):
-                owned, e = block._sum_layer(owned, e, es.name, self.peer.s_plan, self.peer.r_plan, PeerLayerHalo(self.peer, step, layer))
+                owned, e = block._layer(owned, e, es.name, self.peer.s_plan, self.peer.r_plan, PeerLayerHalo(self.peer, step, layer))
             return owned.to(in_dtype), [es._replace(features=e)]
         graph = MultiGraph([owned, None], list(edge_sets))
         for block in self.processor.graphnet_blocks:
@@ -492,8 +493,8 @@ def bench_partitioned(args, world, rank, dev, width, height, layers, metric, uni
     v0 = torch.randn(n, 128, generator=gen)[lg.owned]
     e0 = torch.randn(e_total, 128, generator=gen)[lg.edge_ids]
     coef = torch.randn(n, 128, generator=gen)[lg.owned].to(dev)
-    weights = synthetic.seeded_state_dict(synthetic.processor_shapes(layers, ["mesh_edges"], "sum"), seed=17)
-    shell = MeshGraphNet(3, 128, 2, "sum", layers, "none", ["mesh_edges"])
+    weights = synthetic.seeded_state_dict(synthetic.processor_shapes(layers, ["mesh_edges"], args.aggregator), seed=17)
+    shell = MeshGraphNet(3, 128, 2, args.aggregator, layers, "none", ["mesh_edges"])
     proc = shell.processor
     proc.load_state_dict({k[len("processor."):]: t for k, t in weights.items()})
     proc = proc.to(dev)
@@ -618,7 +619,8 @@ def bench_partitioned(args, world, rank, dev, width, height, layers, metric, uni
             "metric": metric, "value": value, "unit": unit, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "bf16",
             "data": "synthetic (seeded 1000x1000 triangulated grid, seeded weights)",
-            "config": {"workload": "cfg5: 1M-node / 5 992 002-edge triangulated mesh, 15 GraphNet layers, sum aggregator, processor fwd+bwd",
+            "config": {"workload": f"cfg5: 1M-node / 5 992 002-edge triangulated mesh, 15 GraphNet layers, {args.aggregator} aggregator, "
+                                   "processor fwd+bwd",
                        "nodes": n, "edges": e_total, "layers": layers, "latent": 128,
                        "partitioning": f"edge-cut, {world} row slabs, receiver-owner rule, one-ring halo per layer (max {int(halo_rows)} ghost "
                                        f"rows per rank): " + ("rows of the sender table Ps pushed into the peers' tables over NVLink peer memory by a "

@@ -95,6 +95,20 @@ int hgn_segment_reduce_bwd(int dtype, int64_t num_edges, int32_t D,
                            const int32_t* argmax, const int32_t* argmin,
                            void* grad_data, int accumulate, void* stream);
 
+/* Incoming gradient of e' in a GraphNet layer with a 'mean' / 'max' / 'min' / 'pna' aggregator (HGN_BF16, D = 128 only; HGN_F32
+ * returns HGN_ERR_UNSUPPORTED), in one pass over the receiver CSR (perm, rowptr[S+1]) of the num_edges elements:
+ *     agg_grad[r,:]  = g_sum[r,:] + g_mean[r,:] * (1 / max(cnt_r, 1))                                 [S,128], every segment
+ *     edge_grad[e,:] = base[e,:] + [argmax[r_e,:] == e] g_max[r_e,:] + [argmin[r_e,:] == e] g_min[r_e,:]    [E,128]
+ * agg_grad is what hgn_edge_update_backward gathers through the receivers as grad_agg, edge_grad its grad_out; base is the dense
+ * gradient of e' (next layer / loss).  NULL inputs are skipped.  Arithmetic: fp32 starting from +0, terms added in the order above,
+ * g_mean * inv rounded before the addition (no fused multiply-add), each output rounded to bf16 once.  agg_grad may be NULL when
+ * g_sum and g_mean are; edge_grad may be NULL when g_max, g_min and base are; edge_grad must not alias base, nor agg_grad a
+ * gradient input. */
+int hgn_segment_layer_grad(int dtype, int64_t num_edges, int32_t D, const int32_t* perm, const int32_t* rowptr, int64_t num_segments,
+                           const void* g_sum, const void* g_mean, const void* g_max, const void* g_min,
+                           const int32_t* argmax, const int32_t* argmin, const void* base, void* agg_grad, void* edge_grad,
+                           void* stream);
+
 /* Backward of the row gathers v[senders], v[receivers] (torch.index_select -> index_add_ with float
  * atomics in the reference, src/migration/graphnet.py:28-29): out[n,:] = base[n,:] (if base != NULL)
  * + sum_k sum_{j in segment_k(n)} data_k[perm_k[j], :], accumulated in fp32 in a fixed order
