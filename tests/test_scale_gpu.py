@@ -7,8 +7,8 @@
 * the FULL cfg5 mesh (1 000 000 nodes / 5 992 002 edges, 317 tiles per CTA), one layer: sampled edge rows, the aggregation of
   sampled receivers and sampled node rows against the oracle's arithmetic on exactly those rows; the bf16 (tcgen05) and fp32
   (FFMA) backward passes against each other; run-to-run bit identity.
-Tolerances: fp32 1e-5 / bf16 2e-2 on forward quantities (max metric); gradients: fp32 max metric, bf16 relative L2 with the
-bound = the measured figure x 2 (printed by the tests; see GRAD_L2).
+Tolerances: fp32 1e-5 / bf16 2e-2 on forward quantities (max metric); gradients: relative L2 in bf16, and in fp32 above ~10^5 rows x
+layers (the max metric below that), with the bound = the measured figure x 2 (printed by the tests; see GRAD_L2).
 """
 import numpy as np
 import pytest
@@ -30,11 +30,13 @@ GRAD_MAX_FP32 = 1e-4            # max metric, small graphs (a few thousand rows)
 # slab 1.8e-2 / 2.5e-2, 15 layers 2.7e-2 / 4.8e-2) while the L2 metric stays at the share of affected rows.  With 'pna' the same
 # happens to max / min winners (tests/test_gpu_parity.py: fp32_grad_check).  Bounds = the figures measured on the B200 (printed by
 # the tests; profiles/r2_scale_parity.txt) x 2:
-#   fp32: slab 2 layers ..., 15 layers ...;  bf16 (vs the fp32 oracle): slab 5.2e-2 / 8.8e-2 / 9.5e-2 (v, e, worst weight),
+#   fp32: slab 2 layers 1.84e-4 / 3.09e-4 / 3.33e-4 (v, e, worst weight), 15 layers 1.45e-3 / 1.53e-3 / 3.52e-3 (one B200, 1000 W power
+#   limit; the fp32 kernels themselves are held to 5e-5 in the max metric against float64 up to 1.5 M rows by tests/test_mlp_f32_gpu.py);
+#   bf16 (vs the fp32 oracle): slab 5.2e-2 / 8.8e-2 / 9.5e-2 (v, e, worst weight),
 #   15 layers 1.24e-1 / 1.41e-1 / 1.79e-1, cfg5 one layer (vs our fp32 kernels) 4.2e-2 / 8.3e-2 / 1.0e-1.
 # The bf16 kernels themselves are pinned much tighter (1.5e-2) against an emulation with the same rounding points, at the full
 # cfg5 size too (test_cfg5_full_mesh_edge_kernels_vs_bf16_emulation).
-GRAD_L2 = {"fp32": {"slab": 1e-2, "deep": 2e-2}, "bf16": {"slab": 0.18, "deep": 0.36, "cfg5": 0.2, "small": 0.3}}
+GRAD_L2 = {"fp32": {"slab": 6.7e-4, "deep": 7.1e-3}, "bf16": {"slab": 0.18, "deep": 0.36, "cfg5": 0.2, "small": 0.3}}
 
 
 def _processor(arch, aggregator, layers, edge_sets, weights, precision):
