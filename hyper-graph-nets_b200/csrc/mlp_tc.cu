@@ -764,6 +764,28 @@ int tc_pair_wgrad(int64_t rows, const void* Ga, const void* Za, const void* Gb, 
   return HGN_OK;
 }
 
+// dW2 = G2^T H2, dW1 = G1^T H1 and dW0 = G0^T X over one slab of a one-chunk MLP whose data-gradient pass runs elsewhere (the encoder
+// and decoder kernels of io_mlp_tc.cu): per-part fp32 partials [parts][3][128][128], z = 0: W0, 1: W1, 2: W2.  X is [*, 128] bf16,
+// row r of the slab read from row r + x_row_offset.
+int tc_io_wgrad(int64_t rows, int64_t slab0, int64_t slab_rows, int parts, const void* X, int64_t x_row_offset, const void* G2, const void* H2,
+                const void* G1, const void* H1, const void* G0, float* partial, int accumulate, cudaStream_t st) {
+  if (int rc = configure_kernels()) return rc;
+  WgradArgs wa{};
+  wa.G2 = static_cast<const __nv_bfloat16*>(G2); wa.H2 = static_cast<const __nv_bfloat16*>(H2);
+  wa.G1 = static_cast<const __nv_bfloat16*>(G1); wa.H1 = static_cast<const __nv_bfloat16*>(H1);
+  wa.G0 = static_cast<const __nv_bfloat16*>(G0);
+  wa.partial = partial; wa.n_z = 3; wa.accumulate = accumulate;
+  hgn_chunks ch{};
+  ch.n_chunks = 1; ch.src[0] = X; ch.idx[0] = nullptr; ch.row_offset[0] = x_row_offset;
+  const int64_t this_rows = rows - slab0 < slab_rows ? rows - slab0 : slab_rows;
+  const int64_t rpp = ceil_div(ceil_div(this_rows > 0 ? this_rows : 1, parts), kWgRows) * kWgRows;
+  const size_t wg_smem = size_t(kWgStages) * kWgStageBytes + 64;
+  HGN_TIMED("mlp_wgrad_tc", st);
+  mlp_wgrad_tc_kernel<<<dim3(unsigned(parts), 2), kWgThreads, wg_smem, st>>>(rows, slab0, slab_rows, rpp, ch, wa);
+  HGN_LAUNCH_OK("io_wgrad_tc");
+  return HGN_OK;
+}
+
 struct BwdLayoutTc {
   int64_t slab_rows, parts, rows_per_part;
   int groups, n_z;

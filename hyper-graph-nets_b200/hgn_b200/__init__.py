@@ -6,7 +6,7 @@
 ``install_as_reference_modules()`` aliases this package as ``src.migration.*`` / ``src.util`` hot-path
 symbols so the reference's own system models (``FlagModel`` ...) run on it unchanged.
 """
-from .config import precision, set_precision  # noqa: F401
+from .config import io_kernels, precision, set_io_kernels, set_precision  # noqa: F401
 
 
 def invalidate_packed_weights() -> None:

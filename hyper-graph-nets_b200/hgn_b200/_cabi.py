@@ -14,6 +14,7 @@ HGN_F32 = 0
 HGN_BF16 = 1
 AGG_SUM, AGG_MEAN, AGG_MAX, AGG_MIN = 1, 2, 4, 8
 HGN_MAX_CHUNKS = 24
+HGN_IO_ENCODER, HGN_IO_DECODER = 0, 1
 ABI_VERSION = 6            # HGN_B200_ABI_VERSION of include/hgn_b200.h these signatures were written against
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libhgn_b200.so")
@@ -63,6 +64,14 @@ SIGNATURES = {
     "hgn_mlp_backward_workspace_bytes": (c_size_t, [c_int, c_int64, c_int32]),
     "hgn_mlp_backward": (c_int, [c_int, c_int64, POINTER(Chunks), c_void_p, c_void_p, c_int32, POINTER(c_void_p)]
                          + [c_void_p] * 8 + [c_void_p, c_size_t, c_void_p]),
+    "hgn_io_mlp_packed_bytes": (c_size_t, []),
+    "hgn_io_mlp_pack": (c_int, [c_int32, c_int32] + [c_void_p] * 8 + [c_void_p, c_void_p]),
+    "hgn_encoder_forward": (c_int, [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hgn_encoder_backward_workspace_bytes": (c_size_t, [c_int64, c_int32]),
+    "hgn_encoder_backward": (c_int, [c_int64, c_int32] + [c_void_p] * 12 + [c_void_p, c_size_t, c_void_p]),
+    "hgn_decoder_forward": (c_int, [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hgn_decoder_backward_workspace_bytes": (c_size_t, [c_int64, c_int32]),
+    "hgn_decoder_backward": (c_int, [c_int64, c_int32] + [c_void_p] * 10 + [c_void_p, c_size_t, c_void_p]),
     "hgn_edge_project_forward": (c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hgn_edge_project_backward_workspace_bytes": (c_size_t, [c_int, c_int64]),
     "hgn_edge_project_backward": (c_int, [c_int, c_int64] + [c_void_p] * 7 + [c_void_p, c_size_t, c_void_p]),

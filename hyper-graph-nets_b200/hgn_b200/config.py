@@ -32,3 +32,28 @@ def set_edge_storage(value: str) -> None:
     if value not in ('reference', 'receiver_sorted'):
         raise ValueError("edge storage must be 'reference' or 'receiver_sorted'")
     _edge_storage = value
+
+
+_io_kernels = os.environ.get('HGN_B200_IO_KERNELS', '')
+
+
+def _parse_switch(value) -> bool:
+    if isinstance(value, bool):
+        return value
+    text = str(value).strip().lower()
+    if text in ('1', 'true', 'on', 'yes'):
+        return True
+    if text in ('', '0', 'false', 'off', 'no'):
+        return False
+    raise ValueError(f"HGN_B200_IO_KERNELS must be one of 1/0, true/false, on/off, yes/no: got {value!r}")
+
+
+def io_kernels() -> bool:
+    """Whether the encoder and decoder MLPs run on the bf16 tcgen05 kernels (off by default).  It takes effect only where the
+    precision resolves to 'bf16'; the fp32 parity mode always keeps the torch MLPs."""
+    return _parse_switch(_io_kernels)
+
+
+def set_io_kernels(value: bool) -> None:
+    global _io_kernels
+    _io_kernels = _parse_switch(value)

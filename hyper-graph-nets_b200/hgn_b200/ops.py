@@ -139,7 +139,25 @@ def invalidate_packed_weights() -> None:
 def _pack_weights(cache: dict, dtype: torch.dtype, n_chunks: int, params: Sequence[torch.Tensor]) -> torch.Tensor:
     """Layout/precision conversion of the eight parameter tensors, redone only when a parameter changed
     (optimizer steps bump ``_version``)."""
-    key = (dtype, n_chunks)
+    def pack():
+        lib = _cabi.load()
+        code = _cabi.dtype_code(dtype)
+        blob = torch.empty(lib.hgn_mlp_packed_bytes(code, n_chunks), dtype=torch.uint8, device=params[0].device)
+        ps = _master_weights(params)
+        _cabi.check(lib.hgn_mlp_pack(code, n_chunks, *[p.data_ptr() for p in ps], blob.data_ptr(), _cabi.stream_ptr()), "hgn_mlp_pack")
+        return blob
+    return _cached_blob(cache, (dtype, n_chunks), params, pack)
+
+
+def _master_weights(params: Sequence[torch.Tensor]) -> List[torch.Tensor]:
+    ps = [p.detach().contiguous() for p in params]
+    if any(p.dtype != torch.float32 for p in ps):
+        raise _cabi.HgnError("MLP parameters must be float32 (master weights)")
+    return ps
+
+
+def _cached_blob(cache: dict, key, params: Sequence[torch.Tensor], pack) -> torch.Tensor:
+    """``pack()`` (one pack kernel), redone only when a parameter changed (optimizer steps bump ``_version``)."""
     versions = (_PACK_EPOCH[0],) + tuple((p.data_ptr(), p._version) for p in params)
     hit = cache.get(key)
     # While a CUDA graph is being captured the pack kernel always becomes part of the graph: a replay must re-read the master
@@ -147,13 +165,7 @@ def _pack_weights(cache: dict, dtype: torch.dtype, n_chunks: int, params: Sequen
     capturing = torch.cuda.is_current_stream_capturing()
     if hit is not None and hit[0] == versions and not capturing:
         return hit[1]
-    lib = _cabi.load()
-    code = _cabi.dtype_code(dtype)
-    blob = torch.empty(lib.hgn_mlp_packed_bytes(code, n_chunks), dtype=torch.uint8, device=params[0].device)
-    ps = [p.detach().contiguous() for p in params]
-    if any(p.dtype != torch.float32 for p in ps):
-        raise _cabi.HgnError("MLP parameters must be float32 (master weights)")
-    _cabi.check(lib.hgn_mlp_pack(code, n_chunks, *[p.data_ptr() for p in ps], blob.data_ptr(), _cabi.stream_ptr()), "hgn_mlp_pack")
+    blob = pack()
     _count()
     if not capturing:
         cache[key] = (versions, blob)
@@ -686,3 +698,137 @@ def colsum(x: torch.Tensor) -> torch.Tensor:
                                    _cabi.stream_ptr()), "hgn_colsum")
     _count(2)
     return out
+
+
+# ------------------------------------------------------------------------------------------------
+# encoder / decoder MLPs (bf16 tcgen05, csrc/io_mlp_tc.cu): raw fp32 features -> bf16 latents, bf16 latents -> fp32 outputs
+# ------------------------------------------------------------------------------------------------
+IO_ENCODER, IO_DECODER = 0, 1
+IO_MAX_OUT = 16
+_IO_SLAB_ROWS = 1 << 21          # rows per backward pass (io_bwd_layout)
+
+
+def _io_backward_launches(rows: int) -> int:
+    """Kernels of one hgn_encoder_backward / hgn_decoder_backward: per pass the data-gradient kernel (rows > 0), the weight-gradient
+    GEMMs and the two colsum5 kernels; then one reduction."""
+    passes = max(1, -(-rows // _IO_SLAB_ROWS))
+    return passes * (3 + int(rows > 0)) + 1
+
+
+def io_mlp_pack(cache: dict, kind: int, width: int, params: Sequence[torch.Tensor]) -> torch.Tensor:
+    """Packed bf16 blob of an encoder (``width`` = K, eight tensors) or decoder (``width`` = n_out, six tensors) MLP."""
+    def pack():
+        lib = _cabi.load()
+        blob = torch.empty(lib.hgn_io_mlp_packed_bytes(), dtype=torch.uint8, device=params[0].device)
+        ps = _master_weights(params)
+        gamma_beta = [p.data_ptr() for p in ps[6:8]] if kind == IO_ENCODER else [None, None]
+        _cabi.check(lib.hgn_io_mlp_pack(kind, width, *[p.data_ptr() for p in ps[:6]], *gamma_beta, blob.data_ptr(), _cabi.stream_ptr()),
+                    "hgn_io_mlp_pack")
+        return blob
+    return _cached_blob(cache, ("io", kind, width), params, pack)
+
+
+class _EncoderMLP(torch.autograd.Function):
+    """``LN(W2 relu(W1 relu(W0 x + b0) + b1) + b2)`` of raw fp32 features ``x[R, K]`` -> bf16 ``[R, 128]``."""
+
+    @staticmethod
+    def forward(ctx, x, packed, W0, b0, W1, b1, W2, b2, gamma, beta):
+        rows, k = x.shape
+        out = torch.empty((rows, D_LATENT), dtype=torch.bfloat16, device=x.device)
+        with torch.cuda.device(x.device):
+            _cabi.check(_cabi.load().hgn_encoder_forward(rows, k, _cabi.ptr(x), packed.data_ptr(), _cabi.ptr(out), _cabi.stream_ptr()),
+                        "hgn_encoder_forward")
+        _count(int(rows > 0))    # one io_mlp_tc_kernel
+        ctx.save_for_backward(x)
+        ctx.packed = packed
+        ctx.param_shapes = [tuple(p.shape) for p in (W0, b0, W1, b1, W2, b2, gamma, beta)]
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (x,) = ctx.saved_tensors
+        rows, k = x.shape
+        dev = x.device
+        lib = _cabi.load()
+        grad_out = grad_out.contiguous().to(torch.bfloat16)
+        grad_x = torch.empty_like(x) if ctx.needs_input_grad[0] else None
+        gparams = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes]
+        with torch.cuda.device(dev):
+            ws_bytes = lib.hgn_encoder_backward_workspace_bytes(rows, k)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _cabi.check(lib.hgn_encoder_backward(rows, k, _cabi.ptr(x), ctx.packed.data_ptr(), _cabi.ptr(grad_out), _cabi.ptr(grad_x),
+                                                 *[g.data_ptr() for g in gparams], ws.data_ptr(), ws_bytes, _cabi.stream_ptr()),
+                        "hgn_encoder_backward")
+        _count(_io_backward_launches(rows))
+        return (grad_x, None, *gparams)
+
+
+class _DecoderMLP(torch.autograd.Function):
+    """``W2 relu(W1 relu(W0 x + b0) + b1) + b2`` of bf16 latents ``x[N, 128]`` -> fp32 ``[N, n_out]``."""
+
+    @staticmethod
+    def forward(ctx, x, packed, W0, b0, W1, b1, W2, b2):
+        rows, n_out = x.shape[0], W2.shape[0]
+        out = torch.empty((rows, n_out), dtype=torch.float32, device=x.device)
+        with torch.cuda.device(x.device):
+            _cabi.check(_cabi.load().hgn_decoder_forward(rows, n_out, _cabi.ptr(x), packed.data_ptr(), _cabi.ptr(out), _cabi.stream_ptr()),
+                        "hgn_decoder_forward")
+        _count(int(rows > 0))    # one io_mlp_tc_kernel
+        ctx.save_for_backward(x)
+        ctx.packed = packed
+        ctx.n_out = n_out
+        ctx.param_shapes = [tuple(p.shape) for p in (W0, b0, W1, b1, W2, b2)]
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (x,) = ctx.saved_tensors
+        rows, dev = x.shape[0], x.device
+        lib = _cabi.load()
+        grad_out = grad_out.contiguous().to(torch.float32)
+        grad_x = torch.empty_like(x)
+        gparams = [torch.empty(shape, dtype=torch.float32, device=dev) for shape in ctx.param_shapes]
+        with torch.cuda.device(dev):
+            ws_bytes = lib.hgn_decoder_backward_workspace_bytes(rows, ctx.n_out)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _cabi.check(lib.hgn_decoder_backward(rows, ctx.n_out, _cabi.ptr(x), ctx.packed.data_ptr(), _cabi.ptr(grad_out), _cabi.ptr(grad_x),
+                                                 *[g.data_ptr() for g in gparams], ws.data_ptr(), ws_bytes, _cabi.stream_ptr()),
+                        "hgn_decoder_backward")
+        _count(_io_backward_launches(rows))
+        return (grad_x, None, *gparams)
+
+
+def encoder_mlp(params: Sequence[torch.Tensor], packed_cache: dict, x: torch.Tensor) -> torch.Tensor:
+    """bf16 ``[R, 128]`` latents of raw fp32 features ``x[R, K]`` (1 <= K <= 128) through the eight tensors of a reference encoder
+    MLP ``Sequential(LazyMLP([128, 128, 128]), LayerNorm(128))``."""
+    _cabi.require_cuda(x)
+    if x.dtype != torch.float32 or x.dim() != 2:
+        raise _cabi.HgnError(f"encoder kernel takes fp32 [rows, K] features: got {x.dtype} {tuple(x.shape)}")
+    k = x.shape[1]
+    W0, b0, W1, b1, W2, b2, gamma, beta = params
+    if not 1 <= k <= D_LATENT or W0.shape != (D_LATENT, k) or W1.shape != (D_LATENT, D_LATENT) or W2.shape != (D_LATENT, D_LATENT) \
+            or any(p.shape != (D_LATENT,) for p in (b0, b1, b2, gamma, beta)):
+        raise _cabi.HgnError(f"encoder kernel is specialised for 1 <= K <= 128 inputs and latent 128: got K={k}, W0 {tuple(W0.shape)}, "
+                             f"W1 {tuple(W1.shape)}, W2 {tuple(W2.shape)}")
+    x = x.contiguous()
+    with torch.cuda.device(x.device):
+        packed = io_mlp_pack(packed_cache, IO_ENCODER, k, params)
+    return _EncoderMLP.apply(x, packed, *params)
+
+
+def decoder_mlp(params: Sequence[torch.Tensor], packed_cache: dict, x: torch.Tensor) -> torch.Tensor:
+    """fp32 ``[N, n_out]`` outputs (1 <= n_out <= 16) of bf16 latents ``x[N, 128]`` through the six tensors of a reference decoder
+    MLP ``LazyMLP([128, 128, n_out])``."""
+    _cabi.require_cuda(x)
+    if x.dtype != torch.bfloat16 or x.dim() != 2 or x.shape[1] != D_LATENT:
+        raise _cabi.HgnError(f"decoder kernel takes bf16 [rows, 128] latents: got {x.dtype} {tuple(x.shape)}")
+    W0, b0, W1, b1, W2, b2 = params
+    n_out = W2.shape[0]
+    if not 1 <= n_out <= IO_MAX_OUT or W0.shape != (D_LATENT, D_LATENT) or W1.shape != (D_LATENT, D_LATENT) \
+            or W2.shape != (n_out, D_LATENT) or b0.shape != (D_LATENT,) or b1.shape != (D_LATENT,) or b2.shape != (n_out,):
+        raise _cabi.HgnError(f"decoder kernel is specialised for latent 128 and 1 <= n_out <= {IO_MAX_OUT}: got W0 {tuple(W0.shape)}, "
+                             f"W1 {tuple(W1.shape)}, W2 {tuple(W2.shape)}")
+    x = x.contiguous()
+    with torch.cuda.device(x.device):
+        packed = io_mlp_pack(packed_cache, IO_DECODER, n_out, params)
+    return _DecoderMLP.apply(x, packed, *params)

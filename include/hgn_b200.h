@@ -166,6 +166,39 @@ int hgn_mlp_backward(int dtype, int64_t rows, const hgn_chunks* chunks, const vo
                      float* grad_W2, float* grad_b2, float* grad_gamma, float* grad_beta,
                      void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- encoder / decoder MLPs (bf16 tcgen05, fp32 TMEM accumulators; opt-in in the Python layer) ---------------
+ * The reference's _make_mlp with num_layers = 2 (src/migration/meshgraphnet.py:93-108) on either side of the processor
+ * (encoder.py, decoder.py):
+ *   encoder  out[R,128] bf16 = LayerNorm(W2 relu(W1 relu(W0 x + b0) + b1) + b2) * gamma + beta,  x fp32 [R,K], 1 <= K <= 128
+ *   decoder  out[N,n_out] fp32 = W2 relu(W1 relu(W0 x + b0) + b1) + b2,                          x bf16 [N,128], 1 <= n_out <= 16
+ * No residual.  Weights are the nn.Linear tensors: encoder W0[128,K], decoder W2[n_out,128] and b2[n_out], the rest [128,128] /
+ * [128]; hgn_io_mlp_pack stages them (bf16, zero-padded; `width` = K for the encoder, n_out for the decoder; gamma / beta may be
+ * NULL for the decoder).  The forward / backward calls take the same `width` the blob was packed with.
+ * Rounding points: x (encoder) and the weights are rounded to bf16; each hidden layer is fp32 sum + bias + ReLU rounded to bf16;
+ * the encoder's LayerNorm runs in fp32 on acc + b2 and its output is rounded once to bf16; the decoder's output is acc + b2 in
+ * fp32.  Backward: the decoder's upstream gradient is rounded to bf16 (it becomes an MMA operand); the chain follows the MLP tile's
+ * rounding points; the encoder's grad_x[R,K] is fp32 (NULL = not requested), the decoder's grad_x[N,128] bf16 is required.  Weight,
+ * bias, gamma and beta gradients are fp32 in the parameter shapes, overwritten, reduced in a fixed order (bitwise reproducible).
+ * rows == 0 is valid: nothing is written by the forward and the backward writes exactly zero parameter gradients. */
+enum { HGN_IO_ENCODER = 0, HGN_IO_DECODER = 1 };
+#define HGN_IO_MAX_OUT 16
+size_t hgn_io_mlp_packed_bytes(void);
+int hgn_io_mlp_pack(int32_t kind, int32_t width,
+                    const float* W0, const float* b0, const float* W1, const float* b1,
+                    const float* W2, const float* b2, const float* gamma, const float* beta,
+                    void* packed, void* stream);
+int hgn_encoder_forward(int64_t rows, int32_t k_in, const float* x, const void* packed, void* out, void* stream);
+size_t hgn_encoder_backward_workspace_bytes(int64_t rows, int32_t k_in);
+int hgn_encoder_backward(int64_t rows, int32_t k_in, const float* x, const void* packed, const void* grad_out, float* grad_x,
+                         float* grad_W0, float* grad_b0, float* grad_W1, float* grad_b1,
+                         float* grad_W2, float* grad_b2, float* grad_gamma, float* grad_beta,
+                         void* workspace, size_t workspace_bytes, void* stream);
+int hgn_decoder_forward(int64_t rows, int32_t n_out, const void* x, const void* packed, float* out, void* stream);
+size_t hgn_decoder_backward_workspace_bytes(int64_t rows, int32_t n_out);
+int hgn_decoder_backward(int64_t rows, int32_t n_out, const void* x, const void* packed, const float* grad_out, void* grad_x,
+                         float* grad_W0, float* grad_b0, float* grad_W1, float* grad_b1, float* grad_W2, float* grad_b2,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- projected edge update (HGN_BF16 only; HGN_F32 returns HGN_ERR_UNSUPPORTED: use hgn_mlp_* there) --------
  * The edge update of src/migration/graphnet.py:22-32 with the first linear split by input block,
  * W0 = [Ws | Wr | We] (columns 0:128 | 128:256 | 256:384 of edge_models.<set>.0.layers.linear_0.weight):
