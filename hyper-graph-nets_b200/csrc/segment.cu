@@ -325,6 +325,8 @@ static int segment_reduce_impl(const T* data, int64_t E, int32_t D, const int32_
 // Backward of sum / mean / max / min over 128-wide bf16 rows, organised by SEGMENT: half a warp loads the segment's gradient rows
 // (and arg rows) once and writes the gradient row of each of its elements (256 B, fully coalesced per element).  The per-element
 // kernel above re-reads 2 KB of per-segment data for every element; on a triangle mesh (6 elements per segment) that is 6x the traffic.
+// segment_long_bwd_kernel<false> (segment_long.cu) restates this per-element arithmetic for long segments with explicit intrinsics,
+// including the fused multiply-add nvcc makes of `base[i] += f[i] * inv`: a change here, or to that contraction, changes both.
 __global__ void __launch_bounds__(256)
 segment_bwd_bf16_128_kernel(const int32_t* __restrict__ perm, const int32_t* __restrict__ rowptr, int64_t S,
                             const __nv_bfloat16* __restrict__ g_sum, const __nv_bfloat16* __restrict__ g_mean,

@@ -30,6 +30,12 @@ class Chunks(ctypes.Structure):
     ]
 
 
+class SegmentSplit(ctypes.Structure):
+    """``hgn_segment_split`` (include/hgn_b200.h)."""
+    _fields_ = [("num_segments", c_int64), ("num_elements", c_int64), ("n_long", c_int64), ("n_pieces", c_int64), ("n_short", c_int64),
+                ("long_ids", c_void_p), ("piece_ptr", c_void_p), ("pieces", c_void_p), ("perm_short", c_void_p), ("rowptr_short", c_void_p)]
+
+
 HGN_MAX_PEERS = 16
 
 
@@ -57,6 +63,21 @@ SIGNATURES = {
     "hgn_segment_reduce_bwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "hgn_segment_layer_grad": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_int64] + [c_void_p] * 9 + [c_void_p]),
+    "hgn_segment_split_threshold": (c_int32, []),
+    "hgn_segment_split_piece": (c_int32, []),
+    "hgn_segment_split_build_workspace_bytes": (c_size_t, [c_int64, c_int64]),
+    "hgn_segment_split_max_long": (c_int64, [c_int64, c_int64]),
+    "hgn_segment_split_max_pieces": (c_int64, [c_int64]),
+    "hgn_segment_split_build": (c_int, [c_void_p, c_void_p, c_int64, c_int64] + [c_void_p] * 5 + [POINTER(c_int64), c_void_p, c_size_t, c_void_p]),
+    "hgn_segment_split_reduce_workspace_bytes": (c_size_t, [POINTER(SegmentSplit)]),
+    "hgn_segment_reduce_split": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit)]
+                                 + [c_void_p] * 6 + [c_int, c_void_p, c_size_t, c_void_p]),
+    "hgn_segment_sum_pair_split": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit), c_void_p,
+                                           c_void_p, c_void_p, c_int64, POINTER(SegmentSplit), c_void_p, c_void_p, c_size_t, c_void_p]),
+    "hgn_segment_reduce_bwd_split": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit)]
+                                     + [c_void_p] * 7 + [c_void_p]),
+    "hgn_segment_layer_grad_split": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit)]
+                                     + [c_void_p] * 9 + [c_void_p]),
     "hgn_multi_segment_sum": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
     "hgn_mlp_packed_bytes": (c_size_t, [c_int, c_int32]),
     "hgn_mlp_pack": (c_int, [c_int, c_int32] + [c_void_p] * 8 + [c_void_p, c_void_p]),

@@ -61,12 +61,16 @@ class _SegmentAggregate(torch.autograd.Function):
             outs[name] = torch.empty(out_shape, dtype=x.dtype, device=x.device) if mask & bit else None
         argmax = torch.empty(out_shape, dtype=torch.int32, device=x.device) if (need_arg and mask & AGG_MAX) else None
         argmin = torch.empty(out_shape, dtype=torch.int32, device=x.device) if (need_arg and mask & AGG_MIN) else None
+        split = _split_of(plan, S, E) if x.dtype == torch.bfloat16 and D == D_LATENT else None
         with torch.cuda.device(x.device):
-            _cabi.check(lib.hgn_segment_reduce(
-                _cabi.dtype_code(x.dtype), x.data_ptr(), E, D, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S,
-                _cabi.ptr(outs["sum"]), _cabi.ptr(outs["mean"]), _cabi.ptr(outs["max"]), _cabi.ptr(outs["min"]),
-                _cabi.ptr(argmax), _cabi.ptr(argmin), 0, _cabi.stream_ptr()), "hgn_segment_reduce")
-        _count()
+            if split is None:
+                _cabi.check(lib.hgn_segment_reduce(
+                    _cabi.dtype_code(x.dtype), x.data_ptr(), E, D, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S,
+                    _cabi.ptr(outs["sum"]), _cabi.ptr(outs["mean"]), _cabi.ptr(outs["max"]), _cabi.ptr(outs["min"]),
+                    _cabi.ptr(argmax), _cabi.ptr(argmin), 0, _cabi.stream_ptr()), "hgn_segment_reduce")
+                _count()
+            else:
+                _reduce_split(x, plan, split, [outs[name] for name in OP_BITS], argmax, argmin)
         ctx.plan, ctx.mask, ctx.D, ctx.E = plan, mask, D, E
         ctx.in_shape = tuple(x.shape)
         ctx.save_for_backward(*[t for t in (argmax, argmin) if t is not None])
@@ -87,12 +91,20 @@ class _SegmentAggregate(torch.autograd.Function):
             g[name] = gi.contiguous() if gi is not None else None
         ref = next(t for t in g.values() if t is not None)
         grad = torch.empty(ctx.in_shape, dtype=ref.dtype, device=ref.device)
+        split = _split_of(plan, plan.num_segments, ctx.E) if ref.dtype == torch.bfloat16 and ctx.D == D_LATENT else None
         with torch.cuda.device(ref.device):
-            _cabi.check(lib.hgn_segment_reduce_bwd(
-                _cabi.dtype_code(ref.dtype), ctx.E, ctx.D, plan.ids32.data_ptr(), plan.perm.data_ptr(), plan.rowptr.data_ptr(),
-                plan.num_segments, _cabi.ptr(g["sum"]), _cabi.ptr(g["mean"]), _cabi.ptr(g["max"]), _cabi.ptr(g["min"]),
-                _cabi.ptr(argmax), _cabi.ptr(argmin), grad.data_ptr(), 0, _cabi.stream_ptr()), "hgn_segment_reduce_bwd")
-        _count()
+            if split is None:
+                _cabi.check(lib.hgn_segment_reduce_bwd(
+                    _cabi.dtype_code(ref.dtype), ctx.E, ctx.D, plan.ids32.data_ptr(), plan.perm.data_ptr(), plan.rowptr.data_ptr(),
+                    plan.num_segments, _cabi.ptr(g["sum"]), _cabi.ptr(g["mean"]), _cabi.ptr(g["max"]), _cabi.ptr(g["min"]),
+                    _cabi.ptr(argmax), _cabi.ptr(argmin), grad.data_ptr(), 0, _cabi.stream_ptr()), "hgn_segment_reduce_bwd")
+                _count()
+            else:
+                _cabi.check(lib.hgn_segment_reduce_bwd_split(
+                    _BF, ctx.E, D_LATENT, plan.ids32.data_ptr(), plan.perm.data_ptr(), plan.rowptr.data_ptr(), plan.num_segments,
+                    ctypes.byref(split.c), _cabi.ptr(g["sum"]), _cabi.ptr(g["mean"]), _cabi.ptr(g["max"]), _cabi.ptr(g["min"]),
+                    _cabi.ptr(argmax), _cabi.ptr(argmin), grad.data_ptr(), _cabi.stream_ptr()), "hgn_segment_reduce_bwd_split")
+                _count(2)       # hgn_segment_reduce_bwd_split: segment_bwd_bf16_128_kernel on the short CSR, segment_long_bwd_kernel
         return grad, None, None
 
 
@@ -372,9 +384,36 @@ def _node_update_backward(v, aggs, q1, q2, packed, grad_out, grad_v, grad_aggs, 
     _count(2 + 2 * ((k + 1) // 2) + k)
 
 
+def _split_of(plan: SegmentPlan, S: int, E: int):
+    """The plan's split, when the plan has one and the call covers all of its ``S`` segments and ``E`` elements; else ``None`` (the call
+    then runs exactly as without a split)."""
+    split = plan.split
+    return split if split is not None and S == plan.num_segments and E == plan.num_elements else None
+
+
+def _split_workspace(device, *splits) -> torch.Tensor:
+    lib = _cabi.load()
+    n = max(lib.hgn_segment_split_reduce_workspace_bytes(ctypes.byref(sp.c)) if sp is not None else 0 for sp in splits)
+    return torch.empty(max(n, 1), dtype=torch.uint8, device=device)
+
+
+def _reduce_split(data, plan: SegmentPlan, split, outs, argmax, argmin) -> None:
+    """``hgn_segment_reduce_split`` of bf16 rows of width 128 into ``outs`` = (sum, mean, max, min; None = not requested)."""
+    ws = _split_workspace(data.device, split)
+    _cabi.check(_cabi.load().hgn_segment_reduce_split(
+        _BF, data.data_ptr(), data.shape[0], D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(), plan.num_segments, ctypes.byref(split.c),
+        *[_cabi.ptr(o) for o in outs], _cabi.ptr(argmax), _cabi.ptr(argmin), 0, ws.data_ptr(), ws.numel(), _cabi.stream_ptr()),
+        "hgn_segment_reduce_split")
+    _count(3)                   # hgn_segment_reduce_split: one kernel on the short CSR, segment_long_partial, segment_long_combine
+
+
 def _segment_sum(data, plan: SegmentPlan, out) -> None:
     """``out[s] = sum of data's rows in segment s`` for the ``out.shape[0]`` segments of ``plan`` (bf16 rows of width 128)."""
     S = out.shape[0]
+    split = _split_of(plan, S, data.shape[0])
+    if split is not None:
+        _reduce_split(data, plan, split, [out, None, None, None], None, None)
+        return
     _cabi.check(_cabi.load().hgn_segment_reduce(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(),
                                                 S, out.data_ptr(), None, None, None, None, None, 0, _cabi.stream_ptr()),
                 "hgn_segment_reduce")
@@ -385,6 +424,10 @@ def _segment_reduce(data, plan: SegmentPlan, outs, argmax, argmin) -> None:
     """The reductions ``outs`` = (sum, mean, max, min; None = not requested) of ``data``'s bf16 rows of width 128 over the segments of
     ``plan``, with the max / min winners when ``argmax`` / ``argmin`` are given."""
     S = plan.num_segments
+    split = _split_of(plan, S, data.shape[0])
+    if split is not None:
+        _reduce_split(data, plan, split, outs, argmax, argmin)
+        return
     _cabi.check(_cabi.load().hgn_segment_reduce(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(),
                                                 S, *[_cabi.ptr(o) for o in outs], _cabi.ptr(argmax), _cabi.ptr(argmin), 0,
                                                 _cabi.stream_ptr()), "hgn_segment_reduce")
@@ -395,6 +438,15 @@ def _segment_layer_grad(plan: SegmentPlan, E: int, grads: dict, argmax, argmin, 
     """``agg_grad[r] = g_sum[r] + g_mean[r] / cnt_r`` and ``edge_grad[e] = base[e] + the max / min winners' gradients`` over the receiver
     plan (``grads``: reducer name -> gradient of that aggregate)."""
     S = plan.num_segments
+    split = _split_of(plan, S, E)
+    if split is not None:
+        _cabi.check(_cabi.load().hgn_segment_layer_grad_split(
+            _BF, E, D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S, ctypes.byref(split.c),
+            *[_cabi.ptr(grads.get(op)) for op in OP_BITS], _cabi.ptr(argmax), _cabi.ptr(argmin), _cabi.ptr(base), _cabi.ptr(agg_grad),
+            _cabi.ptr(edge_grad), _cabi.stream_ptr()), "hgn_segment_layer_grad_split")
+        # hgn_segment_layer_grad_split: segment_layer_grad_bf16_128_kernel on the short CSR, segment_long_bwd_kernel
+        _count(2 * int(agg_grad is not None or edge_grad is not None))
+        return
     _cabi.check(_cabi.load().hgn_segment_layer_grad(
         _BF, E, D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S, *[_cabi.ptr(grads.get(op)) for op in OP_BITS],
         _cabi.ptr(argmax), _cabi.ptr(argmin), _cabi.ptr(base), _cabi.ptr(agg_grad), _cabi.ptr(edge_grad), _cabi.stream_ptr()),
@@ -405,6 +457,18 @@ def _segment_layer_grad(plan: SegmentPlan, E: int, grads: dict, argmax, argmin, 
 def _segment_sum_pair(data, plan_a: SegmentPlan, out_a, plan_b: SegmentPlan, out_b) -> None:
     """Two ``_segment_sum``s of the same rows under two groupings."""
     S_a, S_b = out_a.shape[0], out_b.shape[0]
+    E = data.shape[0]
+    split_a, split_b = _split_of(plan_a, S_a, E), _split_of(plan_b, S_b, E)
+    if split_a is not None or split_b is not None:
+        ws = _split_workspace(data.device, split_a, split_b)
+        _cabi.check(_cabi.load().hgn_segment_sum_pair_split(
+            _BF, data.data_ptr(), E, D_LATENT, plan_a.perm.data_ptr(), plan_a.rowptr.data_ptr(), S_a,
+            ctypes.byref(split_a.c) if split_a is not None else None, out_a.data_ptr(), plan_b.perm.data_ptr(), plan_b.rowptr.data_ptr(), S_b,
+            ctypes.byref(split_b.c) if split_b is not None else None, out_b.data_ptr(), ws.data_ptr(), ws.numel(), _cabi.stream_ptr()),
+            "hgn_segment_sum_pair_split")
+        # hgn_segment_sum_pair_split: hgn_segment_sum_pair on the short CSRs, then segment_long_partial and _combine per split side
+        _count((1 if S_a > 0 and S_b > 0 else int(S_a > 0) + int(S_b > 0)) + 2 * (split_a is not None) + 2 * (split_b is not None))
+        return
     _cabi.check(_cabi.load().hgn_segment_sum_pair(_BF, data.data_ptr(), data.shape[0], D_LATENT, plan_a.perm.data_ptr(),
                                                   plan_a.rowptr.data_ptr(), S_a, out_a.data_ptr(), plan_b.perm.data_ptr(),
                                                   plan_b.rowptr.data_ptr(), S_b, out_b.data_ptr(), _cabi.stream_ptr()),

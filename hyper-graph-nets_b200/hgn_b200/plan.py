@@ -10,6 +10,7 @@ forward and by the deterministic gather backward.
 from __future__ import annotations
 
 from collections import OrderedDict
+import ctypes
 import os as _os
 import weakref as _weakref
 
@@ -19,14 +20,53 @@ from . import _cabi
 
 
 
+class SegmentSplit:
+    """The long segments of a CSR (more than ``hgn_segment_split_threshold()`` elements, cut into pieces of
+    ``hgn_segment_split_piece()`` perm positions) and the short CSR without them, as built by ``hgn_segment_split_build``.
+    ``c`` is the ``hgn_segment_split`` the ``*_split`` entry points take; the tensors it points into are held here."""
+
+    __slots__ = ("n_long", "n_pieces", "n_short", "long_ids", "piece_ptr", "pieces", "perm_short", "rowptr_short", "c", "nbytes")
+
+    def __init__(self, perm: torch.Tensor, rowptr: torch.Tensor, E: int, S: int):
+        lib = _cabi.load()
+        dev = rowptr.device
+        max_long = lib.hgn_segment_split_max_long(E, S)
+        i32 = dict(dtype=torch.int32, device=dev)
+        long_ids = torch.empty(max(max_long, 1), **i32)
+        piece_ptr = torch.empty(max_long + 1, **i32)
+        pieces = torch.empty(max(3 * lib.hgn_segment_split_max_pieces(E), 1), **i32)
+        perm_short = torch.empty(max(E, 1), **i32)
+        self.rowptr_short = torch.empty(S + 1, **i32)
+        ws_bytes = lib.hgn_segment_split_build_workspace_bytes(E, S)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        counts = (ctypes.c_int64 * 3)()
+        with torch.cuda.device(dev):
+            _cabi.check(lib.hgn_segment_split_build(perm.data_ptr(), rowptr.data_ptr(), E, S, long_ids.data_ptr(), piece_ptr.data_ptr(),
+                                                    pieces.data_ptr(), perm_short.data_ptr(), self.rowptr_short.data_ptr(), counts,
+                                                    ws.data_ptr(), ws_bytes, _cabi.stream_ptr()), "hgn_segment_split_build")
+        self.n_long, self.n_pieces, self.n_short = int(counts[0]), int(counts[1]), int(counts[2])
+        if self.n_long == 0:            # the plan keeps no split
+            return
+        # only what the counts cover is kept (clones: a slice would keep the bound-sized buffer alive)
+        self.long_ids = long_ids[:max(self.n_long, 1)].clone()
+        self.piece_ptr = piece_ptr[:self.n_long + 1].clone()
+        self.pieces = pieces[:max(3 * self.n_pieces, 1)].clone()
+        self.perm_short = perm_short[:max(self.n_short, 1)].clone()
+        self.c = _cabi.SegmentSplit(S, E, self.n_long, self.n_pieces, self.n_short, self.long_ids.data_ptr(), self.piece_ptr.data_ptr(),
+                                    self.pieces.data_ptr(), self.perm_short.data_ptr(), self.rowptr_short.data_ptr())
+        self.nbytes = _tensor_bytes(self.long_ids, self.piece_ptr, self.pieces, self.perm_short, self.rowptr_short)
+
+
 class SegmentPlan:
     """``ids`` with values in ``[0, num_segments)``.
 
     ``ids32``  int32 copy (gather index).
     ``perm``   element ids grouped by segment, ascending id inside a segment (stable).
-    ``rowptr`` ``rowptr[s]:rowptr[s+1]`` delimits segment ``s`` inside ``perm``."""
+    ``rowptr`` ``rowptr[s]:rowptr[s+1]`` delimits segment ``s`` inside ``perm``.
+    ``split``  ``None`` when no segment is long, else the ``SegmentSplit`` the bf16 / width-128 segment calls run on."""
 
-    __slots__ = ("_ids_ref", "_ids_own", "num_segments", "num_elements", "_perm", "_rowptr", "ids32", "version", "__weakref__")
+    __slots__ = ("_ids_ref", "_ids_own", "num_segments", "num_elements", "_perm", "_rowptr", "_split", "_cache_key", "ids32", "version",
+                 "__weakref__")
 
     def __init__(self, ids: torch.Tensor, num_segments: int):
         _cabi.require_cuda(ids)
@@ -41,6 +81,8 @@ class SegmentPlan:
         self.ids32 = ids.to(torch.int32).contiguous() if self.num_elements else torch.zeros(1, dtype=torch.int32, device=ids.device)
         self._perm = None
         self._rowptr = None
+        self._split = False          # not built yet
+        self._cache_key = None
 
     @property
     def ids(self) -> torch.Tensor:
@@ -77,6 +119,20 @@ class SegmentPlan:
         if self._rowptr is None:
             self._build_csr()
         return self._rowptr
+
+    @property
+    def split(self) -> "SegmentSplit | None":
+        """Built on first use (only the bf16 / width-128 segment bindings ask), so plans that never reach them -- fp32 parity mode, the
+        connector and graph builders -- pay nothing for it."""
+        if self._split is False:
+            if self._rowptr is None:
+                self._build_csr()
+            E = self.num_elements
+            split = SegmentSplit(self._perm, self._rowptr, E, self.num_segments) if E > _cabi.load().hgn_segment_split_threshold() else None
+            self._split = split if split is not None and split.n_long > 0 else None
+            if self._split is not None and self._cache_key is not None:
+                _grow(self._cache_key, self, self._split.nbytes)
+        return self._split
 
 
 # ---- cache -------------------------------------------------------------------------------------------------------------------
@@ -124,6 +180,18 @@ def _remember(key, sources, value, nbytes: int) -> None:
         _forget(next(iter(_plans)))
 
 
+def _grow(key, value, nbytes: int) -> None:
+    """Adds ``nbytes`` to the live entry ``key`` (when it still holds ``value``): a plan's split is sized when its CSR is built."""
+    global _plan_bytes
+    hit = _plans.get(key)
+    if hit is None or hit[2] is not value:
+        return
+    _plans[key] = hit[:3] + (hit[3] + int(nbytes),)
+    _plan_bytes += int(nbytes)
+    while _plan_bytes > _CACHE_BYTES and len(_plans) > 1:
+        _forget(next(iter(_plans)))
+
+
 def plan_cache_stats() -> dict:
     return {"entries": len(_plans), "bytes": _plan_bytes, "limit_bytes": _CACHE_BYTES}
 
@@ -136,6 +204,7 @@ def segment_plan(ids: torch.Tensor, num_segments: int) -> SegmentPlan:
     if hit is not None:
         return hit
     plan = SegmentPlan(ids, num_segments)
+    plan._cache_key = key
     # ids (int64, a private copy unless the caller's tensor already was contiguous int64) + ids32 + perm + rowptr
     # ids32 + perm + rowptr (+ a private int64 copy when the caller's tensor was not contiguous int64)
     _remember(key, (ids,), plan, ids.numel() * 8 + (int(num_segments) + 1) * 4 + (ids.numel() * 8 if plan._ids_own is not None else 0))

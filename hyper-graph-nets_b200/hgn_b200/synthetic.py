@@ -211,3 +211,36 @@ def processor_shapes(num_blocks: int, edge_sets: Sequence[str], aggregator: str 
         for name in edge_sets:
             shapes.update(mlp_shapes(f"{p}.edge_models.{name}", 3 * latent, latent, latent))
     return shapes
+
+
+# ----------------------------------------------------------------------------------------------
+# mesh-scale HyperGraphNet / HeteroGraphNet processors (their cluster segments are long)
+# ----------------------------------------------------------------------------------------------
+HYPER_EDGE_SETS = ("mesh_edges", "intra_cluster_to_cluster", "intra_cluster_to_mesh", "inter_cluster")
+
+
+def hyper_grid_edges(width: int, height: int, num_clusters: int) -> Dict[str, Tuple[torch.Tensor, torch.Tensor]]:
+    """(senders, receivers) of the four edge sets of a ``width x height`` grid mesh clustered into ``num_clusters`` bands of
+    consecutive node ids, with the remote sets of ``rmp.hierarchical_connector.connector_indices`` (hyper node j = row n + j)."""
+    from .rmp.hierarchical_connector import connector_indices
+    n = width * height
+    clusters = list(torch.arange(n, dtype=torch.int64).tensor_split(num_clusters))
+    sets = connector_indices(clusters, [], n, fully_connect=True)
+    return {"mesh_edges": grid_edges_two_way(width, height), **sets}
+
+
+def hyper_processor_shapes(architecture: str, aggregator: str, num_blocks: int, latent: int = 128) -> Dict[str, Tuple[int, ...]]:
+    """Shapes of a 'hyper' or 'hetero' processor over ``HYPER_EDGE_SETS``."""
+    k = 4 if aggregator == "pna" else 1
+    shapes: Dict[str, Tuple[int, ...]] = {}
+    for b in range(num_blocks):
+        p = f"processor.graphnet_blocks.{b}"
+        for name in HYPER_EDGE_SETS:
+            shapes.update(mlp_shapes(f"{p}.edge_models.{name}", 3 * latent, latent, latent))
+        if architecture == "hyper":
+            for m in ("node_model_cross", "hyper_node_model_up", "hyper_node_model_cross", "node_model_down"):
+                shapes.update(mlp_shapes(f"{p}.{m}", latent * (1 + k), latent, latent))
+        else:
+            for m in ("node_model_cross", "hyper_node_model_cross"):
+                shapes.update(mlp_shapes(f"{p}.{m}", latent * (1 + k * len(HYPER_EDGE_SETS)), latent, latent))
+    return shapes

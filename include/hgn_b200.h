@@ -109,6 +109,85 @@ int hgn_segment_layer_grad(int dtype, int64_t num_edges, int32_t D, const int32_
                            const int32_t* argmax, const int32_t* argmin, const void* base, void* agg_grad, void* edge_grad,
                            void* stream);
 
+/* ---- long segments: the split plan and its entry points (HGN_BF16, D = 128 only) -------------------------------------------
+ * The four calls above give one segment to half a warp or one warp.  A HyperGraphNet's cluster pooling (intra_cluster_to_cluster,
+ * receivers = the C hyper nodes) and broadcast (intra_cluster_to_mesh, senders = the hyper nodes) turn every cluster into one
+ * segment of ~N/C elements, which one thread group then walks one latency round at a time.  A segment is LONG when it has more than
+ * HGN_SEGMENT_SPLIT_THRESHOLD elements; it is cut into PIECES of HGN_SEGMENT_SPLIT_PIECE consecutive positions of perm (the last
+ * piece may be shorter), and every piece of a call is worked at once.  The short segments go through the calls above, unchanged,
+ * on the split's SHORT CSR (perm_short, rowptr_short): the plan's CSR with every long segment emptied and every short one keeping
+ * its elements in order.  So short segments get exactly the bits of the calls above.
+ *
+ * Arithmetic of a long segment (fp32, no atomics, bitwise reproducible):
+ *   piece partial p_k = sum from +0 of the piece's rows in perm order;  total = (((0 + p_0) + p_1) + ...) in ascending k;
+ *   sum  = bf16_rn(total), or bf16_rn(total + prior) with accumulate_sum (the prior added after the sum, as above);
+ *   mean = bf16_rn(total * (1.0f / cnt));
+ *   max / min and their winners = the sequential first-in-order result of hgn_segment_reduce, bit for bit (piece winners
+ *   combined in ascending order with strict comparisons);
+ *   the backward terms (hgn_segment_reduce_bwd_split, hgn_segment_layer_grad_split) are per element, with the arithmetic of the
+ *   calls they mirror, so they are bit-identical to them. */
+#define HGN_SEGMENT_SPLIT_THRESHOLD 2048
+#define HGN_SEGMENT_SPLIT_PIECE 256
+/* the two constants above, as built into the library */
+int32_t hgn_segment_split_threshold(void);
+int32_t hgn_segment_split_piece(void);
+
+typedef struct {
+  int64_t num_segments, num_elements;   /* S and E of the CSR it was built from */
+  int64_t n_long, n_pieces, n_short;
+  const int32_t* long_ids;              /* [n_long] ascending segment ids */
+  const int32_t* piece_ptr;             /* [n_long + 1]: the pieces of long_ids[i] are piece_ptr[i] .. piece_ptr[i+1]-1 */
+  const int32_t* pieces;                /* [n_pieces][3]: segment, begin, end (positions in perm), grouped by segment ascending */
+  const int32_t* perm_short;            /* [n_short] (a valid pointer even when n_short = 0) */
+  const int32_t* rowptr_short;          /* [S+1] */
+} hgn_segment_split;
+
+/* Builds a split from a CSR (perm[E], rowptr[S+1]) into caller buffers sized from bounds:
+ *   long_ids   >= hgn_segment_split_max_long(E, S) int32,      piece_ptr >= that + 1 int32,
+ *   pieces     >= 3 * hgn_segment_split_max_pieces(E) int32,    perm_short >= max(E, 1) int32,    rowptr_short = S + 1 int32.
+ * host_counts[3] receives n_long, n_pieces, n_short: the call reads them with one small device-to-host copy and synchronises the
+ * stream.  Everything is written whether or not a segment is long (with n_long = 0 the short CSR is the plan's own). */
+size_t hgn_segment_split_build_workspace_bytes(int64_t num_edges, int64_t num_segments);
+int64_t hgn_segment_split_max_long(int64_t num_edges, int64_t num_segments);
+int64_t hgn_segment_split_max_pieces(int64_t num_edges);
+int hgn_segment_split_build(const int32_t* perm, const int32_t* rowptr, int64_t num_edges, int64_t num_segments,
+                            int32_t* long_ids, int32_t* piece_ptr, int32_t* pieces, int32_t* perm_short, int32_t* rowptr_short,
+                            int64_t* host_counts, void* workspace, size_t workspace_bytes, void* stream);
+
+/* fp32 partials of the long pieces: the workspace of hgn_segment_reduce_split and hgn_segment_sum_pair_split (for the pair: the
+ * larger of the two sides' sizes; a NULL split needs none). */
+size_t hgn_segment_split_reduce_workspace_bytes(const hgn_segment_split* split);
+
+/* hgn_segment_reduce over a split plan: the short segments through hgn_segment_reduce on the short CSR, the long ones by pieces.
+ * Same outputs and conventions; (perm, rowptr) are the plan's own CSR. */
+int hgn_segment_reduce_split(int dtype, const void* data, int64_t num_edges, int32_t D,
+                             const int32_t* perm, const int32_t* rowptr, int64_t num_segments, const hgn_segment_split* split,
+                             void* out_sum, void* out_mean, void* out_max, void* out_min,
+                             int32_t* argmax, int32_t* argmin, int accumulate_sum,
+                             void* workspace, size_t workspace_bytes, void* stream);
+
+/* hgn_segment_sum_pair with a split on either side (NULL = that side has no long segment). */
+int hgn_segment_sum_pair_split(int dtype, const void* data, int64_t num_edges, int32_t D,
+                               const int32_t* perm_a, const int32_t* rowptr_a, int64_t num_segments_a,
+                               const hgn_segment_split* split_a, void* out_a,
+                               const int32_t* perm_b, const int32_t* rowptr_b, int64_t num_segments_b,
+                               const hgn_segment_split* split_b, void* out_b,
+                               void* workspace, size_t workspace_bytes, void* stream);
+
+/* hgn_segment_reduce_bwd over a split plan, segment-wise (perm required, grad_data overwritten). */
+int hgn_segment_reduce_bwd_split(int dtype, int64_t num_edges, int32_t D,
+                                 const int32_t* ids32, const int32_t* perm, const int32_t* rowptr, int64_t num_segments,
+                                 const hgn_segment_split* split,
+                                 const void* g_sum, const void* g_mean, const void* g_max, const void* g_min,
+                                 const int32_t* argmax, const int32_t* argmin, void* grad_data, void* stream);
+
+/* hgn_segment_layer_grad over a split plan; the agg_grad row of a long segment is written once. */
+int hgn_segment_layer_grad_split(int dtype, int64_t num_edges, int32_t D, const int32_t* perm, const int32_t* rowptr,
+                                 int64_t num_segments, const hgn_segment_split* split,
+                                 const void* g_sum, const void* g_mean, const void* g_max, const void* g_min,
+                                 const int32_t* argmax, const int32_t* argmin, const void* base, void* agg_grad, void* edge_grad,
+                                 void* stream);
+
 /* Backward of the row gathers v[senders], v[receivers] (torch.index_select -> index_add_ with float
  * atomics in the reference, src/migration/graphnet.py:28-29): out[n,:] = base[n,:] (if base != NULL)
  * + sum_k sum_{j in segment_k(n)} data_k[perm_k[j], :], accumulated in fp32 in a fixed order
