@@ -55,6 +55,52 @@ __global__ void halo_wait_kernel(hgn_halo_flags flags, int n_flags, uint32_t epo
   __threadfence_system();
 }
 
+// Cluster pooling across ranks: one 128-thread block per cluster, thread = feature; the ranks' rows are read in rank order.
+__global__ void __launch_bounds__(128)
+cluster_combine_kernel(const float* __restrict__ slots, int world, int rank, int64_t C, __nv_bfloat16* __restrict__ out_sum,
+                       __nv_bfloat16* __restrict__ out_mean, __nv_bfloat16* __restrict__ out_max, __nv_bfloat16* __restrict__ out_min,
+                       int32_t* __restrict__ argmax, int32_t* __restrict__ argmin, int32_t* __restrict__ count) {
+  constexpr int W = HGN_SEGMENT_PARTIAL_WIDTH;
+  const int c = threadIdx.x;
+  const int64_t k = blockIdx.x;
+  float t = 0.f, mx = 0.f, mn = 0.f;
+  int cnt = 0, wx = -1, wn = -1;
+  for (int r = 0; r < world; ++r) {
+    const float* row = slots + (int64_t(r) * C + k) * W;
+    const int n = __float_as_int(row[384]);
+    t = __fadd_rn(t, row[c]);
+    if (n == 0) continue;                       // a rank without a member of this cluster: its max / min are not values
+    cnt += n;
+    if (out_max || argmax) { const float a = row[128 + c]; if (wx < 0 || a > mx) { mx = a; wx = r; } }
+    if (out_min || argmin) { const float b = row[256 + c]; if (wn < 0 || b < mn) { mn = b; wn = r; } }
+  }
+  const int64_t o = k * 128 + c;
+  if (out_sum) out_sum[o] = __float2bfloat16_rn(t);
+  if (out_mean) out_mean[o] = __float2bfloat16_rn(__fmul_rn(t, 1.0f / float(max(cnt, 1))));
+  if (out_max) out_max[o] = __float2bfloat16_rn(mx);
+  if (out_min) out_min[o] = __float2bfloat16_rn(mn);
+  if (argmax && wx != rank) argmax[o] = -1;
+  if (argmin && wn != rank) argmin[o] = -1;
+  if (count && c == 0) count[k] = cnt;
+}
+
+__global__ void cluster_grad_sum_kernel(const __nv_bfloat16* __restrict__ slots, int world, int64_t n, __nv_bfloat16* __restrict__ out) {
+  const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  if (i >= n) return;
+  float t = 0.f;
+  for (int r = 0; r < world; ++r) t = __fadd_rn(t, __bfloat162float(slots[int64_t(r) * n + i]));
+  out[i] = __float2bfloat16_rn(t);
+}
+
+__global__ void cluster_mean_grad_kernel(const __nv_bfloat16* __restrict__ g_sum, const __nv_bfloat16* __restrict__ g_mean,
+                                         const int32_t* __restrict__ count, int64_t C, __nv_bfloat16* __restrict__ out) {
+  const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  if (i >= C * 128) return;
+  const float inv = 1.0f / float(max(count[i / 128], 1));
+  const float pre = __fadd_rn(0.f, g_sum ? __bfloat162float(g_sum[i]) : 0.f);
+  out[i] = __float2bfloat16_rn(__fmaf_rn(__bfloat162float(g_mean[i]), inv, pre));
+}
+
 }  // namespace hgn
 
 using namespace hgn;
@@ -118,5 +164,43 @@ extern "C" int hgn_halo_wait(const hgn_halo_flags* flags, int32_t n_flags, uint3
   HGN_TIMED("halo_wait", static_cast<cudaStream_t>(stream));
   halo_wait_kernel<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(*flags, n_flags, epoch, nullptr);
   HGN_LAUNCH_OK("halo_wait");
+  return HGN_OK;
+}
+
+extern "C" int hgn_cluster_combine(const float* slots, int32_t world, int32_t rank, int64_t C, void* out_sum, void* out_mean, void* out_max,
+                                   void* out_min, int32_t* argmax, int32_t* argmin, int32_t* count, void* stream) {
+  HGN_CHECK_ARG(world >= 1 && world <= HGN_MAX_PEERS && rank >= 0 && rank < world && C >= 0, "cluster_combine: world=%d rank=%d C=%lld",
+                world, rank, (long long)C);
+  HGN_CHECK_ARG(C == 0 || slots != nullptr, "cluster_combine: null slots");
+  if (C == 0) return HGN_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  HGN_TIMED("cluster_combine", st);
+  cluster_combine_kernel<<<unsigned(C), 128, 0, st>>>(slots, world, rank, C, static_cast<__nv_bfloat16*>(out_sum), static_cast<__nv_bfloat16*>(out_mean),
+                                                      static_cast<__nv_bfloat16*>(out_max), static_cast<__nv_bfloat16*>(out_min), argmax, argmin, count);
+  HGN_LAUNCH_OK("cluster_combine");
+  return HGN_OK;
+}
+
+extern "C" int hgn_cluster_grad_sum(int dtype, const void* slots, int32_t world, int64_t C, int32_t D, void* out, void* stream) {
+  HGN_CHECK_ARG(dtype == HGN_BF16, "cluster_grad_sum: dtype %d, only bf16 (%d) is supported", dtype, int(HGN_BF16));
+  HGN_CHECK_ARG(world >= 1 && world <= HGN_MAX_PEERS && C >= 0 && D > 0, "cluster_grad_sum: world=%d C=%lld D=%d", world, (long long)C, D);
+  HGN_CHECK_ARG(C == 0 || (slots && out), "cluster_grad_sum: null pointer");
+  const int64_t n = C * D;
+  if (n == 0) return HGN_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  HGN_TIMED("cluster_grad_sum", st);
+  cluster_grad_sum_kernel<<<unsigned(ceil_div(n, 256)), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(slots), world, n, static_cast<__nv_bfloat16*>(out));
+  HGN_LAUNCH_OK("cluster_grad_sum");
+  return HGN_OK;
+}
+
+extern "C" int hgn_cluster_mean_grad(const void* g_sum, const void* g_mean, const int32_t* count, int64_t C, void* out, void* stream) {
+  HGN_CHECK_ARG(C >= 0 && (C == 0 || (g_mean && count && out)), "cluster_mean_grad: null pointer");
+  if (C == 0) return HGN_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  HGN_TIMED("cluster_mean_grad", st);
+  cluster_mean_grad_kernel<<<unsigned(ceil_div(C * 128, 256)), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(g_sum), static_cast<const __nv_bfloat16*>(g_mean),
+                                                                           count, C, static_cast<__nv_bfloat16*>(out));
+  HGN_LAUNCH_OK("cluster_mean_grad");
   return HGN_OK;
 }

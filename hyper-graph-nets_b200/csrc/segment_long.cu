@@ -300,6 +300,81 @@ segment_long_bwd_kernel(const int32_t* __restrict__ perm, const int32_t* __restr
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// fp32 partials (hgn_segment_partials): the value each segment's result is rounded from, left unrounded
+// ------------------------------------------------------------------------------------------------
+constexpr int kPartialW = HGN_SEGMENT_PARTIAL_WIDTH;
+static_assert(kPartialW == 3 * 128 + 4 && (kPartialW * 4) % 16 == 0, "partial row: sum | max | min | count + padding, 16-byte rows");
+
+// One warp per segment of the (short) CSR, four features per lane: the sum from +0 in perm order (the order of
+// segment_sum_bf16_128_kernel and segment_reduce_vec_kernel), max / min with strict comparisons and their first-in-order winners,
+// and the element count.  An empty segment leaves 0, -inf, +inf, winners -1 and count 0.
+__global__ void __launch_bounds__(256)
+segment_partial_short_kernel(const __nv_bfloat16* __restrict__ data, const int32_t* __restrict__ perm, const int32_t* __restrict__ rowptr,
+                             int64_t S, int minmax, float* __restrict__ out, int32_t* __restrict__ argmax, int32_t* __restrict__ argmin) {
+  const int lane = threadIdx.x & 31;
+  const int64_t seg = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 5;
+  if (seg >= S) return;
+  const int beg = rowptr[seg], end = rowptr[seg + 1];
+  const int c = lane * 4;
+  float s[4] = {0.f, 0.f, 0.f, 0.f}, mx[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY}, mn[4] = {INFINITY, INFINITY, INFINITY, INFINITY};
+  int ax[4] = {-1, -1, -1, -1}, an[4] = {-1, -1, -1, -1};
+  for (int j = beg; j < end; ++j) {
+    const int e = __ldg(perm + j);
+    const uint2 p = __ldg(reinterpret_cast<const uint2*>(data + int64_t(e) * 128 + c));
+    const float f[4] = {__uint_as_float(p.x << 16), __uint_as_float(p.x & 0xFFFF0000u), __uint_as_float(p.y << 16),
+                        __uint_as_float(p.y & 0xFFFF0000u)};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      s[i] = __fadd_rn(s[i], f[i]);
+      if (minmax) {
+        if (f[i] > mx[i]) { mx[i] = f[i]; ax[i] = e; }
+        if (f[i] < mn[i]) { mn[i] = f[i]; an[i] = e; }
+      }
+    }
+  }
+  float* row = out + seg * kPartialW;
+  *reinterpret_cast<float4*>(row + c) = make_float4(s[0], s[1], s[2], s[3]);
+  if (minmax) {
+    *reinterpret_cast<float4*>(row + 128 + c) = make_float4(mx[0], mx[1], mx[2], mx[3]);
+    *reinterpret_cast<float4*>(row + 256 + c) = make_float4(mn[0], mn[1], mn[2], mn[3]);
+    if (argmax) *reinterpret_cast<int4*>(argmax + seg * 128 + c) = make_int4(ax[0], ax[1], ax[2], ax[3]);
+    if (argmin) *reinterpret_cast<int4*>(argmin + seg * 128 + c) = make_int4(an[0], an[1], an[2], an[3]);
+  }
+  if (lane == 0) *reinterpret_cast<int4*>(row + 384) = make_int4(end - beg, 0, 0, 0);
+}
+
+// segment_long_combine_kernel's combine (ascending piece order, sum from +0, strict comparisons), written unrounded with the count
+template <bool MINMAX>
+__global__ void __launch_bounds__(128)
+segment_long_partial_combine_kernel(const int32_t* __restrict__ long_ids, const int32_t* __restrict__ piece_ptr, const int32_t* __restrict__ rowptr,
+                                    const float* __restrict__ p_sum, const float* __restrict__ p_max, const float* __restrict__ p_min,
+                                    const int32_t* __restrict__ p_amx, const int32_t* __restrict__ p_amn, float* __restrict__ out,
+                                    int32_t* __restrict__ argmax, int32_t* __restrict__ argmin) {
+  const int c = threadIdx.x;
+  const int seg = __ldg(long_ids + blockIdx.x);
+  const int k0 = __ldg(piece_ptr + blockIdx.x), k1 = __ldg(piece_ptr + blockIdx.x + 1);
+  float t = 0.f, mx = -INFINITY, mn = INFINITY;
+  int ax = -1, an = -1;
+  for (int k = k0; k < k1; ++k) {
+    t = __fadd_rn(t, __ldg(p_sum + int64_t(k) * 128 + c));
+    if (MINMAX) {
+      const float a = __ldg(p_max + int64_t(k) * 128 + c), b = __ldg(p_min + int64_t(k) * 128 + c);
+      if (a > mx) { mx = a; ax = __ldg(p_amx + int64_t(k) * 128 + c); }
+      if (b < mn) { mn = b; an = __ldg(p_amn + int64_t(k) * 128 + c); }
+    }
+  }
+  float* row = out + int64_t(seg) * kPartialW;
+  row[c] = t;
+  if (MINMAX) {
+    row[128 + c] = mx;
+    row[256 + c] = mn;
+    if (argmax) argmax[int64_t(seg) * 128 + c] = ax;
+    if (argmin) argmin[int64_t(seg) * 128 + c] = an;
+  }
+  if (c == 0) reinterpret_cast<int32_t*>(row)[384] = __ldg(rowptr + seg + 1) - __ldg(rowptr + seg);
+}
+
 // fp32 sum, max, min and int32 winners per piece and feature, plus a bf16 prior row per piece
 static size_t split_reduce_bytes(const hgn_segment_split* sp) { return sp ? size_t(sp->n_pieces) * 128 * (4 * 5 + 2) : 0; }
 
@@ -524,5 +599,41 @@ extern "C" int hgn_segment_layer_grad_split(int dtype, int64_t E, int32_t D, con
       perm, rowptr, split->pieces, split->n_pieces, (const __nv_bfloat16*)g_sum, (const __nv_bfloat16*)g_mean, (const __nv_bfloat16*)g_max,
       (const __nv_bfloat16*)g_min, argmax, argmin, (const __nv_bfloat16*)base, (__nv_bfloat16*)agg_grad, (__nv_bfloat16*)edge_grad);
   HGN_LAUNCH_OK("segment_long_layer_grad");
+  return HGN_OK;
+}
+
+extern "C" int hgn_segment_partials(int dtype, const void* data, int64_t E, int32_t D, const int32_t* perm, const int32_t* rowptr, int64_t S,
+                                    const hgn_segment_split* split, int minmax, float* out, int32_t* argmax, int32_t* argmin, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  HGN_SPLIT_BF16_128("segment_partials");
+  if (split) if (int rc = check_split(split, E, S, "segment_partials")) return rc;
+  HGN_CHECK_ARG(S >= 0 && E >= 0 && (S == 0 || (rowptr && out)) && (E == 0 || (data && perm)), "segment_partials: null input/output");
+  HGN_CHECK_ARG(minmax || (!argmax && !argmin), "segment_partials: winners need minmax");
+  if (workspace_bytes < split_reduce_bytes(split) || (split && split->n_pieces > 0 && !workspace)) {
+    set_error("segment_partials: workspace %zu < %zu", workspace_bytes, split_reduce_bytes(split));
+    return HGN_ERR_WORKSPACE;
+  }
+  if (S == 0) return HGN_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const __nv_bfloat16* x = static_cast<const __nv_bfloat16*>(data);
+  {
+    HGN_TIMED("segment_partials", st);
+    segment_partial_short_kernel<<<unsigned(ceil_div(S * 32, 256)), 256, 0, st>>>(x, split ? split->perm_short : perm, split ? split->rowptr_short : rowptr,
+                                                                                   S, minmax, out, argmax, argmin);
+    HGN_LAUNCH_OK("segment_partials");
+  }
+  if (!split || split->n_long == 0) return HGN_OK;
+  // the long segments: the pieces of segment_long_partial_kernel, then their combine (it overwrites the rows the short call wrote as
+  // empty).  LongReduce only lays out the workspace and picks the piece kernel here: its out_max slot stands for "max / min wanted".
+  const LongReduce lr(split, rowptr, nullptr, nullptr, minmax ? out : nullptr, nullptr, nullptr, nullptr, 0, workspace);
+  if (int rc = lr.partial(x, perm, st)) return rc;
+  HGN_TIMED("segment_partials_long", st);
+  if (minmax)
+    segment_long_partial_combine_kernel<true><<<unsigned(split->n_long), 128, 0, st>>>(split->long_ids, split->piece_ptr, rowptr, lr.p_sum, lr.p_max,
+                                                                                      lr.p_min, lr.p_amx, lr.p_amn, out, argmax, argmin);
+  else
+    segment_long_partial_combine_kernel<false><<<unsigned(split->n_long), 128, 0, st>>>(split->long_ids, split->piece_ptr, rowptr, lr.p_sum, lr.p_max,
+                                                                                       lr.p_min, lr.p_amx, lr.p_amn, out, argmax, argmin);
+  HGN_LAUNCH_OK("segment_partials_long");
   return HGN_OK;
 }

@@ -14,6 +14,7 @@ HGN_F32 = 0
 HGN_BF16 = 1
 AGG_SUM, AGG_MEAN, AGG_MAX, AGG_MIN = 1, 2, 4, 8
 HGN_MAX_CHUNKS = 24
+HGN_SEGMENT_PARTIAL_WIDTH = 388
 HGN_IO_ENCODER, HGN_IO_DECODER = 0, 1
 ABI_VERSION = 6            # HGN_B200_ABI_VERSION of include/hgn_b200.h these signatures were written against
 
@@ -78,6 +79,8 @@ SIGNATURES = {
                                      + [c_void_p] * 7 + [c_void_p]),
     "hgn_segment_layer_grad_split": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit)]
                                      + [c_void_p] * 9 + [c_void_p]),
+    "hgn_segment_partials": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int64, POINTER(SegmentSplit), c_int]
+                             + [c_void_p] * 4 + [c_size_t, c_void_p]),
     "hgn_multi_segment_sum": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
     "hgn_mlp_packed_bytes": (c_size_t, [c_int, c_int32]),
     "hgn_mlp_pack": (c_int, [c_int, c_int32] + [c_void_p] * 8 + [c_void_p, c_void_p]),
@@ -110,6 +113,9 @@ SIGNATURES = {
     "hgn_peer_free": (c_int, [c_void_p]),
     "hgn_halo_push": (c_int, [c_int, c_void_p, c_void_p, c_int32, c_void_p, c_int32, ctypes.c_uint32, c_void_p, c_void_p]),
     "hgn_halo_wait": (c_int, [c_void_p, c_int32, ctypes.c_uint32, c_void_p]),
+    "hgn_cluster_combine": (c_int, [c_void_p, c_int32, c_int32, c_int64] + [c_void_p] * 7 + [c_void_p]),
+    "hgn_cluster_grad_sum": (c_int, [c_int, c_void_p, c_int32, c_int64, c_int32, c_void_p, c_void_p]),
+    "hgn_cluster_mean_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "hgn_colsum": (c_int, [c_int, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_size_t, c_void_p]),
     "hgn_colsum_workspace_bytes": (c_size_t, [c_int64, c_int32]),
     "hgn_world_edges_workspace_bytes": (c_size_t, [c_int64, c_int64]),

@@ -484,6 +484,60 @@ def _rows_add(rows, index32, dst) -> None:
     _count(int(n > 0))          # hgn_rows_scatter: one rows_scatter_kernel
 
 
+def _segment_partials(data, plan: SegmentPlan, out, minmax: bool, argmax, argmin) -> None:
+    """``out[S, HGN_SEGMENT_PARTIAL_WIDTH]`` fp32 = each segment's unrounded sum (and max / min with ``minmax``) and element count, as
+    the bf16 segment reductions of ``plan`` would round them (``data``: bf16 rows of width 128)."""
+    S, E = plan.num_segments, data.shape[0]
+    split = _split_of(plan, S, E)
+    ws = _split_workspace(data.device, split)
+    _cabi.check(_cabi.load().hgn_segment_partials(
+        _BF, data.data_ptr(), E, D_LATENT, plan.perm.data_ptr(), plan.rowptr.data_ptr(), S, ctypes.byref(split.c) if split is not None else None,
+        int(minmax), out.data_ptr(), _cabi.ptr(argmax), _cabi.ptr(argmin), ws.data_ptr(), ws.numel(), _cabi.stream_ptr()), "hgn_segment_partials")
+    # segment_partial_short_kernel; with a long segment also segment_long_partial and segment_long_partial_combine
+    _count(int(S > 0) + 2 * int(S > 0 and split is not None))
+
+
+def _segment_backward(plan: SegmentPlan, E: int, g_sum, g_max, g_min, argmax, argmin, grad) -> None:
+    """``grad[e] = g_sum[r] + the max / min winners' gradients`` over the segments of ``plan`` (bf16 rows of width 128): the backward of
+    ``segment_aggregate`` without a 'mean' term."""
+    S = plan.num_segments
+    split = _split_of(plan, S, E)
+    lib = _cabi.load()
+    g = [_cabi.ptr(g_sum), None, _cabi.ptr(g_max), _cabi.ptr(g_min), _cabi.ptr(argmax), _cabi.ptr(argmin)]
+    if split is not None:
+        _cabi.check(lib.hgn_segment_reduce_bwd_split(_BF, E, D_LATENT, plan.ids32.data_ptr(), plan.perm.data_ptr(), plan.rowptr.data_ptr(), S,
+                                                     ctypes.byref(split.c), *g, grad.data_ptr(), _cabi.stream_ptr()), "hgn_segment_reduce_bwd_split")
+        _count(2)               # segment_bwd_bf16_128_kernel on the short CSR, segment_long_bwd_kernel
+        return
+    _cabi.check(lib.hgn_segment_reduce_bwd(_BF, E, D_LATENT, plan.ids32.data_ptr(), plan.perm.data_ptr(), plan.rowptr.data_ptr(), S, *g,
+                                           grad.data_ptr(), 0, _cabi.stream_ptr()), "hgn_segment_reduce_bwd")
+    _count()                    # one backward kernel
+
+
+def _cluster_combine(slots, world: int, rank: int, outs, argmax, argmin, count) -> None:
+    """Rank-ordered reduction of every rank's partial rows ``slots[world, C, HGN_SEGMENT_PARTIAL_WIDTH]`` into ``outs`` = (sum, mean, max,
+    min; None = not wanted), bf16 ``[C, 128]``; clears this rank's winners where another rank won and writes the total counts."""
+    C = slots.shape[1]
+    _cabi.check(_cabi.load().hgn_cluster_combine(slots.data_ptr(), world, rank, C, *[_cabi.ptr(o) for o in outs], _cabi.ptr(argmax),
+                                                 _cabi.ptr(argmin), _cabi.ptr(count), _cabi.stream_ptr()), "hgn_cluster_combine")
+    _count(int(C > 0))          # one cluster_combine_kernel
+
+
+def _cluster_grad_sum(slots, out) -> None:
+    """``out[C, D] = sum over ranks, in rank order, of slots[r]`` (bf16 rows, fp32 accumulation, one rounding)."""
+    world, C, D = slots.shape
+    _cabi.check(_cabi.load().hgn_cluster_grad_sum(_BF, slots.data_ptr(), world, C, D, out.data_ptr(), _cabi.stream_ptr()), "hgn_cluster_grad_sum")
+    _count(int(C * D > 0))      # one cluster_grad_sum_kernel
+
+
+def _cluster_mean_grad(g_sum, g_mean, count, out) -> None:
+    """``out = g_sum + g_mean / count`` per cluster row (bf16 ``[C, 128]``, one rounding)."""
+    C = g_mean.shape[0]
+    _cabi.check(_cabi.load().hgn_cluster_mean_grad(_cabi.ptr(g_sum), g_mean.data_ptr(), count.data_ptr(), C, out.data_ptr(), _cabi.stream_ptr()),
+                "hgn_cluster_mean_grad")
+    _count(int(C > 0))          # one cluster_mean_grad_kernel
+
+
 class _NodeProjection(torch.autograd.Function):
     """``Ps = v W0[:, 0:128]^T``, ``Pr = v W0[:, 128:256]^T`` -- the sender / receiver blocks of the edge MLP's first
     linear (graphnet.py:28-31 concatenation order), applied once per node instead of once per edge."""

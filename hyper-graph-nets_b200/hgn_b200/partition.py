@@ -20,13 +20,15 @@ Nothing here does arithmetic on latents besides the pack / scatter-add row kerne
 """
 from __future__ import annotations
 
+import ctypes
 from dataclasses import dataclass
-from typing import List, NamedTuple, Optional, Sequence
+from typing import Dict, List, NamedTuple, Optional, Sequence
 
 import torch
 import torch.distributed as dist
 
 from . import _cabi, ops
+from ._cabi import HgnError
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -118,6 +120,57 @@ def build_local_graph(senders: torch.Tensor, receivers: torch.Tensor, part: torc
     return LocalGraph(rank=rank, world=world, owned=owned, ghosts=ghosts, ghost_splits=ghost_splits,
                       send_index=torch.cat(send_lists), send_splits=[int(t.numel()) for t in send_lists],
                       edge_ids=edge_ids, senders=local_of[s_glob], receivers=local_of[r_glob], n_interior=n_interior)
+
+
+HYPER_REMOTE_SETS = ("intra_cluster_to_cluster", "inter_cluster", "intra_cluster_to_mesh")
+
+
+class LocalEdges(NamedTuple):
+    edge_ids: torch.Tensor         # [e_loc] global ids of the local edges (ascending)
+    senders: torch.Tensor          # [e_loc] local sender index into [owned | hyper]
+    receivers: torch.Tensor        # [e_loc] local receiver index into [owned | hyper]
+
+
+@dataclass
+class LocalHyperGraph:
+    """One rank's share of a HyperGraphNet graph.  The mesh edges follow ``build_local_graph``; in the remote edge sets the local node
+    list is ``[owned | hyper]`` (hyper node c is local row ``n_own + c``, the reference's ``[mesh, hyper]`` layout), and
+    ``intra_cluster_to_cluster`` keeps the edges of an owned sender, ``intra_cluster_to_mesh`` those of an owned receiver and
+    ``inter_cluster`` every edge."""
+    mesh: LocalGraph
+    num_clusters: int
+    remote: Dict[str, LocalEdges]
+
+    @property
+    def n_own(self) -> int:
+        return self.mesh.n_own
+
+
+def build_local_hyper_graph(index_lists, num_nodes: int, num_clusters: int, part: torch.Tensor, rank: int, world: int) -> LocalHyperGraph:
+    """Rank ``rank``'s share of the four edge sets of a HyperGraphNet graph.  ``index_lists``: set name -> global ``(senders,
+    receivers)``, with hyper node c numbered ``num_nodes + c`` (``rmp.hierarchical_connector.connector_indices``)."""
+    names = set(index_lists)
+    if names != {"mesh_edges", *HYPER_REMOTE_SETS}:
+        raise HgnError(f"build_local_hyper_graph: edge sets must be exactly mesh_edges and {', '.join(HYPER_REMOTE_SETS)}; got {sorted(names)}")
+    part = part.cpu()
+    mesh = build_local_graph(*index_lists["mesh_edges"], part, rank, world)
+    n_own = mesh.n_own
+    local_of = torch.full((num_nodes,), -1, dtype=torch.int64)
+    local_of[mesh.owned] = torch.arange(n_own)
+    mesh_side = {"intra_cluster_to_cluster": (True, False), "inter_cluster": (False, False), "intra_cluster_to_mesh": (False, True)}
+    remote = {}
+    for name in HYPER_REMOTE_SETS:
+        s, r = (t.cpu().to(torch.int64) for t in index_lists[name])
+        mesh_s, mesh_r = mesh_side[name]
+        for ids, is_mesh in ((s, mesh_s), (r, mesh_r)):
+            lo, hi = (0, num_nodes) if is_mesh else (num_nodes, num_nodes + num_clusters)
+            if ids.numel() and (int(ids.min()) < lo or int(ids.max()) >= hi):
+                raise HgnError(f"build_local_hyper_graph: {name} indices outside [{lo}, {hi})")
+        owner_side = s if mesh_s else (r if mesh_r else None)
+        edge_ids = torch.arange(s.numel()) if owner_side is None else torch.nonzero(part[owner_side] == rank).flatten()
+        loc = lambda ids, is_mesh: local_of[ids] if is_mesh else n_own + (ids - num_nodes)
+        remote[name] = LocalEdges(edge_ids, loc(s[edge_ids], mesh_s), loc(r[edge_ids], mesh_r))
+    return LocalHyperGraph(mesh=mesh, num_clusters=int(num_clusters), remote=remote)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -378,6 +431,197 @@ class PeerLayerHalo(NamedTuple):
         self.peer.push_backward(self.step, self.layer, gs)
 
 
+class PeerPool:
+    """Every rank's ``[C, W]`` rows of one cross-rank cluster exchange, in NVLink peer memory (csrc/peer.cu).  A partitioned
+    HyperGraphNet block has three such exchanges: the fp32 partials of its cluster pooling (forward, ``POOL``), and in the backward pass
+    the gradients of the replicated hyper rows its down-edge senders (``DOWN``) and up-edge receivers (``UP``) read.  Each rank pushes
+    its rows into slot ``rank`` of every rank's pool (its own included) with ``hgn_halo_push``, waits for the peers' flags with
+    ``hgn_halo_wait``, and reduces slots ``0 .. world-1`` in rank order: every rank runs the same arithmetic on the same bytes.
+
+    Pool layout (bytes): ``[flags: 3 directions x world uint32 | push counter | per (step parity, layer): POOL world x C x 388 fp32,
+    DOWN and UP world x C x 128 bf16]``.  Slots are per (step parity, layer, direction), like ``PeerHalo``'s tables, and every rank
+    waits for every other in each exchange, so no rank can be far enough ahead to overwrite rows that are still to be read.  Unlike
+    ``PeerHalo``, every peer is mapped."""
+
+    POOL, DOWN, UP = 0, 1, 2
+
+    def __init__(self, num_clusters: int, layers: int, device, group=None):
+        lib = _cabi.load()
+        self.C, self.layers, self.group, self.device = int(num_clusters), int(layers), group, torch.device(device)
+        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
+        if self.world > _cabi.HGN_MAX_PEERS:
+            raise HgnError(f"PeerPool: {self.world} ranks, at most {_cabi.HGN_MAX_PEERS}")
+        self.row_bytes = {self.POOL: _cabi.HGN_SEGMENT_PARTIAL_WIDTH * 4, self.DOWN: ops.D_LATENT * 2, self.UP: ops.D_LATENT * 2}
+        self.dir_off, off = {}, 0
+        for d in (self.POOL, self.DOWN, self.UP):
+            self.dir_off[d] = off
+            off += self.world * self.C * self.row_bytes[d]
+        self.layer_bytes = 256 * ((off + 255) // 256)
+        self.off_counter = 3 * self.world * 4
+        self.off_slots = 256 * ((self.off_counter + 4 + 255) // 256)
+        self.nbytes = self.off_slots + 2 * self.layers * self.layer_bytes
+        with torch.cuda.device(self.device):
+            ptr = ctypes.c_void_p()
+            handle = ctypes.create_string_buffer(64)
+            _cabi.check(lib.hgn_peer_alloc(self.nbytes, ctypes.byref(ptr), handle), "hgn_peer_alloc")
+        self.base = int(ptr.value)
+        self.pool = torch.as_tensor(_DeviceBytes(self.base, self.nbytes), device=self.device)
+        handles = [None] * self.world
+        dist.all_gather_object(handles, bytes(handle.raw), group=group)
+        self.peer_base = [0] * self.world
+        with torch.cuda.device(self.device):
+            for q in range(self.world):
+                if q != self.rank:
+                    mapped = ctypes.c_void_p()
+                    _cabi.check(lib.hgn_peer_open(handles[q], ctypes.byref(mapped)), "hgn_peer_open")
+                    self.peer_base[q] = int(mapped.value)
+        self.index32 = torch.arange(self.C, dtype=torch.int32).repeat(self.world).to(self.device)
+        dist.barrier(group=group)                             # every pool exists and is mapped before anybody pushes
+
+    def close(self) -> None:
+        lib = _cabi.load()
+        torch.cuda.synchronize(self.device)
+        dist.barrier(group=self.group)
+        for q, p in enumerate(self.peer_base):
+            if p:
+                lib.hgn_peer_close(p)
+                self.peer_base[q] = 0
+        if self.base:
+            self.pool = None
+            lib.hgn_peer_free(self.base)
+            self.base = 0
+
+    def _slot_offset(self, step: int, layer: int, direction: int) -> int:
+        return self.off_slots + ((step & 1) * self.layers + layer) * self.layer_bytes + self.dir_off[direction]
+
+    def exchange(self, rows: torch.Tensor, step: int, layer: int, direction: int) -> torch.Tensor:
+        """Pushes ``rows`` ([C, W], contiguous: fp32 partials for ``POOL``, bf16 gradients otherwise) into slot ``rank`` of every rank's
+        pool, waits for the other ranks' rows and returns this rank's ``[world, C, W]`` view of all of them, in rank order."""
+        lib = _cabi.load()
+        off, rb = self._slot_offset(step, layer, direction), self.row_bytes[direction]
+        assert rows.is_contiguous() and rows.shape[0] == self.C and rows.shape[1] * rows.element_size() == rb
+        # epochs rise within a direction: the forward visits the layers in ascending order, the backward in descending order
+        epoch = (1 + step * self.layers + (layer if direction == self.POOL else self.layers - 1 - layer)) & 0x7FFFFFFF
+        peers, flags = _cabi.HaloPeers(), _cabi.HaloFlags()
+        n_wait = 0
+        for q in range(self.world):
+            base = self.base if q == self.rank else self.peer_base[q]
+            peers.dst[q] = base + off + self.rank * self.C * rb
+            peers.flag[q] = None if q == self.rank else base + (direction * self.world + self.rank) * 4
+            peers.row_begin[q] = q * self.C
+            if q != self.rank:
+                flags.flag[n_wait] = self.base + (direction * self.world + q) * 4
+                n_wait += 1
+        peers.row_begin[self.world] = self.world * self.C
+        with torch.cuda.device(self.device):
+            st = _cabi.stream_ptr()
+            _cabi.check(lib.hgn_halo_push(_cabi.dtype_code(rows.dtype), rows.data_ptr(), self.index32.data_ptr(), rows.shape[1], ctypes.byref(peers),
+                                          self.world, epoch, self.base + self.off_counter, st), "hgn_halo_push")
+            _cabi.check(lib.hgn_halo_wait(ctypes.byref(flags), n_wait, epoch, st), "hgn_halo_wait")
+        ops._count(1 + int(n_wait > 0))               # csrc/peer.cu: one push kernel, one wait kernel when there are peers
+        n = self.world * self.C * rb
+        return self.pool[off: off + n].view(rows.dtype).view(self.world, self.C, rows.shape[1])
+
+
+class _ClusterPool(torch.autograd.Function):
+    """The cluster pooling of the up edges across ranks: this rank's fp32 partials (``hgn_segment_partials`` over its own up edges,
+    keyed by cluster) -> every rank's pool -> ``hgn_cluster_combine`` in rank order -> the bf16 ``[C, 128]`` aggregates of ``reducers``,
+    bit-identical on every rank.  Backward: each rank's partial receives the full gradient of the aggregates ('mean' divided by the
+    global count; max / min only where this rank holds the winner, as the combine cleared the other winners), through the existing
+    segment backward over the local elements."""
+
+    @staticmethod
+    def forward(ctx, e, plan, pool: PeerPool, step, layer, reducers):
+        C, dev = plan.num_segments, e.device
+        minmax = "max" in reducers or "min" in reducers
+        winners = minmax and ctx.needs_input_grad[0]
+        new_arg = lambda op: torch.empty((C, ops.D_LATENT), dtype=torch.int32, device=dev) if winners and op in reducers else None
+        argmax, argmin = new_arg("max"), new_arg("min")
+        partial = torch.empty((C, _cabi.HGN_SEGMENT_PARTIAL_WIDTH), dtype=torch.float32, device=dev)
+        outs = {op: torch.empty((C, ops.D_LATENT), dtype=torch.bfloat16, device=dev) for op in reducers}
+        count = torch.empty(C, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            ops._segment_partials(e, plan, partial, minmax, argmax, argmin)
+            slots = pool.exchange(partial, step, layer, PeerPool.POOL)
+            ops._cluster_combine(slots, pool.world, pool.rank, [outs.get(op) for op in ops.OP_BITS], argmax, argmin, count)
+        ctx.save_for_backward(argmax, argmin, count)
+        ctx.plan, ctx.reducers, ctx.E = plan, reducers, e.shape[0]
+        return tuple(outs[op] for op in reducers)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        argmax, argmin, count = ctx.saved_tensors
+        g = {op: gi.contiguous().to(torch.bfloat16) for op, gi in zip(ctx.reducers, grads) if gi is not None}
+        ref = next(iter(g.values()))
+        grad = torch.empty((ctx.E, ops.D_LATENT), dtype=torch.bfloat16, device=ref.device)
+        with torch.cuda.device(ref.device):
+            g_sum = g.get("sum")
+            if "mean" in g:
+                g_sum_mean = torch.empty_like(g["mean"])
+                ops._cluster_mean_grad(g_sum, g["mean"], count, g_sum_mean)
+                g_sum = g_sum_mean
+            ops._segment_backward(ctx.plan, ctx.E, g_sum, g.get("max"), g.get("min"), argmax if "max" in g else None,
+                                  argmin if "min" in g else None, grad)
+        return grad, None, None, None, None, None
+
+
+class _EnterLocal(torch.autograd.Function):
+    """Where the replicated hyper rows feed rank-local edges: the identity forward; backward, the rank-ordered sum of every rank's
+    gradient (``hgn_cluster_grad_sum``), so the gradient that reaches the replicated computation is complete and the same on every
+    rank."""
+
+    @staticmethod
+    def forward(ctx, h, pool: PeerPool, step, layer, direction):
+        ctx.pool, ctx.step, ctx.layer, ctx.direction = pool, step, layer, direction
+        return h.view_as(h)
+
+    @staticmethod
+    def backward(ctx, g):
+        g = g.contiguous().to(torch.bfloat16)
+        out = torch.empty_like(g)
+        with torch.cuda.device(g.device):
+            slots = ctx.pool.exchange(g, ctx.step, ctx.layer, ctx.direction)
+            ops._cluster_grad_sum(slots, out)
+        return out, None, None, None, None
+
+
+_HYPER_SCOPE = ("the partitioned processor takes plain GraphNet blocks, or HyperGraphNet blocks with edge sets exactly mesh_edges, "
+                "intra_cluster_to_cluster, inter_cluster and intra_cluster_to_mesh, the 'sum', 'mean', 'max', 'min' or 'pna' aggregator, "
+                "bf16 latents of width 128, a PeerHalo and the rank's LocalHyperGraph (build_local_hyper_graph); HeteroGraphNet, "
+                "MultiScaleGraphNet, world_edges and fp32 parity mode are not supported")
+
+
+class _HyperLocal:
+    """Device-side index tensors and segment plans of a ``LocalHyperGraph`` (the tensors stay referenced: plans are cached by them)."""
+
+    def __init__(self, hyper: LocalHyperGraph, device):
+        from .plan import segment_plan
+        n_own, C = hyper.n_own, hyper.num_clusters
+        self.n_own, self.C = n_own, C
+
+        def plans(s, r, n):
+            s, r = s.to(device), r.to(device)
+            return s, r, segment_plan(s, n), segment_plan(r, n)
+        rem = hyper.remote
+        self.up = plans(rem["intra_cluster_to_cluster"].senders, rem["intra_cluster_to_cluster"].receivers, n_own + C)
+        self.down = plans(rem["intra_cluster_to_mesh"].senders, rem["intra_cluster_to_mesh"].receivers, n_own + C)
+        # the across phase runs on the C hyper rows alone: every rank computes it from the same rows
+        self.across = plans(rem["inter_cluster"].senders - n_own, rem["inter_cluster"].receivers - n_own, C)
+        self.cluster_ids = (rem["intra_cluster_to_cluster"].receivers - n_own).to(device)
+        self.cluster_plan = segment_plan(self.cluster_ids, C)
+
+
+def _edge(block, name, v, e, s_plan, r_plan, want_agg):
+    from .migration.graphnet import _mlp_parameters, _packed_cache
+    model = block.edge_models[name]
+    return ops.edge_update(_mlp_parameters(model, 3 * v.shape[1], v), _packed_cache(model), v, e, s_plan, r_plan, want_agg)
+
+
+def _node(model, rows, aggs):
+    from .migration.graphnet import _mlp_parameters, _packed_cache
+    return ops.node_update(_mlp_parameters(model, (1 + len(aggs)) * rows.shape[1], rows), _packed_cache(model), rows, aggs)
+
+
 class PartitionedProcessor(torch.nn.Module):
     """Runs a (reference-API) ``Processor`` on one rank's share of the graph.
 
@@ -386,13 +630,30 @@ class PartitionedProcessor(torch.nn.Module):
     Fast path (``PeerHalo`` given, and every block takes the whole-layer route of ``GraphNet``: one edge set, bf16, any of the
     'sum' / 'mean' / 'max' / 'min' / 'pna' aggregators -- the cfg5 benchmark): ``ops.graphnet_layer`` per block with the halo of that
     layer; halo rows travel as peer-memory stores issued by a kernel of the sending rank.  Every edge of an owned receiver is local,
-    so the aggregates (max / min winners included) need no exchange of their own."""
+    so the aggregates (max / min winners included) need no exchange of their own.
+    HyperGraphNet path (``hyper`` = this rank's ``LocalHyperGraph``, a ``PeerHalo`` given): ``_hyper_block`` per block, with the C hyper
+    rows replicated on every rank and the cluster pooling combined across ranks through a ``PeerPool`` (DESIGN.md s6.1).  Other
+    hierarchical blocks raise ``HgnError``."""
 
-    def __init__(self, processor: torch.nn.Module, plan: HaloPlan, peer: Optional[PeerHalo] = None):
+    def __init__(self, processor: torch.nn.Module, plan: HaloPlan, peer: Optional[PeerHalo] = None, hyper: Optional[LocalHyperGraph] = None):
         super().__init__()
+        from .migration.graphnet import PNA_OPS
+        from .migration.heterographnet import HeteroGraphNet
+        from .migration.hypergraphnet import HyperGraphNet
+        from .migration.multiscalegraphnet import MultiScaleGraphNet
         self.processor = processor
         self.plan = plan
         self.peer = peer
+        self.hyper = self.pool = None
+        blocks = list(processor.graphnet_blocks)
+        if hyper is not None or any(isinstance(b, (HyperGraphNet, HeteroGraphNet, MultiScaleGraphNet)) for b in blocks):
+            # the generic route would read a HyperGraphNet's hyper slot as the ghosts: only the schedule of _hyper_block is right
+            sets = {"mesh_edges", *HYPER_REMOTE_SETS}
+            if not all(type(b) is HyperGraphNet and set(b.edge_models.keys()) == sets and b.message_passing_aggregator in PNA_OPS + ("pna",)
+                       for b in blocks) or peer is None or hyper is None:
+                raise HgnError(_HYPER_SCOPE)
+            self.hyper = _HyperLocal(hyper, peer.device)
+            self.pool = PeerPool(hyper.num_clusters, len(blocks), peer.device, peer.group)
         if peer is not None:
             from .plan import segment_plan
             lg, dev = peer.lg, peer.device
@@ -406,7 +667,24 @@ class PartitionedProcessor(torch.nn.Module):
         return (self.peer is not None and len(blocks) == self.peer.layers
                 and all(takes_whole_layer(b, owned, edge_sets) for b in blocks))
 
-    def forward(self, owned: torch.Tensor, edge_sets):
+    def replicated_parameters(self) -> List[torch.nn.Parameter]:
+        """The parameters every rank computes redundantly from the same rows (the hyper-node MLPs and the ``inter_cluster`` edge MLP of a
+        HyperGraphNet block): their gradients are complete and identical on every rank, so ``allreduce_gradients`` leaves them out."""
+        if self.hyper is None:
+            return []
+        return [p for b in self.processor.graphnet_blocks
+                for m in (b.hyper_node_model_up, b.hyper_node_model_cross, b.edge_models["inter_cluster"]) for p in m.parameters()]
+
+    def close(self) -> None:
+        """Frees the cluster exchange pool of a HyperGraphNet processor (the ``PeerHalo`` belongs to the caller)."""
+        if self.pool is not None:
+            self.pool.close()
+
+    def forward(self, owned: torch.Tensor, edge_sets, hyper_nodes: Optional[torch.Tensor] = None):
+        """``(owned', edge_sets')``; for HyperGraphNet blocks ``(owned', edge_sets', hyper')`` from the C replicated hyper rows
+        ``hyper_nodes`` (the same on every rank), with the edge sets' local indices of ``build_local_hyper_graph``."""
+        if self.hyper is not None:
+            return self._hyper_forward(owned, edge_sets, hyper_nodes)
         from . import config
         from .util import MultiGraph
         precision = getattr(self.processor, "precision", None) or config.precision()
@@ -429,10 +707,57 @@ class PartitionedProcessor(torch.nn.Module):
         out_nodes = graph.node_features[0].to(in_dtype)
         return out_nodes, list(graph.edge_sets)      # edge latents stay in the compute dtype (see Processor.forward)
 
+    def _hyper_forward(self, owned, edge_sets, hyper_nodes):
+        from . import config
+        precision = getattr(self.processor, "precision", None) or config.precision()
+        names = [es.name for es in edge_sets]
+        if precision != "bf16" or hyper_nodes is None or sorted(names) != sorted(("mesh_edges",) + HYPER_REMOTE_SETS):
+            raise HgnError(_HYPER_SCOPE + f" (got precision {precision!r}, edge sets {names}, hyper rows {'given' if hyper_nodes is not None else 'missing'})")
+        in_dtype = owned.dtype
+        owned, hyper = owned.to(torch.bfloat16), hyper_nodes.to(torch.bfloat16)
+        feats = {es.name: es.features.to(torch.bfloat16) for es in edge_sets}
+        step = self.peer.steps_done
+        self.peer.steps_done += 1
+        for layer, block in enumerate(self.processor.graphnet_blocks):
+            owned, hyper = self._hyper_block(block, step, layer, owned, hyper, feats)
+        # edge latents stay in the compute dtype (see Processor.forward); both node lists go back, like Processor.forward's
+        return owned.to(in_dtype), [es._replace(features=feats[es.name]) for es in edge_sets], hyper.to(in_dtype)
 
-def allreduce_gradients(module: torch.nn.Module, group=None) -> None:
-    """Sum the per-rank partial weight gradients (one flat fp32 all-reduce)."""
-    grads = [p.grad for p in module.parameters() if p.grad is not None]
+    def _hyper_block(self, block, step, layer, owned, hyper, feats):
+        """One HyperGraphNet block (hypergraphnet.py) on this rank's share; ``feats`` (set name -> edge latents) is updated in place.
+        The mesh phase is the fused layer with the NVLink halo; the up phase pools its owned members' edges into fp32 partials combined
+        across ranks; the across phase (C rows, ~C^2 edges) runs on every rank from the same rows; the down phase is local."""
+        h = self.hyper
+        agg = block.message_passing_aggregator
+        reducers = tuple(ops.OP_BITS) if agg == "pna" else (agg,)
+        peer, pool = self.peer, self.pool
+        # mesh phase (hypergraphnet.py:29-34)
+        owned, feats["mesh_edges"] = block._layer(owned, feats["mesh_edges"], "mesh_edges", peer.s_plan, peer.r_plan,
+                                                  PeerLayerHalo(peer, step, layer))
+        # node -> hyper-node pooling (:37-39)
+        _, _, s_plan, r_plan = h.up
+        v = torch.cat([owned, _EnterLocal.apply(hyper, pool, step, layer, PeerPool.UP)])
+        feats["intra_cluster_to_cluster"], _ = _edge(block, "intra_cluster_to_cluster", v, feats["intra_cluster_to_cluster"], s_plan, r_plan, False)
+        pooled = _ClusterPool.apply(feats["intra_cluster_to_cluster"], h.cluster_plan, pool, step, layer, reducers)
+        hyper = _node(block.hyper_node_model_up, hyper, list(pooled))
+        # hyper-node <-> hyper-node (:42-47), on the C hyper rows alone
+        _, _, s_plan, r_plan = h.across
+        feats["inter_cluster"], a = _edge(block, "inter_cluster", hyper, feats["inter_cluster"], s_plan, r_plan, agg == "sum")
+        hyper = _node(block.hyper_node_model_cross, hyper, [a] if agg == "sum" else ops.segment_aggregate(feats["inter_cluster"], r_plan, reducers))
+        # hyper-node -> node broadcast (:50-52)
+        _, _, s_plan, r_plan = h.down
+        v = torch.cat([owned, _EnterLocal.apply(hyper, pool, step, layer, PeerPool.DOWN)])
+        feats["intra_cluster_to_mesh"], a = _edge(block, "intra_cluster_to_mesh", v, feats["intra_cluster_to_mesh"], s_plan, r_plan, agg == "sum")
+        aggs = [a] if agg == "sum" else ops.segment_aggregate(feats["intra_cluster_to_mesh"], r_plan, reducers)
+        owned = _node(block.node_model_down, owned, [x[:h.n_own] for x in aggs])
+        return owned, hyper
+
+
+def allreduce_gradients(module: torch.nn.Module, group=None, exclude: Sequence[torch.nn.Parameter] = ()) -> None:
+    """Sum the per-rank partial weight gradients (one flat fp32 all-reduce).  ``exclude``: parameters whose gradients are already
+    complete on every rank (``PartitionedProcessor.replicated_parameters``)."""
+    skip = {id(p) for p in exclude}
+    grads = [p.grad for p in module.parameters() if p.grad is not None and id(p) not in skip]
     if not grads:
         return
     flat = torch.cat([g.reshape(-1) for g in grads])

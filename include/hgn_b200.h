@@ -188,6 +188,17 @@ int hgn_segment_layer_grad_split(int dtype, int64_t num_edges, int32_t D, const 
                                  const int32_t* argmax, const int32_t* argmin, const void* base, void* agg_grad, void* edge_grad,
                                  void* stream);
 
+/* fp32 partials of a segment reduction (the cluster pooling of a partitioned HyperGraphNet, combined across ranks before rounding):
+ * row s of out ([S, HGN_SEGMENT_PARTIAL_WIDTH] fp32) is [sum 0..127 | max 128..255 | min 256..383 | count (int32 bits) | 3 x 0],
+ * holding the values hgn_segment_reduce / hgn_segment_reduce_split would round to bf16 -- the same summation order, on the short
+ * CSR and by pieces for the long segments -- and the segment's element count.  max / min and the winners are written only with
+ * minmax; an empty segment leaves sum 0, max -inf, min +inf, winners -1, count 0.  bf16 rows of width 128; split may be NULL (no long
+ * segment); the workspace is hgn_segment_split_reduce_workspace_bytes(split). */
+#define HGN_SEGMENT_PARTIAL_WIDTH 388
+int hgn_segment_partials(int dtype, const void* data, int64_t num_edges, int32_t D, const int32_t* perm, const int32_t* rowptr,
+                         int64_t num_segments, const hgn_segment_split* split, int minmax, float* out, int32_t* argmax, int32_t* argmin,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* Backward of the row gathers v[senders], v[receivers] (torch.index_select -> index_add_ with float
  * atomics in the reference, src/migration/graphnet.py:28-29): out[n,:] = base[n,:] (if base != NULL)
  * + sum_k sum_{j in segment_k(n)} data_k[perm_k[j], :], accumulated in fp32 in a fixed order
@@ -373,6 +384,20 @@ int hgn_peer_free(void* ptr);
 int hgn_halo_push(int dtype, const void* table, const int32_t* send_index, int32_t D, const hgn_halo_peers* peers, int32_t n_peers,
                   uint32_t epoch, void* counter, void* stream);
 int hgn_halo_wait(const hgn_halo_flags* flags, int32_t n_flags, uint32_t epoch, void* stream);
+
+/* ---- cluster pooling across ranks (partitioned HyperGraphNet; the rows travel with hgn_halo_push / hgn_halo_wait) -------------
+ * hgn_cluster_combine: slots = [world][C][HGN_SEGMENT_PARTIAL_WIDTH] fp32, every rank's hgn_segment_partials rows in rank order.
+ * Per cluster and feature, in rank order: sum = bf16_rn((((0 + s_0) + s_1) + ...)), mean = bf16_rn(total * (1.0f / max(cnt, 1))),
+ * max / min over the ranks with a nonzero count (strict comparisons: the lowest rank wins a tie; 0 when every count is 0).  Any output
+ * may be NULL.  argmax / argmin are this rank's local winners: cleared to -1 where another rank won.  count (may be NULL) receives
+ * the total counts.  Every rank runs this on the same bytes, so the outputs are bit-identical on every rank.
+ * hgn_cluster_grad_sum: out[C, D] = bf16_rn(sum over r in rank order of slots[r]) from +0 in fp32; slots = [world][C][D] bf16.
+ * hgn_cluster_mean_grad: out = bf16_rn(fma(g_mean, 1.0f / max(count, 1), 0 + g_sum)) per [C, 128] bf16 row (g_sum may be NULL):
+ * the 'sum' and 'mean' gradient of a pooled cluster as one sum term for hgn_segment_reduce_bwd on the local elements. */
+int hgn_cluster_combine(const float* slots, int32_t world, int32_t rank, int64_t num_clusters, void* out_sum, void* out_mean,
+                        void* out_max, void* out_min, int32_t* argmax, int32_t* argmin, int32_t* count, void* stream);
+int hgn_cluster_grad_sum(int dtype, const void* slots, int32_t world, int64_t num_clusters, int32_t D, void* out, void* stream);
+int hgn_cluster_mean_grad(const void* g_sum, const void* g_mean, const int32_t* count, int64_t num_clusters, void* out, void* stream);
 
 /* ---- world edges: fixed-radius neighbour search ----------------------------------------------------
  * Replaces the dense search of PlateModel.build_graph (src/model/plate.py:86-110): torch.cdist over all
